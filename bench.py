@@ -4,7 +4,7 @@ scanned per second (BASELINE.json: "Gnt/s scanned (both strands) per
 descriptor at 1/2/4/8 B200; hits bit-exact").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl gpumotif|reference]
-                    [--descr trna] [--mnt 1024] [--configs all|none|a,b,..]
+                    [--descr trna] [--mnt 1024] [--configs all|none|a,b,..] [--dump-outputs DIR]
 
 A step is one pass of the hot path over one batch: every start offset on the
 searched strands of a synthetic database (i.i.d. uniform acgt, SURVEY.md 8d).
@@ -405,6 +405,7 @@ class Bench:
         if self.world > 1:
             self.dist.barrier()
         res["parity"] = par
+        res["hits"] = hits_res
         ms.close()
         return res
 
@@ -493,6 +494,31 @@ def write_fasta(path, n_rec, rec_nt, seed, width=70):
             if rest:
                 fh.write(lut[rng.integers(0, 4, size=rest, dtype=np.uint8)].tobytes() + b"\n")
     return n_rec * rec_nt
+
+
+DUMP_BYTES = 64_000_000
+NPY_HEADER_RESERVE = 4096  # the .npy headers of one workload's 13 files (128 bytes each)
+
+
+def dump_hits(out_dir, workload, hits, budget):
+    """The candidates of the last timed resident step of one workload, one float64 array per
+    field of the hit record (integers, all exact in float64), as out_dir/<workload>.<field>.npy.
+    `rows` holds the indices of the written candidates: all of them when the files fit in
+    `budget` bytes, else a fixed, seeded sample in enumeration order."""
+    nd = hits.dtype["el"].shape[0]
+    row_bytes = 8 * (1 + 8 + 4 * nd)
+    n = len(hits)
+    cap = max(0, (budget - NPY_HEADER_RESERVE) // row_bytes)
+    rows = np.arange(n) if n <= cap else np.sort(np.random.default_rng(0).choice(n, size=cap, replace=False))
+    h = hits[rows]
+    cols = {"rows": rows}
+    for f in ("rec", "szero", "seq", "comp", "lctx_off", "lctx_len", "rctx_off", "rctx_len"):
+        cols[f] = h[f]
+    for f in ("off", "len", "mpr", "mm"):
+        cols["el_" + f] = h["el"][f].reshape(len(h), nd)
+    os.makedirs(out_dir, exist_ok=True)
+    for f, a in cols.items():
+        np.save(os.path.join(out_dir, f"{workload}.{f}.npy"), np.asarray(a, dtype=np.float64))
 
 
 def _pipeline_rate(summary):
@@ -587,12 +613,16 @@ def run_gpu_arm(args):
     B = Bench(args)
     rank, world = B.rank, B.world
     pk, which = peaks()
+    names = [] if args.configs == "none" else (list(CONFIGS) if args.configs == "all" else args.configs.split(","))
+    dump_budget = DUMP_BYTES // (1 + len(names))
 
     # ---- headline: BASELINE.json's target config ----------------------------------
     plan = load_plan(args.descr)
     rec_off, total = B.database([1_000_000] * max(1, args.mnt), 1001)
     res = B.measure(plan, rec_off, total, args.steps, args.warmup, clocks=True,
                     prefix_recs=(16 if not args.no_parity else 0), tile=args.tile)
+    if args.dump_outputs and rank == 0:
+        dump_hits(args.dump_outputs, args.descr, res["hits"], dump_budget)
     name, dom_ms, alg, share, k_ms, f_ms = dominant_kernel(res, args.steps, res["n_descr"])
     line = None
     if rank == 0:
@@ -643,7 +673,6 @@ def run_gpu_arm(args):
 
     # ---- the other configs of BASELINE.json ------------------------------------------
     per_config = []
-    names = [] if args.configs == "none" else (list(CONFIGS) if args.configs == "all" else args.configs.split(","))
     for cname in names:
         pname, lengths, seed, pre = CONFIGS[cname]
         cplan = load_plan(pname)
@@ -652,6 +681,8 @@ def run_gpu_arm(args):
                       prefix_recs=(pre if not args.no_parity else 0), score=load_score(pname))
         if rank != 0:
             continue
+        if args.dump_outputs:
+            dump_hits(args.dump_outputs, cname, r["hits"], dump_budget)
         kname, kms, kalg, kshare, kk_ms, kf_ms = dominant_kernel(r, args.cfg_steps, r["n_descr"])
         entry = {
             "config": cname, "workload": f"{pname}.descr over {len(lengths)} records, {c_total / 1e6:.1f} Mnt per GPU "
@@ -709,7 +740,7 @@ def main():
     ap.add_argument("--mnt", type=int, default=1024, help="Mnt of synthetic sequence per GPU (headline)")
     ap.add_argument("--configs", default="all", help="per_config block: all, none, or a comma list of "
                     + ",".join(CONFIGS))
-    ap.add_argument("--cfg-steps", type=int, default=2)
+    ap.add_argument("--cfg-steps", type=int, default=None, help="timed steps of each per_config workload (default: --steps)")
     ap.add_argument("--cfg-warmup", type=int, default=3)
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle prefix checks")
@@ -717,7 +748,14 @@ def main():
     ap.add_argument("--binary-mnt", type=int, default=1024, help="Mnt of the FASTA file the program leg reads")
     ap.add_argument("--upload", default="chars,hostpack", help="e2e leg: chars, hostpack, or both (the faster is reported)")
     ap.add_argument("--tile", type=int, default=0, help="starts per tile (0 = library default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the candidates of each workload's last timed step (rank 0) as DIR/<workload>.<field>.npy "
+                         "(float64, at most 64 MB in all; a seeded sample of the rows beyond that)")
     args = ap.parse_args()
+    if args.cfg_steps is None:
+        args.cfg_steps = args.steps
+    if args.steps < 1 or args.cfg_steps < 1:
+        ap.error("--steps and --cfg-steps must be at least 1")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -75,6 +75,26 @@ def ctx_rows(hits):
     return np.stack([hits["lctx_off"], hits["lctx_len"], hits["rctx_off"], hits["rctx_len"]], axis=1).astype(np.int32)
 
 
+def gbrna_sample():
+    """(ids, defs, seq, rec_off) of the records sampled from the reference's test database
+    (tests/golden/gbrna/make_gbrna.py)."""
+    from rnamotif_b200 import fastn
+    with gzip.open(os.path.join(GOLDEN, "gbrna", "sample.fastn.gz"), "rb") as fh:
+        return fastn.parse_fastn(fh.read())
+
+
+def stream_md5(head, els, ctx=None):
+    """md5 of a candidate stream in enumeration order: per candidate rec comp szero, the
+    {off len mispairs mismatches} of every element and, if given, the context fields, as
+    int32.  The same digest of the reference's stream is stored in tests/golden/gbrna/."""
+    import hashlib
+    cols = [np.asarray(head, dtype=np.int32), np.asarray(els, dtype=np.int32)]
+    if ctx is not None:
+        cols.append(np.asarray(ctx, dtype=np.int32))
+    n = len(cols[0])
+    return hashlib.md5(np.ascontiguousarray(np.concatenate([c.reshape(n, -1) for c in cols], axis=1)).tobytes()).hexdigest()
+
+
 def assert_same_hits(a, b, what=""):
     ha, ea = hits_to_rows(a)
     hb, eb = hits_to_rows(b)

@@ -5,15 +5,19 @@ score/efn/printer on the host, search in libgpumotif) against
       runs pass the reference's test/*.chk goldens, oracle/check_goldens.sh), and
   (b) the reference binary itself (oracle/_ref/rnamotif), run side by side.
 Needs the prebuilt programs and test inputs under oracle/_ref/ and
-rnamotif_b200/host/_build/ (they travel with the snapshot)."""
+rnamotif_b200/host/_build/, built from the reference's sources; they skip without them.
+The tests at the end of the file check the library's side of the same command lines
+against the reference's stored outputs and need neither."""
 import hashlib
 import json
 import os
 import subprocess
 
+import numpy as np
 import pytest
 
 import helpers
+import shard
 
 pytestmark = pytest.mark.gpu
 
@@ -104,3 +108,134 @@ def test_fmt_option_chk_goldens(name):
     out = run(GPU_BIN, name, {"GPUMOTIF_FMT": "l"})
     with open(os.path.join(DATA, "test", name + ".chk"), "rb") as fh:
         assert out == fh.read(), f"{name}: differs from the reference's {name}.chk"
+
+
+# ---- the library on the device against the reference's stored outputs ----------------------
+# Records sampled from the reference's test database and what the reference printed over them
+# (tests/golden/gbrna/, make_gbrna.py): the digest of rnamotif_cand -O0's candidate stream for
+# every `make test` command line, the same of the candidates RM_score accepts, rnamotif's stdout
+# and that stdout through `rmfmt -l`.  They need no reference build.
+
+GBRNA = os.path.join(helpers.GOLDEN, "gbrna")
+STREAMS = json.load(open(os.path.join(GBRNA, "streams.json")))
+PURE_SCORE = {"score.1", "score.2", "mp.ends"}  # score programs that only filter (tests/test_score_prescreen.py)
+
+
+def _base(name):
+    return name[:-len(".strict")] if name.endswith(".strict") else name
+
+
+SCORED = [n for n in sorted(MD5) if helpers.load_score(_base(n)) is not None
+          and helpers.score_present(helpers.load_score(_base(n)))]
+
+
+@pytest.fixture(scope="module")
+def sample():
+    ids, defs, seq, off = helpers.gbrna_sample()
+    return seq, off
+
+
+def assert_stream(hits, want, what):
+    assert len(hits) == want["n"], f"{what}: {len(hits)} candidates, the reference {want['n']}"
+    if want["n"]:
+        head, els = helpers.hits_to_rows(hits)
+        got = helpers.stream_md5(head, els, helpers.ctx_rows(hits) if want["context"] else None)
+        assert got == want["md5"], f"{what}: candidate stream differs from the reference's"
+
+
+@pytest.mark.parametrize("name", sorted(MD5))
+def test_device_stream_equals_reference_on_gbrna_sample(name, sample):
+    """One upload of every sampled record: the candidate stream is the reference's, and it
+    is not empty for any command line that prints hits over the whole database."""
+    from rnamotif_b200 import gpumotif
+    want = STREAMS[name]
+    assert want["n"] > 0 or MD5[name]["hits"] == 0, f"{name}: the sample holds none of its hits"
+    ms = gpumotif.MotifSearch(helpers.load_plan(name))
+    assert_stream(ms.find_motif(*sample), want, name)
+    ms.close()
+
+
+@pytest.mark.parametrize("name", ["trna", "pk1", "qu+tr.strict", "getbest"])
+def test_device_small_uploads_equal_reference_stream(name, sample):
+    """The records over many uploads of one context (at most 30 knt each), the candidate
+    lists of the uploads concatenated in order, record numbers offset by each upload's first."""
+    from rnamotif_b200 import gpumotif
+    seq, off = sample
+    ms = gpumotif.MotifSearch(helpers.load_plan(name))
+    parts, a, n_rec = [], 0, len(off) - 1
+    while a < n_rec:
+        b = a + 1
+        while b < n_rec and off[b + 1] - off[a] <= 30000:
+            b += 1
+        ms.upload(seq[off[a]:off[b]], off[a:b + 1] - off[a])
+        h = ms.scan()
+        h["rec"] += np.uint32(a)
+        parts.append(h)
+        a = b
+    ms.close()
+    assert len(parts) > 5
+    assert_stream(np.concatenate(parts), STREAMS[name], name)
+
+
+@pytest.mark.parametrize("name", ["trna", "getbest", "pk1.strict"])
+def test_device_range_shards_merged_equal_reference_stream(name, sample):
+    """The batch cut into three ranges of start positions, one context each (on two GPUs
+    where there are), the candidate lists merged into enumeration order (tests/shard.py)."""
+    import torch
+    from rnamotif_b200 import gpumotif
+    seq, off = sample
+    devs = [0, 1, 0] if torch.cuda.device_count() > 1 else [0, 0, 0]
+    plan = helpers.load_plan(name)
+    parts = []
+    for dev, (lo, hi) in zip(devs, shard.shard_ranges(int(off[-1]), len(devs))):
+        ms = gpumotif.MotifSearch(plan, device=dev)
+        ms.upload(seq, off)
+        parts.append(ms.scan(lo, hi))
+        ms.close()
+    assert_stream(shard.merge_hits(parts), STREAMS[name], name)
+
+
+@pytest.mark.parametrize("name", SCORED)
+def test_device_prescreen_against_reference_verdicts_on_gbrna_sample(name, sample):
+    """The score section's pre-screen on the device: it never drops a candidate the reference
+    accepts, and for programs that only filter it keeps exactly the accepted ones."""
+    from rnamotif_b200 import gpumotif
+    want = STREAMS[name]
+    ms = gpumotif.MotifSearch(helpers.load_plan(name))
+    ms.set_score(helpers.load_score(_base(name)))
+    kept = ms.find_motif(*sample)
+    st = ms.stats()
+    ms.close()
+    assert len(kept) + st.n_score_rejected == want["n"]
+    if _base(name) in PURE_SCORE:
+        assert_stream(kept, want["accepted"], name + " (accepted)")
+    else:
+        assert len(kept) >= want["accepted"]["n"]
+
+
+@pytest.mark.parametrize("name", sorted(MD5))
+def test_gm_rmfmt_prints_what_rmfmt_l_printed(name, tmp_path):
+    """gm_rmfmt (GPUMOTIF_FMT=l): from rnamotif's stdout, what `rmfmt -l` printed from it."""
+    import ctypes as C
+    import ctypes.util
+    import gzip
+    from rnamotif_b200 import gpumotif
+
+    def stored(what):
+        with gzip.open(os.path.join(GBRNA, f"{name}.{what}.gz"), "rb") as fh:
+            return fh.read()
+
+    L = gpumotif.lib()
+    L.gm_rmfmt.argtypes = [C.c_char_p, C.c_size_t, C.c_int, C.c_void_p]
+    libc = C.CDLL(ctypes.util.find_library("c"))
+    libc.fopen.restype = C.c_void_p
+    libc.fopen.argtypes = [C.c_char_p, C.c_char_p]
+    libc.fclose.argtypes = [C.c_void_p]
+    raw = stored("rnamotif")
+    path = str(tmp_path / "fmt.out")
+    fp = libc.fopen(path.encode(), b"w")
+    assert fp
+    rc = L.gm_rmfmt(raw, len(raw), 1, fp)
+    assert libc.fclose(fp) == 0
+    assert rc == 0, L.gm_last_error()
+    assert open(path, "rb").read() == stored("rmfmt_l"), f"{name}: differs from `rmfmt -l`"

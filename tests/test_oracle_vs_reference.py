@@ -1,36 +1,22 @@
-"""CPU, needs oracle/_ref (built by `make -C oracle ref` where /root/reference is
-mounted; the built files travel with the snapshot): the oracle port against the
-instrumented REFERENCE binary, live, on real GenBank records
-(test/gbrna.111.0.fastn, first 400 records) -- upper case, IUPAC letters, N runs,
-records shorter than the motif.  Skipped where the reference build is absent;
-tests/golden/ holds the same comparison as committed fixtures."""
+"""CPU: the oracle port against the instrumented REFERENCE binary (rnamotif_cand -O0,
+oracle/cand_hook.c) on real GenBank records sampled from the reference's
+test/gbrna.111.0.fastn -- upper case, IUPAC letters, N runs, records shorter than
+the motif.  The records and the reference's candidate streams are stored under
+tests/golden/gbrna/ (make_gbrna.py regenerates them from a reference build)."""
 import os
-import subprocess
 
 import numpy as np
 import pytest
 
 from oracle import oracle_port
-from rnamotif_b200 import fastn
 import helpers
 
-REF = helpers.REF
-CAND = os.path.join(REF, "rnamotif_cand")
-DUMP = os.path.join(helpers.ROOT, "rnamotif_b200", "host", "_build", "rm_plan_dump")
-GB = os.path.join(REF, "data", "test", "gbrna.111.0.fastn")
-have = all(os.path.exists(p) for p in (CAND, DUMP, GB))
-pytestmark = pytest.mark.skipif(not have, reason="reference build (oracle/_ref) not present")
+GBRNA = os.path.join(helpers.GOLDEN, "gbrna")
 
 
 @pytest.fixture(scope="module")
-def gb400(tmp_path_factory):
-    data = open(GB, "rb").read()
-    idx = -1
-    for _ in range(401):
-        idx = data.find(b">", idx + 1)
-    p = tmp_path_factory.mktemp("gb") / "gb400.fastn"
-    p.write_bytes(data[:idx])
-    return str(p)
+def sample():
+    return helpers.gbrna_sample()
 
 
 @pytest.mark.parametrize("name,flags", [
@@ -38,22 +24,17 @@ def gb400(tmp_path_factory):
     ("trna.strict", ["-sh", "-context", "-Dctx_maxlen=5"]),
     ("score.1.strict", ["-sh", "-context", "-Dctx_maxlen=5"]),
 ])
-def test_oracle_port_equals_reference_binary(name, flags, gb400, tmp_path):
-    d = os.path.join(REF, "data", "test")
-    env = dict(os.environ, EFNDATA=os.path.join(REF, "data", "efndata"),
-               GM_PLAN_OUT=str(tmp_path / "p.plan"), GM_CAND_FILE=str(tmp_path / "c.txt"))
-    subprocess.run([DUMP, *flags, "-descr", name + ".descr"], cwd=d, env=env, check=True, capture_output=True)
-    subprocess.run([CAND, "-O0", *flags, "-descr", name + ".descr", gb400], cwd=d, env=env, check=True,
-                   capture_output=True)
-    plan = open(env["GM_PLAN_OUT"], "rb").read()
-    assert plan == helpers.load_plan(name), "committed plan fixture is stale"
-    ids, defs, seq, off = fastn.read_fastn(gb400)
-    both = bool(np.frombuffer(plan, dtype=np.int32, count=9)[8])
+def test_oracle_port_equals_reference_binary(name, flags, sample):
+    """`flags`: the reference's command line the stored stream was made with."""
+    plan = helpers.load_plan(name)
+    hdr = np.frombuffer(plan, dtype=np.int32, count=9)
+    assert bool(hdr[7]) == ("-sh" in flags), "plan and reference run disagree on -sh"
+    ids, defs, seq, off = sample
+    both = bool(hdr[8])
     hits, _ = oracle_port.scan_db(plan, seq, off, both)
     head, els = helpers.hits_to_rows(hits)
-    rows = [ln.split() for ln in open(env["GM_CAND_FILE"])]
+    ref = np.load(os.path.join(GBRNA, "cands.npz"))[name]
     nd = oracle_port.plan_n_descr(plan)
-    ref = np.array(rows, dtype=np.int64).reshape(len(rows), -1) if rows else np.zeros((0, 5 + 4 * nd), np.int64)
     assert len(head) == len(ref)
     if len(ref):
         assert (head == ref[:, :3]).all()

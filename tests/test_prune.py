@@ -6,6 +6,7 @@ returns), the expected verdicts from oracle/_ref/rnamotif | oracle/_ref/rmprune
 over the reference's test database.  Descriptors are those whose every
 candidate is printed (no REJECT in the score section), so that hit i of the
 candidate stream is hit i of rnamotif's output."""
+import gzip
 import os
 import subprocess
 
@@ -83,24 +84,25 @@ def locus(name: str) -> str:
     return parts[-2] if len(parts) >= 3 else name[:-1]
 
 
-@pytest.mark.skipif(not (have and os.path.exists(os.path.join(REF, "rmfmt"))), reason="oracle/_ref not built")
 @pytest.mark.parametrize("name", ["efn", "trna"])
 def test_order_matches_reference_rmfmt(name):
     """gm_order_hits against `rnamotif | rmfmt -l` (efn: real scores, every candidate
-    printed; trna: all scores equal).  sort(1) breaks ties in every key by comparing
-    whole lines, the library keeps enumeration order there, so the comparison is on
-    the key tuples of the two orders (identical sequences) and on the lines as a set."""
-    env = dict(os.environ, EFNDATA=os.path.join(REF, "data", "efndata"), LC_ALL="C")
-    raw = subprocess.run([os.path.join(REF, "rnamotif"), "-descr", name + ".descr", "gbrna.111.0.fastn"],
-                         cwd=DATA, env=env, capture_output=True, timeout=600, check=True).stdout
-    fmt = subprocess.run([os.path.join(REF, "rmfmt"), "-l"], input=raw, cwd=DATA, env=env, capture_output=True,
-                         timeout=600, check=True).stdout
+    printed; trna: all scores equal) over records sampled from the reference's
+    test database, both outputs stored under tests/golden/gbrna/.  sort(1) breaks ties
+    in every key by comparing whole lines, the library keeps enumeration order there,
+    so the comparison is on the key tuples of the two orders (identical sequences)
+    and on the lines as a set."""
+    gbrna = os.path.join(helpers.GOLDEN, "gbrna")
+    with gzip.open(os.path.join(gbrna, name + ".rnamotif.gz"), "rb") as fh:
+        raw = fh.read()
+    with gzip.open(os.path.join(gbrna, name + ".rmfmt_l.gz"), "rb") as fh:
+        fmt = fh.read()
     all_hits = hit_lines(raw)
     ref_rows = [l.split() for l in fmt.decode("latin-1").split("\n") if l and not l.startswith("#")]
     assert len(ref_rows) == len(all_hits)
 
     plan = helpers.load_plan(name)
-    ids, defs, seq, off = fastn.read_fastn(os.path.join(DATA, "gbrna.111.0.fastn"))
+    ids, defs, seq, off = helpers.gbrna_sample()
     cands, _ = oracle_port.scan_db(plan, seq, off, bool(gpumotif.plan_field(plan, 8)))
     assert len(cands) == len(all_hits)
     scores = np.array([float(h[1].split()[1]) for h in all_hits])
