@@ -122,6 +122,27 @@ int gm_db_upload_chars(gm_ctx *c, const char *seq, const int64_t *rec_off, int n
 int gm_db_upload_chars_hostpack(gm_ctx *c, const char *seq, const int64_t *rec_off, int n_rec);
 int gm_host_pack(const char *seq, int64_t n, uint8_t *packed, int n_threads);
 
+/* A batch of records in UCSC .2bit packing -- a quarter of a byte per nucleotide over
+ * PCIe and no host work.  Record r has rec_off[r+1] - rec_off[r] nucleotides; its
+ * bases start at dna[dna_off[r]], four to a byte, the first in the two most significant
+ * bits, T=0 C=1 A=2 G=3, every record on a byte of its own.  `dna` may be the bytes of
+ * a .2bit file as read from disk, with dna_off pointing past each record's header: the
+ * span from dna[dna_off[0]] to the end of the last record's bases is copied as it is,
+ * headers between records included.  nblk holds n_nblk half-open N ranges
+ * [nblk[2k], nblk[2k+1]) in rec_off coordinates (the file's N blocks shifted by their
+ * record's rec_off), sorted and disjoint (adjacent is fine); they read as n.  Mask
+ * blocks are not needed: the search folds case.  Refused, before the previous batch is
+ * touched: dna_off not ascending, a record's bytes overlapping the next record's or
+ * running past n_bytes, N ranges out of order, overlapping, ending before they start or
+ * outside [0, total), and every record table gm_db_upload_chars refuses.  Replaces the
+ * previous batch; cut into chunks and asynchronous like gm_db_upload_chars (`dna` must
+ * stay valid and unchanged until the next gm_scan has returned when it is pinned).  The
+ * codes on the device are exact (a, c, g, t, n), so gm_hit_windows and gm_db_get_chars
+ * work after it; gm_db_records gives hdr_off = NULL.  gm_scan_stats_t::h2d_bytes =
+ * the span + the record table + dna_off + the N ranges. */
+int gm_db_upload_2bit(gm_ctx *c, const uint8_t *dna, size_t n_bytes, const int64_t *dna_off,
+		      const int64_t *rec_off, int n_rec, const int64_t *nblk, int64_t n_nblk);
+
 /* Same, for characters that already live in device memory (a CUDA device
  * pointer, e.g. torch tensor storage). */
 int gm_db_set_device_chars(gm_ctx *c, const void *d_seq, const int64_t *rec_off, int n_rec);

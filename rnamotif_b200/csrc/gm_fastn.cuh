@@ -302,7 +302,11 @@ __global__ void __launch_bounds__(256) gm_fastn_emit(const uint8_t *__restrict__
 // complementary strand, mk_rcmp's mapping (src/rnamot.c:193-216: a<->t, c<->g,
 // anything else -> n).  Window i covers strand offsets [szero - lead,
 // szero - lead + wlen); positions outside the record read as 0.
-__global__ void __launch_bounds__(128) gm_window_kernel(const uint8_t *__restrict__ chars,
+// CODES: `src` is not characters but the 4-bit codes (nucleotide g in nibble g & 1 of byte
+// g >> 1), read back through the inverse of the code table -- exact after gm_db_upload_2bit,
+// whose codes are a, c, g, t and n only.
+template <bool CODES>
+__global__ void __launch_bounds__(128) gm_window_kernel(const uint8_t *__restrict__ src,
 	const int64_t *__restrict__ rec_off, const uint32_t *__restrict__ hits, unsigned long long n_hits,
 	int stride_words, int lead, int wlen, uint8_t *__restrict__ win)
 {
@@ -316,9 +320,14 @@ __global__ void __launch_bounds__(128) gm_window_kernel(const uint8_t *__restric
 			const int p = szero - lead + j;
 			unsigned ch = 0;
 			if (p >= 0 && p < slen) {
-				ch = chars[r0 + (comp ? slen - 1 - p : p)] | 0x20;
-				if (ch == 'u')
-					ch = 't';
+				const int64_t g = r0 + (comp ? slen - 1 - p : p);
+				if (CODES) {
+					ch = (unsigned char)"?acmgrsvtwyhkdbn"[(src[g >> 1] >> (4 * (g & 1))) & 15];
+				} else {
+					ch = src[g] | 0x20;
+					if (ch == 'u')
+						ch = 't';
+				}
 				if (comp)
 					ch = ch == 'a' ? 't' : ch == 't' ? 'a' : ch == 'c' ? 'g' : ch == 'g' ? 'c' : 'n';
 			}

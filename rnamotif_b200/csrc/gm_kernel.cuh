@@ -2,6 +2,7 @@
 //
 //   gm_pack_kernel     chars (what FN_fgetseq leaves, src/dbutil.c:105-111)
 //                      -> 4-bit IUPAC codes, two per byte
+//   gm_unpack2_kernel  UCSC .2bit bytes + N ranges -> the same 4-bit codes
 //   gm_search_kernel   persistent CTAs; each takes tiles of consecutive start
 //                      positions from a global counter, stages the packed
 //                      tile + halo into shared memory with one TMA bulk copy
@@ -16,6 +17,7 @@
 #include <stdint.h>
 #include "gm_search.cuh"
 #include "gm_score.h"
+#include "gm_twobit.h"
 
 namespace gm {
 
@@ -97,6 +99,112 @@ __global__ void __launch_bounds__(256) gm_pack_kernel(const uint8_t *__restrict_
 		}
 		// packed is allocated rounded up to 16 nucleotides
 		*reinterpret_cast<uint2 *>(packed + (i >> 1)) = make_uint2(out[0], out[1]);
+	}
+}
+
+// last r in [lo, hi] with a[r] <= x (a ascending, a[lo] <= x)
+__device__ __forceinline__ int64_t last_le(const int64_t *__restrict__ a, int64_t lo, int64_t hi, int64_t x)
+{
+	while (lo < hi) {
+		const int64_t mid = (lo + hi + 1) >> 1;
+		if (a[mid] <= x)
+			lo = mid;
+		else
+			hi = mid - 1;
+	}
+	return lo;
+}
+
+// first k in [lo, hi) with a[2k] >= x (a[0], a[2], ... ascending), hi if none
+__device__ __forceinline__ int64_t first_ge2(const int64_t *__restrict__ a, int64_t lo, int64_t hi, int64_t x)
+{
+	while (lo < hi) {
+		const int64_t mid = (lo + hi) >> 1;
+		if (a[2 * mid] < x)
+			lo = mid + 1;
+		else
+			hi = mid;
+	}
+	return lo;
+}
+
+// gm_db_upload_2bit: UCSC .2bit bytes -> the 4-bit codes gm_pack_kernel writes, for nucleotides
+// [g0, g0 + n) of the concatenation (g0 a multiple of 16; nucleotides past g0 + n, the end of the
+// database, read 0).  Record r's bases start at src[dna_off[r]], first base in the two most
+// significant bits of its byte.  nblk holds n_nblk sorted, disjoint half-open N ranges
+// [nblk[2k], nblk[2k+1]) in concatenation coordinates: those positions read n (15).
+// One thread per 16-nucleotide group, one 8-byte store.  A block takes 256 consecutive groups and
+// first brackets the records and N ranges they can touch, so the threads' own binary searches run
+// inside that bracket (usually one record and no N range: nothing to search).  Fast path: the group
+// lies in one record and touches no N range -- the five source bytes that cover it, aligned with a
+// funnel shift (the group starts at any phase of its record's bytes) and expanded in a register
+// (gm_twobit.h).  Otherwise nucleotide by nucleotide.
+__global__ void __launch_bounds__(256) gm_unpack2_kernel(const uint8_t *__restrict__ src,
+	const int64_t *__restrict__ dna_off, const int64_t *__restrict__ rec_off, int n_rec,
+	const int64_t *__restrict__ nblk, int64_t n_nblk, int64_t g0, int64_t n, uint8_t *__restrict__ packed)
+{
+	__shared__ int64_t br[4]; // records of the block's first and last nucleotide; N ranges [br[2], br[3]) touch it
+	const int64_t span = 256 * 16, end = g0 + n;
+	for (int64_t b0 = g0 + (int64_t)blockIdx.x * span; b0 < end; b0 += (int64_t)gridDim.x * span) {
+		const int64_t b1 = min(b0 + span, end);
+		if (threadIdx.x == 0)
+			br[0] = last_le(rec_off, 0, n_rec - 1, b0);
+		else if (threadIdx.x == 1)
+			br[1] = last_le(rec_off, 0, n_rec - 1, b1 - 1);
+		else if (threadIdx.x == 2) {
+			// the first range that ends after b0 (the ends ascend too: the ranges are disjoint)
+			int64_t lo = 0, hi = n_nblk;
+			while (lo < hi) {
+				const int64_t mid = (lo + hi) >> 1;
+				if (nblk[2 * mid + 1] <= b0)
+					lo = mid + 1;
+				else
+					hi = mid;
+			}
+			br[2] = lo;
+		} else if (threadIdx.x == 3)
+			br[3] = first_ge2(nblk, 0, n_nblk, b1);
+		__syncthreads();
+		const int64_t r_lo = br[0], r_hi = br[1], k_lo = br[2], k_hi = br[3];
+		const int64_t gg = b0 + (int64_t)threadIdx.x * 16;
+		if (gg < b1) {
+			const int64_t r = last_le(rec_off, r_lo, r_hi, gg);
+			bool fast = gg + 16 <= rec_off[r + 1] && gg + 16 <= end;
+			if (fast && k_lo < k_hi) {
+				// the last range that starts before the group's end has the largest end of those that do
+				const int64_t k = first_ge2(nblk, k_lo, k_hi, gg + 16) - 1;
+				fast = k < k_lo || nblk[2 * k + 1] <= gg;
+			}
+			uint32_t lo = 0, hi = 0;
+			if (fast) {
+				const int64_t q = gg - rec_off[r];
+				const int phase = (int)(q & 3);
+				const uint8_t *s = src + dna_off[r] + (q >> 2);
+				const uint32_t be4 = ((uint32_t)s[0] << 24) | ((uint32_t)s[1] << 16) | ((uint32_t)s[2] << 8) | s[3];
+				const uint32_t b4 = phase ? s[4] : 0; // phase 0: the group ends with byte 3, which may be the record's last
+				twobit_expand16(twobit_window(be4, b4, phase), lo, hi);
+			} else {
+				for (int j = 0; j < 16; j++) {
+					const int64_t g = gg + j;
+					if (g >= end)
+						break;
+					const int64_t rr = last_le(rec_off, r_lo, r_hi, g);
+					const int64_t q = g - rec_off[rr];
+					uint32_t code = twobit_code4((src[dna_off[rr] + (q >> 2)] >> (6 - 2 * (int)(q & 3))) & 3);
+					if (k_lo < k_hi) {
+						const int64_t k = first_ge2(nblk, k_lo, k_hi, g + 1) - 1;
+						if (k >= k_lo && g < nblk[2 * k + 1])
+							code = 15;
+					}
+					if (j < 8)
+						lo |= code << (4 * j);
+					else
+						hi |= code << (4 * (j - 8));
+				}
+			}
+			*reinterpret_cast<uint2 *>(packed + (gg >> 1)) = make_uint2(lo, hi);
+		}
+		__syncthreads(); // br is rewritten by the next round
 	}
 }
 

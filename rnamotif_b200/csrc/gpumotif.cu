@@ -115,6 +115,12 @@ struct gm_ctx {
 	size_t fsum_cap, fstart_cap;
 	std::vector<int64_t> hdr_off;
 	const uint8_t *d_seq_chars; // the uploaded characters as they sit on the device (window gather)
+	// 2-bit upload (gm_db_upload_2bit): its bytes go to d_chars; per-record byte offsets into them,
+	// then the N ranges, on the device (d_tb) and on the host (tb)
+	int64_t *d_tb;
+	size_t tb_cap;           // bytes
+	std::vector<int64_t> tb;
+	bool codes_exact;        // the last upload was 2-bit: d_packed holds only a, c, g, t, n, and they decode to characters
 	// windows around the candidates (gm_hit_windows)
 	uint8_t *d_win, *h_win;
 	size_t win_cap, h_win_cap;
@@ -1150,6 +1156,9 @@ extern "C" int gm_ctx_create(gm_ctx **out, const gm_plan_t *plan, int device)
 	c->d_fsum = c->d_fstart = NULL;
 	c->text_cap = c->hdr_cap = c->fsum_cap = c->fstart_cap = 0;
 	c->d_seq_chars = NULL;
+	c->d_tb = NULL;
+	c->tb_cap = 0;
+	c->codes_exact = false;
 	c->d_win = c->h_win = NULL;
 	c->win_cap = c->h_win_cap = 0;
 	c->d_rec_off = NULL;
@@ -1296,6 +1305,7 @@ extern "C" void gm_ctx_destroy(gm_ctx *c)
 	cudaFree(c->d_chars);
 	cudaFree(c->d_text);
 	cudaFree(c->d_hdr_off);
+	cudaFree(c->d_tb);
 	cudaFree(c->d_fsum);
 	cudaFree(c->d_fstart);
 	cudaFree(c->d_win);
@@ -1382,7 +1392,7 @@ static int ensure(void **p, size_t *cap, size_t need)
 	return 0;
 }
 
-static int set_records(gm_ctx *c, const int64_t *rec_off, int n_rec)
+static int check_records(const int64_t *rec_off, int n_rec)
 {
 	if (n_rec < 0 || rec_off == NULL)
 		return fail("bad record table");
@@ -1394,6 +1404,13 @@ static int set_records(gm_ctx *c, const int64_t *rec_off, int n_rec)
 		if (rec_off[r + 1] - rec_off[r] > 0x7ffffff0ll)
 			return fail("record %d longer than 2^31", r);
 	}
+	return 0;
+}
+
+static int set_records(gm_ctx *c, const int64_t *rec_off, int n_rec)
+{
+	if (check_records(rec_off, n_rec))
+		return -1;
 	c->rec_off.assign(rec_off, rec_off + n_rec + 1);
 	c->hdr_off.clear();
 	c->total_nt = rec_off[n_rec];
@@ -1439,6 +1456,45 @@ static int wait_published(gm_ctx *c, int i)
 	return 0;
 }
 
+// Cut an upload of n nucleotides into the chunks gm_scan_launch streams in: chunk_ev[i] is to fire
+// when nucleotides [0, chunk_end[i]) are packed.  A chunk is at least floor_nt (GPUMOTIF_CHUNK_NT lowers
+// the floor: tests run the chunk-streamed scan on small inputs) and a multiple of `align` nucleotides,
+// and there are at most n_target chunks.  Fills chunk_end and makes sure chunk_ev (and, with `copies`,
+// cp_ev: chunk i has arrived) hold an event per chunk; *chunk = the chunk size.
+static int cut_chunks(gm_ctx *c, int64_t n, int64_t floor_nt, int n_target, int64_t align, bool copies, int64_t *chunk)
+{
+	if (getenv("GPUMOTIF_CHUNK_NT") != NULL && atoll(getenv("GPUMOTIF_CHUNK_NT")) >= 4096)
+		floor_nt = atoll(getenv("GPUMOTIF_CHUNK_NT"));
+	int64_t ch = std::max<int64_t>(floor_nt, (n + n_target - 1) / n_target);
+	ch = (ch + align - 1) / align * align;
+	const int n_chunks = n > 0 ? (int)((n + ch - 1) / ch) : 0;
+	while ((int)c->chunk_ev.size() < n_chunks) {
+		cudaEvent_t e;
+		CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+		c->chunk_ev.push_back(e);
+	}
+	while (copies && (int)c->cp_ev.size() < n_chunks) {
+		cudaEvent_t e;
+		CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+		c->cp_ev.push_back(e);
+	}
+	c->chunk_end.clear();
+	for (int i = 0; i < n_chunks; i++)
+		c->chunk_end.push_back(std::min<int64_t>(n, (int64_t)(i + 1) * ch));
+	*chunk = ch;
+	return 0;
+}
+
+// Chunks of an upload packed on the device: at least 64 Mnt, at most 16 (every chunk costs a kernel
+// launch with its own ramp and tail; GPUMOTIF_CHUNKS lowers the count), a multiple of 16 nucleotides.
+static int cut_device_chunks(gm_ctx *c, int64_t n, bool copies, int64_t *chunk)
+{
+	int n_target = 16; // (trna, 1 Gnt: 72.3 G strand-nt/s end to end with 16 chunks, 69.2 with 8)
+	if (getenv("GPUMOTIF_CHUNKS") != NULL)
+		n_target = std::max(1, std::min(16, atoi(getenv("GPUMOTIF_CHUNKS"))));
+	return cut_chunks(c, n, (int64_t)64 << 20, n_target, 16, copies, chunk);
+}
+
 // Enqueue the upload on copy_stream in chunks: [H2D copy of chunk i,] pack chunk i,
 // record chunk_ev[i].  Returns without waiting.
 static int upload_chunks(gm_ctx *c, const uint8_t *h_chars, const uint8_t *d_src, bool mark_start = true)
@@ -1450,38 +1506,20 @@ static int upload_chunks(gm_ctx *c, const uint8_t *h_chars, const uint8_t *d_src
 		return -1;
 	if (h_chars != NULL && ensure((void **)&c->d_chars, &c->chars_cap, (size_t)n + 64))
 		return -1;
-	// chunk size: at least 64 Mnt, at most 16 chunks (every chunk costs a kernel
-	// launch with its own ramp and tail), a multiple of 16 nucleotides
-	// (GPUMOTIF_CHUNK_NT lowers the 64 Mnt floor: tests run the chunk-streamed scan on small inputs)
-	int64_t floor_nt = (int64_t)64 << 20;
-	if (getenv("GPUMOTIF_CHUNK_NT") != NULL && atoll(getenv("GPUMOTIF_CHUNK_NT")) >= 4096)
-		floor_nt = atoll(getenv("GPUMOTIF_CHUNK_NT"));
-	int n_target = 16; // (trna, 1 Gnt: 72.3 G strand-nt/s end to end with 16 chunks, 69.2 with 8)
-	if (getenv("GPUMOTIF_CHUNKS") != NULL)
-		n_target = std::max(1, std::min(16, atoi(getenv("GPUMOTIF_CHUNKS"))));
-	int64_t chunk = std::max<int64_t>(floor_nt, (n + n_target - 1) / n_target);
-	chunk = (chunk + 15) & ~(int64_t)15;
-	const int n_chunks = n > 0 ? (int)((n + chunk - 1) / chunk) : 0;
-	while ((int)c->chunk_ev.size() < n_chunks) {
-		cudaEvent_t e;
-		CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-		c->chunk_ev.push_back(e);
-	}
-	c->chunk_end.clear();
+	int64_t chunk;
+	if (cut_device_chunks(c, n, h_chars != NULL, &chunk))
+		return -1;
+	const int n_chunks = (int)c->chunk_end.size();
 	c->up_published = -1;
 	c->d_seq_chars = h_chars != NULL ? c->d_chars : d_src;
+	c->codes_exact = false;
 	if (mark_start)
 		CU(cudaEventRecord(c->up_ev[0], c->copy_stream));
-	while (h_chars != NULL && (int)c->cp_ev.size() < n_chunks) {
-		cudaEvent_t e;
-		CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-		c->cp_ev.push_back(e);
-	}
 	// from the host: copies back to back on the copy stream, pack kernels on the pack stream behind
 	// each chunk's copy; on the device: pack kernels on the copy stream
 	cudaStream_t ps = h_chars != NULL ? c->pack_stream : c->copy_stream;
 	for (int i = 0; i < n_chunks; i++) {
-		const int64_t o = (int64_t)i * chunk, len = std::min<int64_t>(chunk, n - o);
+		const int64_t o = (int64_t)i * chunk, len = c->chunk_end[i] - o;
 		const uint8_t *src = d_src;
 		if (h_chars != NULL) {
 			CU(cudaMemcpyAsync(c->d_chars + o, h_chars + o, (size_t)len, cudaMemcpyHostToDevice, c->copy_stream));
@@ -1494,7 +1532,6 @@ static int upload_chunks(gm_ctx *c, const uint8_t *h_chars, const uint8_t *d_src
 		gm_pack_kernel<<<blocks, 256, 0, ps>>>(src + o, c->d_packed + (o >> 1), len);
 		CU(cudaGetLastError());
 		CU(cudaEventRecord(c->chunk_ev[i], ps));
-		c->chunk_end.push_back(o + len);
 	}
 	CU(cudaEventRecord(c->up_ev[1], c->copy_stream));
 	c->upload_fresh = true;
@@ -1607,28 +1644,6 @@ extern "C" int gm_db_upload_chars_hostpack(gm_ctx *c, const char *seq, const int
 	const size_t pbytes = (size_t)(((n + 15) / 16) * 8) + 1024;
 	if (ensure((void **)&c->d_packed, &c->packed_cap, pbytes))
 		return -1;
-	// at most 16 chunks (gm_scan_launch streams up to 16 in) of at least 16 Mnt, a multiple of
-	// 4096 nucleotides; GPUMOTIF_CHUNK_NT lowers the floor (tests)
-	int64_t floor_nt = (int64_t)16 << 20;
-	if (getenv("GPUMOTIF_CHUNK_NT") != NULL && atoll(getenv("GPUMOTIF_CHUNK_NT")) >= 4096)
-		floor_nt = atoll(getenv("GPUMOTIF_CHUNK_NT"));
-	int64_t chunk = std::max<int64_t>(floor_nt, (n + 15) / 16);
-	chunk = (chunk + 4095) & ~(int64_t)4095;
-	const int n_chunks = n > 0 ? (int)((n + chunk - 1) / chunk) : 0;
-	const size_t slot_need = (size_t)(chunk >> 1) + 64;
-	if (c->slot_cap < slot_need) {
-		for (int i = 0; i < GM_PACK_SLOTS; i++) {
-			cudaFreeHost(c->h_slot[i]);
-			c->h_slot[i] = NULL;
-		}
-		c->slot_cap = 0;
-		for (int i = 0; i < GM_PACK_SLOTS; i++)
-			CU(cudaMallocHost((void **)&c->h_slot[i], slot_need));
-		c->slot_cap = slot_need;
-	}
-	for (int i = 0; i < GM_PACK_SLOTS; i++)
-		if (c->slot_ev[i] == NULL)
-			CU(cudaEventCreateWithFlags(&c->slot_ev[i], cudaEventDisableTiming));
 	if (c->team == NULL)
 		c->team = new PackTeam(host_pack_default_threads());
 	// share of every chunk packed on the host: all of it from pageable memory (a DMA from
@@ -1647,20 +1662,28 @@ extern "C" int gm_db_upload_chars_hostpack(gm_ctx *c, const char *seq, const int
 	}
 	if (frac < 1.0 && ensure((void **)&c->d_chars, &c->chars_cap, (size_t)n + 64))
 		return -1;
-	while (frac < 1.0 && (int)c->cp_ev.size() < n_chunks) {
-		cudaEvent_t e;
-		CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-		c->cp_ev.push_back(e);
+	// at most 16 chunks (gm_scan_launch streams up to 16 in) of at least 16 Mnt, a multiple of
+	// 4096 nucleotides
+	int64_t chunk;
+	if (cut_chunks(c, n, (int64_t)16 << 20, 16, 4096, frac < 1.0, &chunk))
+		return -1;
+	const int n_chunks = (int)c->chunk_end.size();
+	const size_t slot_need = (size_t)(chunk >> 1) + 64;
+	if (c->slot_cap < slot_need) {
+		for (int i = 0; i < GM_PACK_SLOTS; i++) {
+			cudaFreeHost(c->h_slot[i]);
+			c->h_slot[i] = NULL;
+		}
+		c->slot_cap = 0;
+		for (int i = 0; i < GM_PACK_SLOTS; i++)
+			CU(cudaMallocHost((void **)&c->h_slot[i], slot_need));
+		c->slot_cap = slot_need;
 	}
-	while ((int)c->chunk_ev.size() < n_chunks) {
-		cudaEvent_t e;
-		CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-		c->chunk_ev.push_back(e);
-	}
-	c->chunk_end.clear();
-	for (int i = 0; i < n_chunks; i++)
-		c->chunk_end.push_back(std::min<int64_t>(n, (int64_t)(i + 1) * chunk));
+	for (int i = 0; i < GM_PACK_SLOTS; i++)
+		if (c->slot_ev[i] == NULL)
+			CU(cudaEventCreateWithFlags(&c->slot_ev[i], cudaEventDisableTiming));
 	c->d_seq_chars = NULL;
+	c->codes_exact = false;
 	c->up_published = 0;
 	c->up_err[0] = 0;
 	CU(cudaEventRecord(c->up_ev[0], c->copy_stream));
@@ -1702,6 +1725,113 @@ extern "C" int gm_db_set_device_chars(gm_ctx *c, const void *d_seq, const int64_
 	if (upload_chunks(c, NULL, (const uint8_t *)d_seq))
 		return -1;
 	c->stats.h2d_bytes = (uint64_t)(n_rec + 1) * 8;
+	return 0;
+}
+
+// UCSC .2bit input: the byte span from the first record's bases to the end of the last one goes
+// over as it is, in chunks cut like gm_db_upload_chars's; chunk i copies from where chunk i-1's copy
+// ended to the byte that holds its last nucleotide, and gm_unpack2_kernel expands it behind that
+// copy, so a byte two chunks share is written by one copy and read after it.
+extern "C" int gm_db_upload_2bit(gm_ctx *c, const uint8_t *dna, size_t n_bytes, const int64_t *dna_off,
+				 const int64_t *rec_off, int n_rec, const int64_t *nblk, int64_t n_nblk)
+{
+	if (c == NULL)
+		return fail("ctx is NULL");
+	if (c->pending)
+		return fail("a scan is in flight");
+	// everything is checked before the previous batch is touched
+	if (check_records(rec_off, n_rec))
+		return -1;
+	const int64_t n = rec_off[n_rec];
+	if (n_rec > 0 && dna_off == NULL)
+		return fail("dna_off is NULL");
+	if (n_nblk < 0 || (n_nblk > 0 && nblk == NULL))
+		return fail("bad N range table");
+	int64_t b_end = 0; // end of the previous record's bytes
+	for (int r = 0; r < n_rec; r++) {
+		const int64_t nb = (rec_off[r + 1] - rec_off[r] + 3) / 4;
+		if (dna_off[r] < 0)
+			return fail("dna_off[%d] = %lld is negative", r, (long long)dna_off[r]);
+		if (r > 0 && dna_off[r] < b_end)
+			return fail("dna_off[%d] = %lld: not ascending, or the previous record's bytes run into record %d's", r,
+				    (long long)dna_off[r], r);
+		if ((uint64_t)(dna_off[r] + nb) > (uint64_t)n_bytes)
+			return fail("record %d's bytes [%lld, %lld) run past the %zu bytes of dna", r, (long long)dna_off[r],
+				    (long long)(dna_off[r] + nb), n_bytes);
+		b_end = dna_off[r] + nb;
+	}
+	if (n > 0 && dna == NULL)
+		return fail("dna is NULL");
+	for (int64_t k = 0; k < n_nblk; k++) {
+		const int64_t s = nblk[2 * k], e = nblk[2 * k + 1];
+		if (e < s)
+			return fail("N range %lld [%lld, %lld) ends before it starts", (long long)k, (long long)s, (long long)e);
+		if (s < 0 || e > n)
+			return fail("N range %lld [%lld, %lld) outside the %lld nucleotides", (long long)k, (long long)s, (long long)e,
+				    (long long)n);
+		if (k > 0 && s < nblk[2 * k - 1])
+			return fail("N range %lld [%lld, %lld) is out of order or overlaps the one before", (long long)k, (long long)s,
+				    (long long)e);
+	}
+	if (join_uploader(c))
+		return -1;
+	CU(cudaSetDevice(c->device));
+	if (sync_uploads(c)) // the previous upload's staging is reused
+		return -1;
+	if (set_records(c, rec_off, n_rec))
+		return -1;
+	// the span copied: [b0, b_end) of dna, record r's bases at dna_off[r] - b0 on the device
+	const int64_t b0 = n_rec > 0 ? dna_off[0] : 0;
+	const int64_t span = b_end - b0;
+	c->tb.resize((size_t)n_rec + 2 * (size_t)n_nblk);
+	for (int r = 0; r < n_rec; r++)
+		c->tb[r] = dna_off[r] - b0;
+	if (n_nblk > 0)
+		memcpy(c->tb.data() + n_rec, nblk, (size_t)n_nblk * 2 * sizeof(int64_t));
+	const size_t tb_bytes = c->tb.size() * sizeof(int64_t);
+	const size_t pbytes = (size_t)(((n + 15) / 16) * 8) + 1024; // slack: kernels read whole 16-byte groups past the end
+	if (ensure((void **)&c->d_packed, &c->packed_cap, pbytes) || ensure((void **)&c->d_chars, &c->chars_cap, (size_t)span + 64) ||
+	    ensure((void **)&c->d_tb, &c->tb_cap, tb_bytes + 16))
+		return -1;
+	int64_t chunk;
+	if (cut_device_chunks(c, n, true, &chunk))
+		return -1;
+	const int n_chunks = (int)c->chunk_end.size();
+	c->up_published = -1;
+	c->d_seq_chars = NULL;
+	c->codes_exact = true;
+	CU(cudaEventRecord(c->up_ev[0], c->copy_stream));
+	if (tb_bytes > 0)
+		CU(cudaMemcpyAsync(c->d_tb, c->tb.data(), tb_bytes, cudaMemcpyHostToDevice, c->copy_stream));
+	const int64_t *d_dna_off = c->d_tb, *d_nblk = c->d_tb + n_rec;
+	int64_t copied = 0; // bytes of the span on the device (or on their way) so far
+	int r = 0;          // record of the current chunk's last nucleotide
+	for (int i = 0; i < n_chunks; i++) {
+		const int64_t o = (int64_t)i * chunk, len = c->chunk_end[i] - o;
+		int64_t upto = span; // the last chunk takes the rest of the span
+		if (i < n_chunks - 1) {
+			const int64_t g = c->chunk_end[i] - 1;
+			while (rec_off[r + 1] <= g)
+				r++;
+			upto = c->tb[r] + (g - rec_off[r]) / 4 + 1;
+		}
+		if (upto > copied)
+			CU(cudaMemcpyAsync(c->d_chars + copied, dna + b0 + copied, (size_t)(upto - copied), cudaMemcpyHostToDevice,
+					   c->copy_stream));
+		copied = std::max(copied, upto);
+		CU(cudaEventRecord(c->cp_ev[i], c->copy_stream));
+		CU(cudaStreamWaitEvent(c->pack_stream, c->cp_ev[i], 0));
+		const int64_t groups = (len + 15) / 16;
+		const int blocks = (int)std::min<int64_t>((groups + 255) / 256, (int64_t)c->n_sm * 16);
+		gm_unpack2_kernel<<<blocks, 256, 0, c->pack_stream>>>(c->d_chars, d_dna_off, c->d_rec_off, n_rec, d_nblk, n_nblk, o, len,
+								      c->d_packed);
+		CU(cudaGetLastError());
+		CU(cudaEventRecord(c->chunk_ev[i], c->pack_stream));
+	}
+	CU(cudaEventRecord(c->up_ev[1], c->copy_stream));
+	c->upload_fresh = true;
+	// bytes over the link: the span, the record table, dna_off and the N ranges
+	c->stats.h2d_bytes = (uint64_t)span + (uint64_t)(n_rec + 1) * 8 + (uint64_t)tb_bytes;
 	return 0;
 }
 
@@ -1805,7 +1935,7 @@ extern "C" int gm_db_get_chars(gm_ctx *c, int64_t off, int64_t n, char *out)
 {
 	if (c == NULL || out == NULL || off < 0 || n < 0)
 		return fail("bad argument");
-	if (c->d_seq_chars == NULL)
+	if (c->d_seq_chars == NULL && !c->codes_exact)
 		return fail(c->up_published >= 0 ? "the device holds no characters after gm_db_upload_chars_hostpack (the caller has them)"
 					   : "no database uploaded");
 	if (off + n > c->total_nt)
@@ -1814,6 +1944,19 @@ extern "C" int gm_db_get_chars(gm_ctx *c, int64_t off, int64_t n, char *out)
 	CU(cudaSetDevice(c->device));
 	if (sync_uploads(c))
 		return -1;
+	if (c->codes_exact) {
+		// after gm_db_upload_2bit: the 4-bit codes back, decoded here (a, c, g, t and n are all they hold)
+		if (n == 0)
+			return 0;
+		const int64_t b0 = off >> 1, b1 = (off + n + 1) >> 1;
+		std::vector<uint8_t> pk((size_t)(b1 - b0));
+		CU(cudaMemcpy(pk.data(), c->d_packed + b0, pk.size(), cudaMemcpyDeviceToHost));
+		for (int64_t i = 0; i < n; i++) {
+			const int64_t g = off + i;
+			out[i] = "?acmgrsvtwyhkdbn"[(pk[(size_t)((g >> 1) - b0)] >> (4 * (g & 1))) & 15];
+		}
+		return 0;
+	}
 	if (n > 0)
 		CU(cudaMemcpy(out, c->d_seq_chars + off, (size_t)n, cudaMemcpyDeviceToHost));
 	for (int64_t i = 0; i < n; i++) {
@@ -2261,7 +2404,7 @@ extern "C" int gm_hit_windows(gm_ctx *c, int lead, int trail, const char **win, 
 		return fail("bad argument");
 	if (c->pending)
 		return fail("a scan is in flight");
-	if (c->d_seq_chars == NULL)
+	if (c->d_seq_chars == NULL && !c->codes_exact)
 		return fail(c->up_published >= 0 ? "the device holds no characters after gm_db_upload_chars_hostpack (the caller has them)"
 					   : "no database uploaded");
 	CU(cudaSetDevice(c->device));
@@ -2282,8 +2425,14 @@ extern "C" int gm_hit_windows(gm_ctx *c, int lead, int trail, const char **win, 
 	}
 	if (n_dev > 0) {
 		const int blocks = (int)std::min<size_t>(n_dev, (size_t)c->n_sm * 32);
-		gm_window_kernel<<<blocks, 128, 0, c->stream>>>(c->d_seq_chars, c->d_rec_off, c->dev_sorted ? c->d_sorted : c->d_hits, n_dev, c->stride_words,
-			lead, wlen, c->d_win);
+		// after a 2-bit upload the windows are decoded from the 4-bit codes
+		const uint32_t *h = c->dev_sorted ? c->d_sorted : c->d_hits;
+		if (c->codes_exact)
+			gm_window_kernel<true><<<blocks, 128, 0, c->stream>>>(c->d_packed, c->d_rec_off, h, n_dev, c->stride_words, lead, wlen,
+									      c->d_win);
+		else
+			gm_window_kernel<false><<<blocks, 128, 0, c->stream>>>(c->d_seq_chars, c->d_rec_off, h, n_dev, c->stride_words, lead,
+									       wlen, c->d_win);
 		CU(cudaGetLastError());
 		CU(cudaMemcpyAsync(c->h_win, c->d_win, bytes, cudaMemcpyDeviceToHost, c->stream));
 		CU(cudaStreamSynchronize(c->stream));

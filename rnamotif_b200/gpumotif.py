@@ -37,6 +37,7 @@ _lib = None
 
 EXPORTS = ["gm_last_error", "gm_version", "gm_device_count", "gm_host_alloc", "gm_host_free", "gm_ctx_create", "gm_ctx_destroy",
            "gm_plan_check", "gm_plan_describe", "gm_db_upload_chars", "gm_db_upload_chars_hostpack", "gm_host_pack", "gm_db_set_device_chars", "gm_db_upload_fastn",
+           "gm_db_upload_2bit",
            "gm_db_records", "gm_db_get_chars", "gm_db_total_nt", "gm_hit_windows",
            "gm_scan", "gm_scan_launch", "gm_scan_finish", "gm_hits", "gm_stats",
            "gm_set_hit_capacity", "gm_set_tile", "gm_stream", "gm_prune_hits", "gm_order_hits",
@@ -62,6 +63,8 @@ def lib():
         L.gm_host_pack.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_int]
         L.gm_db_set_device_chars.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
         L.gm_db_upload_fastn.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
+        L.gm_db_upload_2bit.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
+                                        C.c_int64]
         L.gm_db_records.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_int)]
         L.gm_hit_windows.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]
         L.gm_db_get_chars.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p]
@@ -235,6 +238,25 @@ class MotifSearch:
 
     def upload_fastn_ptr(self, host_ptr: int, n_bytes: int):
         self._ck(lib().gm_db_upload_fastn(self._ctx, host_ptr, n_bytes), "gm_db_upload_fastn")
+
+    def upload_2bit(self, tb, first: int = 0, last: int | None = None):
+        """gm_db_upload_2bit: records [first, last) of a parsed .2bit file (twobit.read_2bit),
+        its bytes passed as they are -- a quarter of a byte per nucleotide over PCIe.  Read
+        the file into pinned memory (read_2bit's `out`) for an asynchronous upload."""
+        rec_off, dna_off, nblk = tb.tables(first, last)
+        data = np.ascontiguousarray(tb.data, dtype=np.uint8)
+        self._keep = data  # the upload is asynchronous: keep the buffer alive until the next scan
+        self.upload_2bit_ptr(data.ctypes.data, data.size, dna_off, rec_off, nblk)
+
+    def upload_2bit_ptr(self, host_ptr: int, n_bytes: int, dna_off, rec_off, nblk=None):
+        """gm_db_upload_2bit from a raw host pointer: record r's packed bases at byte dna_off[r],
+        nblk = flat [start, end) N ranges in rec_off coordinates."""
+        dna_off = np.ascontiguousarray(dna_off, dtype=np.int64)
+        rec_off = np.ascontiguousarray(rec_off, dtype=np.int64)
+        nblk = np.zeros(0, dtype=np.int64) if nblk is None else np.ascontiguousarray(nblk, dtype=np.int64)
+        self._ck(lib().gm_db_upload_2bit(self._ctx, host_ptr, n_bytes, dna_off.ctypes.data, rec_off.ctypes.data,
+                                         len(rec_off) - 1, nblk.ctypes.data if nblk.size else None, nblk.size // 2),
+                 "gm_db_upload_2bit")
 
     def records(self):
         """(rec_off, hdr_off) of the uploaded batch; hdr_off is None unless it came
