@@ -158,9 +158,35 @@ int gm_db_set_device_chars(gm_ctx *c, const void *d_seq, const int64_t *rec_off,
  * on asynchronously like gm_db_upload_chars. */
 int gm_db_upload_fastn(gm_ctx *c, const char *text, size_t n_bytes);
 
+/* FASTA compressed as BGZF (bgzip, htslib): `gz` is the file's bytes as read from disk,
+ * about a third of a byte per nucleotide over PCIe for 60-column acgt at bgzip's default
+ * level.  It is gm_db_upload_fastn(c, T, |T|) where T is the concatenation of the
+ * decompressed members: every call after it sees what that call would give, hdr_off in T's
+ * coordinates.  The members are inflated on the device, one thread each, straight into
+ * the text buffer, while the next chunk of members is still copying; each member's
+ * length and CRC-32 are checked against its trailer.  n_bytes == 0, or only empty members,
+ * gives an empty database.  Refused, before the previous batch is touched: a member header
+ * that is not gzip (magic 31 139, CM 8, no reserved FLG bits) or not BGZF (FEXTRA with a
+ * BC subfield of SLEN 2; plain gzip has its own message), FNAME, FCOMMENT or FHCRC running
+ * past the member, BSIZE too small for header and trailer or running past n_bytes, ISIZE
+ * over 65536, more than 2^40 bytes of text, bytes left after the last member.  Refused
+ * after inflating, naming the first failing member and its byte offset in gz: invalid
+ * deflate data, output length other than ISIZE, CRC mismatch, text not beginning with
+ * '>'; the context then holds no database (gm_scan, gm_hit_windows, gm_db_get_chars and
+ * gm_db_get_text refuse) until the next upload succeeds.  Blocks until the record table
+ * is known, so gz may be reused when it returns; the pack runs on asynchronously.
+ * gm_scan_stats_t::h2d_bytes = n_bytes + the member table (32 bytes a member). */
+int gm_db_upload_fastn_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_bytes);
+
+/* Bytes [off, off + n) of the text of the last gm_db_upload_fastn or
+ * gm_db_upload_fastn_bgzf, read back from the device: the ids and definition lines
+ * where hdr_off points, for a caller that never had the text on the host.  Refused
+ * after the other uploads and outside [0, hdr_off[n_rec]). */
+int gm_db_get_text(gm_ctx *c, int64_t off, int64_t n, char *out);
+
 /* Record table of the uploaded batch: rec_off[0..n_rec] as in
- * gm_db_upload_chars, and -- after gm_db_upload_fastn only, else NULL --
- * hdr_off[r] = offset in `text` of record r's '>' (hdr_off[n_rec] = n_bytes), so
+ * gm_db_upload_chars, and -- after gm_db_upload_fastn or gm_db_upload_fastn_bgzf only,
+ * else NULL -- hdr_off[r] = offset in `text` of record r's '>' (hdr_off[n_rec] = n_bytes), so
  * the caller can read ids and definition lines where they lie.  Owned by the
  * context until the next upload. */
 int gm_db_records(const gm_ctx *c, const int64_t **rec_off, const int64_t **hdr_off, int *n_rec);

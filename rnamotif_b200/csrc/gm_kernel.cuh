@@ -3,6 +3,7 @@
 //   gm_pack_kernel     chars (what FN_fgetseq leaves, src/dbutil.c:105-111)
 //                      -> 4-bit IUPAC codes, two per byte
 //   gm_unpack2_kernel  UCSC .2bit bytes + N ranges -> the same 4-bit codes
+//   gm_inflate_kernel  BGZF members -> FASTA text, one thread per member
 //   gm_search_kernel   persistent CTAs; each takes tiles of consecutive start
 //                      positions from a global counter, stages the packed
 //                      tile + halo into shared memory with one TMA bulk copy
@@ -18,6 +19,7 @@
 #include "gm_search.cuh"
 #include "gm_score.h"
 #include "gm_twobit.h"
+#include "gm_inflate.h"
 
 namespace gm {
 
@@ -206,6 +208,40 @@ __global__ void __launch_bounds__(256) gm_unpack2_kernel(const uint8_t *__restri
 		}
 		__syncthreads(); // br is rewritten by the next round
 	}
+}
+
+// One BGZF member, as the host reads it from the member's header and trailer.
+struct BgzfMember {
+	uint64_t src;   // the deflate data's offset in the compressed bytes
+	uint64_t dst;   // the output's offset in the text
+	uint32_t len;   // bytes of deflate data
+	uint32_t isize; // bytes of output (the trailer's ISIZE)
+	uint32_t crc;   // the trailer's CRC-32
+	uint32_t pad_;
+};
+
+// BGZF members [m0, m1) -> text: one thread per member inflates it (gm_inflate.h, tables in
+// local memory) straight to its offset and checks the output's CRC-32 against the trailer's
+// (the table in shared memory).  status[m] = gm_inflate.h's status; *first_bad = the lowest
+// failing member (the host sets it to ~0u first).  A member writes only its own [dst, dst + isize).
+__global__ void __launch_bounds__(32) gm_inflate_kernel(const uint8_t *__restrict__ gz, const BgzfMember *__restrict__ mem,
+	int m0, int m1, uint8_t *__restrict__ text, uint8_t *__restrict__ status, unsigned int *__restrict__ first_bad)
+{
+	__shared__ uint32_t crc_tab[256];
+	for (int i = threadIdx.x; i < 256; i += blockDim.x)
+		crc_tab[i] = crc32_entry((uint32_t)i);
+	__syncthreads();
+	const int m = m0 + (int)(blockIdx.x * blockDim.x + threadIdx.x);
+	if (m >= m1)
+		return;
+	const BgzfMember e = mem[m];
+	uint32_t n_out;
+	int st = inflate(gz + e.src, e.len, text + e.dst, e.isize, &n_out);
+	if (st == GM_INF_OK && crc32(crc_tab, text + e.dst, e.isize) != e.crc)
+		st = GM_INF_CRC;
+	status[m] = (uint8_t)st;
+	if (st != GM_INF_OK)
+		atomicMin(first_bad, (unsigned int)m);
 }
 
 // ------------------------------------------------------------- TMA helpers

@@ -121,6 +121,13 @@ struct gm_ctx {
 	size_t tb_cap;           // bytes
 	std::vector<int64_t> tb;
 	bool codes_exact;        // the last upload was 2-bit: d_packed holds only a, c, g, t, n, and they decode to characters
+	// BGZF upload (gm_db_upload_fastn_bgzf): the compressed bytes (d_gz); the member table, then the first
+	// failing member (u32), then a status byte per member (d_bgzf); the member table on the host (bgzf)
+	uint8_t *d_gz;
+	size_t gz_cap;
+	void *d_bgzf;
+	size_t bgzf_cap;
+	std::vector<BgzfMember> bgzf;
 	// windows around the candidates (gm_hit_windows)
 	uint8_t *d_win, *h_win;
 	size_t win_cap, h_win_cap;
@@ -1159,6 +1166,9 @@ extern "C" int gm_ctx_create(gm_ctx **out, const gm_plan_t *plan, int device)
 	c->d_tb = NULL;
 	c->tb_cap = 0;
 	c->codes_exact = false;
+	c->d_gz = NULL;
+	c->d_bgzf = NULL;
+	c->gz_cap = c->bgzf_cap = 0;
 	c->d_win = c->h_win = NULL;
 	c->win_cap = c->h_win_cap = 0;
 	c->d_rec_off = NULL;
@@ -1306,6 +1316,8 @@ extern "C" void gm_ctx_destroy(gm_ctx *c)
 	cudaFree(c->d_text);
 	cudaFree(c->d_hdr_off);
 	cudaFree(c->d_tb);
+	cudaFree(c->d_gz);
+	cudaFree(c->d_bgzf);
 	cudaFree(c->d_fsum);
 	cudaFree(c->d_fstart);
 	cudaFree(c->d_win);
@@ -1835,40 +1847,20 @@ extern "C" int gm_db_upload_2bit(gm_ctx *c, const uint8_t *dna, size_t n_bytes, 
 	return 0;
 }
 
-// FN_fgetseq on the device, src/dbutil.c:42-128 (gm_fastn.cuh): text -> kept
-// characters + record table -> 4-bit codes.
-extern "C" int gm_db_upload_fastn(gm_ctx *c, const char *text, size_t n_bytes)
+// FN_fgetseq on the device, src/dbutil.c:42-128 (gm_fastn.cuh), over the n bytes of FASTA text in
+// d_text (enqueued on copy_stream, or already there): text -> kept characters + record table
+// (rec_off, hdr_off; blocks until they are known) -> 4-bit codes, asynchronously.
+static int read_fastn(gm_ctx *c, int64_t n)
 {
-	if (c == NULL)
-		return fail("ctx is NULL");
-	if (c->pending)
-		return fail("a scan is in flight");
-	if (n_bytes > 0 && text == NULL)
-		return fail("text is NULL");
-	if (n_bytes > ((size_t)1 << 40))
-		return fail("text too long");
-	if (join_uploader(c))
-		return -1;
-	c->up_published = -1;
-	CU(cudaSetDevice(c->device));
-	if (sync_uploads(c))
-		return -1;
-	NvtxRange nvtx_("gpumotif: upload fastn (H2D + device reader)");
-	if (n_bytes > 0 && text[0] != '>')
-		return fail("fastn text does not begin with '>' (src/dbutil.c:56-60)");
-	const int64_t n = (int64_t)n_bytes;
 	const int n_seg = (int)((n + GM_FASTN_SEG - 1) / GM_FASTN_SEG);
-	if (ensure((void **)&c->d_text, &c->text_cap, n_bytes + 64) ||
-	    ensure((void **)&c->d_chars, &c->chars_cap, n_bytes + 64) ||
+	if (ensure((void **)&c->d_chars, &c->chars_cap, (size_t)n + 64) ||
 	    ensure(&c->d_fsum, &c->fsum_cap, (size_t)(n_seg + 1) * sizeof(FastnSum) + 16) ||
 	    ensure(&c->d_fstart, &c->fstart_cap, (size_t)(n_seg + 1) * sizeof(FastnSegStart)))
 		return -1;
 	unsigned long long *d_tot = reinterpret_cast<unsigned long long *>(
 		static_cast<uint8_t *>(c->d_fsum) + (size_t)(n_seg + 1) * sizeof(FastnSum));
-	CU(cudaEventRecord(c->up_ev[0], c->copy_stream));
 	unsigned long long tot[2] = {0, 0};
 	if (n > 0) {
-		CU(cudaMemcpyAsync(c->d_text, text, n_bytes, cudaMemcpyHostToDevice, c->copy_stream));
 		const int blocks = (n_seg * 32 + 255) / 256;
 		gm_fastn_summarize<<<blocks, 256, 0, c->copy_stream>>>(c->d_text, n, static_cast<FastnSum *>(c->d_fsum), n_seg);
 		CU(cudaGetLastError());
@@ -1910,7 +1902,223 @@ extern "C" int gm_db_upload_fastn(gm_ctx *c, const char *text, size_t n_bytes)
 			return fail("record %d longer than 2^31", r);
 	if (upload_chunks(c, NULL, c->d_chars, false))
 		return -1;
+	return 0;
+}
+
+extern "C" int gm_db_upload_fastn(gm_ctx *c, const char *text, size_t n_bytes)
+{
+	if (c == NULL)
+		return fail("ctx is NULL");
+	if (c->pending)
+		return fail("a scan is in flight");
+	if (n_bytes > 0 && text == NULL)
+		return fail("text is NULL");
+	if (n_bytes > ((size_t)1 << 40))
+		return fail("text too long");
+	if (join_uploader(c))
+		return -1;
+	c->up_published = -1;
+	CU(cudaSetDevice(c->device));
+	if (sync_uploads(c))
+		return -1;
+	NvtxRange nvtx_("gpumotif: upload fastn (H2D + device reader)");
+	if (n_bytes > 0 && text[0] != '>')
+		return fail("fastn text does not begin with '>' (src/dbutil.c:56-60)");
+	if (ensure((void **)&c->d_text, &c->text_cap, n_bytes + 64))
+		return -1;
+	CU(cudaEventRecord(c->up_ev[0], c->copy_stream));
+	if (n_bytes > 0)
+		CU(cudaMemcpyAsync(c->d_text, text, n_bytes, cudaMemcpyHostToDevice, c->copy_stream));
+	if (read_fastn(c, (int64_t)n_bytes))
+		return -1;
 	c->stats.h2d_bytes = (uint64_t)n_bytes;
+	return 0;
+}
+
+static uint32_t le32(const uint8_t *p) { return p[0] | (p[1] << 8) | (p[2] << 16) | ((uint32_t)p[3] << 24); }
+
+// The context holds no database: gm_scan, gm_hit_windows, gm_db_get_chars and gm_db_get_text refuse
+// until the next upload succeeds.
+static void drop_database(gm_ctx *c)
+{
+	c->rec_off.clear();
+	c->hdr_off.clear();
+	c->total_nt = 0;
+	c->d_seq_chars = NULL;
+	c->codes_exact = false;
+	c->chunk_end.clear();
+	c->upload_fresh = false;
+}
+
+// BGZF: the member table comes from the headers alone (each member's trailer gives its output
+// size, so its offset in the text is known), the compressed bytes go over in chunks of whole
+// members, and gm_inflate_kernel inflates chunk i on pack_stream behind its copy while chunk i+1
+// is copying.  Then the text is read as gm_db_upload_fastn reads it.
+extern "C" int gm_db_upload_fastn_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_bytes)
+{
+	if (c == NULL)
+		return fail("ctx is NULL");
+	if (c->pending)
+		return fail("a scan is in flight");
+	if (n_bytes > 0 && gz == NULL)
+		return fail("gz is NULL");
+	// the member table; everything is checked before the previous batch is touched
+	std::vector<BgzfMember> mem;
+	std::vector<size_t> starts; // each member's offset in gz
+	uint64_t total = 0;
+	for (size_t p = 0; p < n_bytes;) {
+		const size_t left = n_bytes - p;
+		const uint8_t *h = gz + p;
+		const int k = (int)mem.size();
+		if (left < 18)
+			return fail("%zu bytes left over after the last BGZF member, at byte %zu", left, p);
+		if (h[0] != 31 || h[1] != 139)
+			return fail("member %d at byte %zu: not gzip (magic %d %d)", k, p, h[0], h[1]);
+		if (h[2] != 8)
+			return fail("member %d at byte %zu: compression method %d, not deflate (8)", k, p, h[2]);
+		const uint8_t flg = h[3];
+		if (flg & 0xe0)
+			return fail("member %d at byte %zu: reserved FLG bits set (FLG %#x)", k, p, flg);
+		if (!(flg & 4))
+			return fail("member %d at byte %zu: not BGZF: recompress with bgzip (plain gzip has no BC extra field)", k, p);
+		const size_t xlen = h[10] | (h[11] << 8);
+		if (12 + xlen > left)
+			return fail("member %d at byte %zu: the extra field runs past the %zu bytes", k, p, n_bytes);
+		int64_t bsize = -1;
+		for (size_t q = 12; q + 4 <= 12 + xlen;) {
+			const size_t slen = h[q + 2] | (h[q + 3] << 8);
+			if (q + 4 + slen > 12 + xlen)
+				break;
+			if (h[q] == 'B' && h[q + 1] == 'C' && slen == 2)
+				bsize = h[q + 4] | (h[q + 5] << 8);
+			q += 4 + slen;
+		}
+		if (bsize < 0)
+			return fail("member %d at byte %zu: not BGZF: recompress with bgzip (no BC subfield of SLEN 2)", k, p);
+		const size_t size = (size_t)bsize + 1;
+		if (size < 12 + xlen + 8)
+			return fail("member %d at byte %zu: BSIZE %lld too small for its header and trailer", k, p, (long long)bsize);
+		if (size > left)
+			return fail("member %d at byte %zu: BSIZE %lld runs past the %zu bytes", k, p, (long long)bsize, n_bytes);
+		size_t q = 12 + xlen; // FNAME, FCOMMENT (zero-terminated), FHCRC, then the deflate data
+		for (int f = 3; f <= 4; f++) {
+			if (!(flg & (1 << f)))
+				continue;
+			while (q < size - 8 && h[q] != 0)
+				q++;
+			if (q >= size - 8)
+				return fail("member %d at byte %zu: %s runs past the member", k, p, f == 3 ? "FNAME" : "FCOMMENT");
+			q++;
+		}
+		if ((flg & 2) && (q += 2) > size - 8)
+			return fail("member %d at byte %zu: FHCRC runs past the member", k, p);
+		BgzfMember e;
+		e.src = p + q;
+		e.dst = total;
+		e.len = (uint32_t)(size - 8 - q);
+		e.crc = le32(h + size - 8);
+		e.isize = le32(h + size - 4);
+		e.pad_ = 0;
+		if (e.isize > 65536)
+			return fail("member %d at byte %zu: ISIZE %u over 65536", k, p, e.isize);
+		total += e.isize;
+		if (total > ((uint64_t)1 << 40))
+			return fail("text too long: the members hold more than 2^40 bytes");
+		mem.push_back(e);
+		starts.push_back(p);
+		p += size;
+	}
+	if (mem.size() > 0x7fffffffu)
+		return fail("too many BGZF members");
+	if (join_uploader(c))
+		return -1;
+	c->up_published = -1;
+	CU(cudaSetDevice(c->device));
+	if (sync_uploads(c))
+		return -1;
+	NvtxRange nvtx_("gpumotif: upload BGZF fastn (H2D + inflate + device reader)");
+	const int n_mem = (int)mem.size();
+	const size_t tab = (size_t)n_mem * sizeof(BgzfMember);
+	if (ensure((void **)&c->d_text, &c->text_cap, (size_t)total + 64) || ensure((void **)&c->d_gz, &c->gz_cap, n_bytes + 16) ||
+	    ensure(&c->d_bgzf, &c->bgzf_cap, tab + 8 + (size_t)n_mem))
+		return -1;
+	c->bgzf.swap(mem);
+	BgzfMember *d_mem = static_cast<BgzfMember *>(c->d_bgzf);
+	unsigned int *d_first = reinterpret_cast<unsigned int *>(static_cast<uint8_t *>(c->d_bgzf) + tab);
+	uint8_t *d_status = static_cast<uint8_t *>(c->d_bgzf) + tab + 8;
+	CU(cudaEventRecord(c->up_ev[0], c->copy_stream));
+	if (n_mem > 0) {
+		CU(cudaMemcpyAsync(d_mem, c->bgzf.data(), tab, cudaMemcpyHostToDevice, c->copy_stream));
+		CU(cudaMemsetAsync(d_first, 0xff, sizeof(unsigned int), c->copy_stream));
+		// chunks of the compressed bytes (at least 64 MiB, at most 16; GPUMOTIF_CHUNK_NT lowers the
+		// floor), each ending where the first member starting at or after its cut begins
+		int64_t chunk;
+		if (cut_chunks(c, (int64_t)n_bytes, (int64_t)64 << 20, 16, 1, true, &chunk))
+			return -1;
+		const int n_chunks = (int)c->chunk_end.size();
+		int m0 = 0;
+		size_t copied = 0;
+		for (int i = 0; i < n_chunks; i++) {
+			int m1 = m0;
+			while (m1 < n_mem && (i == n_chunks - 1 || (int64_t)starts[m1] < c->chunk_end[i]))
+				m1++;
+			const size_t upto = m1 < n_mem ? starts[m1] : n_bytes;
+			if (upto > copied)
+				CU(cudaMemcpyAsync(c->d_gz + copied, gz + copied, upto - copied, cudaMemcpyHostToDevice, c->copy_stream));
+			copied = std::max(copied, upto);
+			CU(cudaEventRecord(c->cp_ev[i], c->copy_stream));
+			if (m1 > m0) {
+				CU(cudaStreamWaitEvent(c->pack_stream, c->cp_ev[i], 0));
+				// one thread per member, spread over the SMs: the decode is a chain of dependent loads
+				const int m = m1 - m0;
+				const int tpb = std::min(32, std::max(1, (m + c->n_sm - 1) / c->n_sm));
+				gm_inflate_kernel<<<(m + tpb - 1) / tpb, tpb, 0, c->pack_stream>>>(c->d_gz, d_mem, m0, m1, c->d_text, d_status,
+												    d_first);
+				CU(cudaGetLastError());
+			}
+			m0 = m1;
+		}
+		// the first failing member, its status and the text's first byte
+		struct {
+			unsigned int first;
+			uint8_t st, ch;
+		} res = {0xffffffffu, 0, '>'};
+		CU(cudaMemcpyAsync(&res.first, d_first, sizeof res.first, cudaMemcpyDeviceToHost, c->pack_stream));
+		if (total > 0)
+			CU(cudaMemcpyAsync(&res.ch, c->d_text, 1, cudaMemcpyDeviceToHost, c->pack_stream));
+		CU(cudaStreamSynchronize(c->pack_stream));
+		if (res.first != 0xffffffffu) {
+			const unsigned int k = res.first;
+			drop_database(c);
+			CU(cudaMemcpy(&res.st, d_status + k, 1, cudaMemcpyDeviceToHost));
+			return fail("BGZF member %u at byte %zu: %s", k, starts[k], inflate_status_name(res.st));
+		}
+		if (res.ch != '>') {
+			drop_database(c);
+			return fail("the text of the BGZF members does not begin with '>' (src/dbutil.c:56-60)");
+		}
+	}
+	if (read_fastn(c, (int64_t)total))
+		return -1;
+	c->stats.h2d_bytes = (uint64_t)n_bytes + (uint64_t)tab;
+	return 0;
+}
+
+extern "C" int gm_db_get_text(gm_ctx *c, int64_t off, int64_t n, char *out)
+{
+	if (c == NULL || out == NULL || off < 0 || n < 0)
+		return fail("bad argument");
+	if (c->rec_off.empty() || c->hdr_off.size() != c->rec_off.size())
+		return fail(c->rec_off.empty() ? "no database uploaded"
+					       : "no FASTA text on the device: the last upload was not gm_db_upload_fastn or gm_db_upload_fastn_bgzf");
+	const int64_t len = c->hdr_off.back();
+	if (off + n > len)
+		return fail("range [%lld, %lld) outside the %lld bytes of text", (long long)off, (long long)(off + n), (long long)len);
+	CU(cudaSetDevice(c->device));
+	if (sync_uploads(c))
+		return -1;
+	if (n > 0)
+		CU(cudaMemcpy(out, c->d_text + off, (size_t)n, cudaMemcpyDeviceToHost));
 	return 0;
 }
 
@@ -2129,6 +2337,8 @@ extern "C" int gm_scan_launch(gm_ctx *c, int64_t g_begin, int64_t g_end, int str
 		return fail("a scan is already in flight");
 	if (strands != 1 && strands != 2)
 		return fail("strands must be 1 or 2");
+	if (c->rec_off.empty())
+		return fail("no database uploaded");
 	if (g_begin < 0 || g_end > c->total_nt || g_begin > g_end)
 		return fail("range [%lld, %lld) outside the database of %lld nt", (long long)g_begin,
 			    (long long)g_end, (long long)c->total_nt);
