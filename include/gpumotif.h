@@ -94,11 +94,25 @@ int gm_plan_describe(const gm_plan_t *plan, char *out, size_t cap);
 int gm_host_alloc(void **out, size_t n_bytes);
 void gm_host_free(void *p);
 
+/*
+ * Database.  Each upload below replaces the batch the context holds, and all of them
+ * keep one contract:
+ *   - bad input (a record table, a NULL pointer, a 2-bit or BGZF table, text that
+ *     does not begin with '>' ...) is refused with the previous batch intact;
+ *   - any later failure (an allocation, a copy, the device reader, an inflate error)
+ *     leaves the context with no database: gm_scan, gm_db_records, gm_db_get_text,
+ *     gm_db_get_chars and gm_hit_windows refuse and gm_db_total_nt is 0 until an
+ *     upload succeeds;
+ *   - an upload forgets the last scan's candidates: gm_hits reports none and
+ *     gm_hit_windows no rows until the next scan.  Buffers they handed out stay
+ *     allocated.
+ */
+
 /* Upload a batch of records given as the characters FN_fgetseq leaves in its
  * buffer (src/dbutil.c:42-128: letters only, any case, u or t): record r is
  * seq[rec_off[r] .. rec_off[r+1]).  The copy goes host -> device as is and is
  * packed to 4-bit IUPAC codes on the device.  `seq` may be pinned or pageable
- * host memory.  Replaces the previous batch.  The copy is ASYNCHRONOUS when
+ * host memory.  The copy is ASYNCHRONOUS when
  * `seq` is pinned: it is cut into chunks on a copy stream and the first gm_scan
  * after it starts searching chunk 0 while the rest is still in flight, so `seq`
  * must stay valid and unchanged until that scan has returned. */
@@ -131,13 +145,12 @@ int gm_host_pack(const char *seq, int64_t n, uint8_t *packed, int n_threads);
  * headers between records included.  nblk holds n_nblk half-open N ranges
  * [nblk[2k], nblk[2k+1]) in rec_off coordinates (the file's N blocks shifted by their
  * record's rec_off), sorted and disjoint (adjacent is fine); they read as n.  Mask
- * blocks are not needed: the search folds case.  Refused, before the previous batch is
- * touched: dna_off not ascending, a record's bytes overlapping the next record's or
- * running past n_bytes, N ranges out of order, overlapping, ending before they start or
- * outside [0, total), and every record table gm_db_upload_chars refuses.  Replaces the
- * previous batch; cut into chunks and asynchronous like gm_db_upload_chars (`dna` must
- * stay valid and unchanged until the next gm_scan has returned when it is pinned).  The
- * codes on the device are exact (a, c, g, t, n), so gm_hit_windows and gm_db_get_chars
+ * blocks are not needed: the search folds case.  Refused: dna_off not ascending, a
+ * record's bytes overlapping the next record's or running past n_bytes, N ranges out of
+ * order, overlapping, ending before they start or outside [0, total), and every record
+ * table gm_db_upload_chars refuses.  Cut into chunks and asynchronous like
+ * gm_db_upload_chars (`dna` must stay valid and unchanged until the next gm_scan has
+ * returned when it is pinned).  The codes on the device are exact (a, c, g, t, n), so gm_hit_windows and gm_db_get_chars
  * work after it; gm_db_records gives hdr_off = NULL.  gm_scan_stats_t::h2d_bytes =
  * the span + the record table + dna_off + the N ranges. */
 int gm_db_upload_2bit(gm_ctx *c, const uint8_t *dna, size_t n_bytes, const int64_t *dna_off,
@@ -165,16 +178,13 @@ int gm_db_upload_fastn(gm_ctx *c, const char *text, size_t n_bytes);
  * coordinates.  The members are inflated on the device, one thread each, straight into
  * the text buffer, while the next chunk of members is still copying; each member's
  * length and CRC-32 are checked against its trailer.  n_bytes == 0, or only empty members,
- * gives an empty database.  Refused, before the previous batch is touched: a member header
- * that is not gzip (magic 31 139, CM 8, no reserved FLG bits) or not BGZF (FEXTRA with a
+ * gives an empty database.  Refused as bad input: a member header that is not gzip (magic 31 139, CM 8, no reserved FLG bits) or not BGZF (FEXTRA with a
  * BC subfield of SLEN 2; plain gzip has its own message), FNAME, FCOMMENT or FHCRC running
  * past the member, BSIZE too small for header and trailer or running past n_bytes, ISIZE
  * over 65536, more than 2^40 bytes of text, bytes left after the last member.  Refused
  * after inflating, naming the first failing member and its byte offset in gz: invalid
  * deflate data, output length other than ISIZE, CRC mismatch, text not beginning with
- * '>'; the context then holds no database (gm_scan, gm_hit_windows, gm_db_get_chars and
- * gm_db_get_text refuse) until the next upload succeeds.  Blocks until the record table
- * is known, so gz may be reused when it returns; the pack runs on asynchronously.
+ * '>'.  Blocks until the record table is known, so gz may be reused when it returns; the pack runs on asynchronously.
  * gm_scan_stats_t::h2d_bytes = n_bytes + the member table (32 bytes a member). */
 int gm_db_upload_fastn_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_bytes);
 

@@ -58,6 +58,11 @@ struct NvtxRange {
 
 #define GM_PACK_SLOTS 4
 
+// What the context's database is (gm_ctx::db).  DB_CHARS: characters on the device (d_seq_chars) and
+// their 4-bit codes; DB_HOSTPACK: the codes only; DB_2BIT: codes that decode to characters (a, c, g, t,
+// n); DB_FASTN: FASTA text, its characters, their codes and the header offsets (hdr_off).
+enum DbKind { DB_NONE, DB_CHARS, DB_HOSTPACK, DB_2BIT, DB_FASTN };
+
 struct gm_ctx {
 	gm_plan_t plan;
 	DevParams par;
@@ -97,13 +102,15 @@ struct gm_ctx {
 	gm_plan_t *d_plan;
 	DevSearch *d_ds;
 	gm_score_t *d_score;   // score pre-screen (gm_ctx_set_score) or NULL
-	// database
+	// database; every upload sets db as its last step, on success only, and nothing below is read while
+	// db is DB_NONE
+	DbKind db;
 	uint8_t *d_chars;      // staging for uploaded characters
 	size_t chars_cap;
 	uint8_t *d_packed;
 	size_t packed_cap;
 	int64_t *d_rec_off;
-	size_t rec_cap;
+	size_t rec_cap;        // bytes
 	std::vector<int64_t> rec_off;
 	int64_t total_nt;
 	// FASTA text parsed on the device (gm_db_upload_fastn)
@@ -120,7 +127,6 @@ struct gm_ctx {
 	int64_t *d_tb;
 	size_t tb_cap;           // bytes
 	std::vector<int64_t> tb;
-	bool codes_exact;        // the last upload was 2-bit: d_packed holds only a, c, g, t, n, and they decode to characters
 	// BGZF upload (gm_db_upload_fastn_bgzf): the compressed bytes (d_gz); the member table, then the first
 	// failing member (u32), then a status byte per member (d_bgzf); the member table on the host (bgzf)
 	uint8_t *d_gz;
@@ -1165,7 +1171,7 @@ extern "C" int gm_ctx_create(gm_ctx **out, const gm_plan_t *plan, int device)
 	c->d_seq_chars = NULL;
 	c->d_tb = NULL;
 	c->tb_cap = 0;
-	c->codes_exact = false;
+	c->db = DB_NONE;
 	c->d_gz = NULL;
 	c->d_bgzf = NULL;
 	c->gz_cap = c->bgzf_cap = 0;
@@ -1399,7 +1405,11 @@ static int ensure(void **p, size_t *cap, size_t need)
 	*p = NULL;
 	*cap = 0;
 	size_t n = need + need / 8 + 256;
-	CU(cudaMalloc(p, n));
+	if (cudaMalloc(p, n) != cudaSuccess) {
+		// read and cleared here: the next launch's cudaGetLastError() must not report this allocation
+		const cudaError_t e = cudaGetLastError();
+		return fail("cudaMalloc(%zu bytes): %s", n, cudaGetErrorString(e));
+	}
 	*cap = n;
 	return 0;
 }
@@ -1419,19 +1429,15 @@ static int check_records(const int64_t *rec_off, int n_rec)
 	return 0;
 }
 
+// a record table check_records has passed, on the host and (enqueued) on the device
 static int set_records(gm_ctx *c, const int64_t *rec_off, int n_rec)
 {
-	if (check_records(rec_off, n_rec))
-		return -1;
+	const size_t tab = (size_t)(n_rec + 1) * sizeof(int64_t);
 	c->rec_off.assign(rec_off, rec_off + n_rec + 1);
-	c->hdr_off.clear();
 	c->total_nt = rec_off[n_rec];
-	size_t cap_bytes = c->rec_cap * sizeof(int64_t);
-	if (ensure((void **)&c->d_rec_off, &cap_bytes, (size_t)(n_rec + 1) * sizeof(int64_t)))
+	if (ensure((void **)&c->d_rec_off, &c->rec_cap, tab))
 		return -1;
-	c->rec_cap = cap_bytes / sizeof(int64_t);
-	CU(cudaMemcpyAsync(c->d_rec_off, c->rec_off.data(), (size_t)(n_rec + 1) * sizeof(int64_t),
-			   cudaMemcpyHostToDevice, c->copy_stream));
+	CU(cudaMemcpyAsync(c->d_rec_off, c->rec_off.data(), tab, cudaMemcpyHostToDevice, c->copy_stream));
 	return 0;
 }
 
@@ -1443,17 +1449,49 @@ static int sync_uploads(gm_ctx *c)
 	return 0;
 }
 
-// The uploader thread of the last host-packed upload has enqueued everything (or failed).
-static int join_uploader(gm_ctx *c)
+// The context holds no database: gm_scan, gm_db_records, gm_db_get_text, gm_db_get_chars and
+// gm_hit_windows refuse until an upload succeeds.  The last scan's candidates go with it (their record
+// indices belong to the old batch); the host buffers already handed out stay allocated.
+static void drop_database(gm_ctx *c)
 {
+	c->db = DB_NONE;
+	c->n_hits = c->n_raw = 0;
+	c->hits_view = NULL;
+}
+
+// Every upload, once its host-side input has been checked, starts here: the uploader thread of the
+// last host-packed upload has enqueued everything (or failed), the previous upload has left the
+// device (its staging is reused), and the context holds no database, so a failure anywhere later
+// leaves none.  The upload sets c->db as its last step.
+static int begin_upload(gm_ctx *c)
+{
+	if (c == NULL)
+		return fail("ctx is NULL");
+	if (c->pending)
+		return fail("a scan is in flight");
 	if (c->up_thread.joinable())
 		c->up_thread.join();
+	c->up_published = -1;
+	drop_database(c); // also when that thread failed: its chunks would never be published
 	if (c->up_err[0]) {
 		fail("%s", c->up_err);
 		c->up_err[0] = 0;
 		return -1;
 	}
-	return 0;
+	CU(cudaSetDevice(c->device));
+	return sync_uploads(c);
+}
+
+// the 4-bit codes of n nucleotides; slack: kernels read whole 16-byte groups past the end
+static int ensure_packed(gm_ctx *c, int64_t n)
+{
+	return ensure((void **)&c->d_packed, &c->packed_cap, (size_t)(((n + 15) / 16) * 8) + 1024);
+}
+
+// blocks of 256 threads for a pack / expand kernel over len nucleotides, one 16-nt group per thread
+static int pack_blocks(const gm_ctx *c, int64_t len)
+{
+	return (int)std::min<int64_t>(((len + 15) / 16 + 255) / 256, (int64_t)c->n_sm * 16);
 }
 
 // chunk_ev[i] has been recorded (host-packed uploads record it from the uploader thread)
@@ -1513,8 +1551,7 @@ static int upload_chunks(gm_ctx *c, const uint8_t *h_chars, const uint8_t *d_src
 {
 	NvtxRange nvtx_("gpumotif: upload chunks (H2D + pack)");
 	const int64_t n = c->total_nt;
-	const size_t pbytes = (size_t)(((n + 15) / 16) * 8) + 1024; // slack: kernels read whole 16-byte groups past the end
-	if (ensure((void **)&c->d_packed, &c->packed_cap, pbytes))
+	if (ensure_packed(c, n))
 		return -1;
 	if (h_chars != NULL && ensure((void **)&c->d_chars, &c->chars_cap, (size_t)n + 64))
 		return -1;
@@ -1522,9 +1559,7 @@ static int upload_chunks(gm_ctx *c, const uint8_t *h_chars, const uint8_t *d_src
 	if (cut_device_chunks(c, n, h_chars != NULL, &chunk))
 		return -1;
 	const int n_chunks = (int)c->chunk_end.size();
-	c->up_published = -1;
 	c->d_seq_chars = h_chars != NULL ? c->d_chars : d_src;
-	c->codes_exact = false;
 	if (mark_start)
 		CU(cudaEventRecord(c->up_ev[0], c->copy_stream));
 	// from the host: copies back to back on the copy stream, pack kernels on the pack stream behind
@@ -1539,9 +1574,7 @@ static int upload_chunks(gm_ctx *c, const uint8_t *h_chars, const uint8_t *d_src
 			CU(cudaStreamWaitEvent(ps, c->cp_ev[i], 0));
 			src = c->d_chars;
 		}
-		const int64_t groups = (len + 15) / 16;
-		const int blocks = (int)std::min<int64_t>((groups + 255) / 256, (int64_t)c->n_sm * 16);
-		gm_pack_kernel<<<blocks, 256, 0, ps>>>(src + o, c->d_packed + (o >> 1), len);
+		gm_pack_kernel<<<pack_blocks(c, len), 256, 0, ps>>>(src + o, c->d_packed + (o >> 1), len);
 		CU(cudaGetLastError());
 		CU(cudaEventRecord(c->chunk_ev[i], ps));
 	}
@@ -1552,23 +1585,23 @@ static int upload_chunks(gm_ctx *c, const uint8_t *h_chars, const uint8_t *d_src
 
 extern "C" int gm_db_upload_chars(gm_ctx *c, const char *seq, const int64_t *rec_off, int n_rec)
 {
-	if (c == NULL)
-		return fail("ctx is NULL");
-	if (c->pending)
-		return fail("a scan is in flight");
-	if (join_uploader(c))
+	if (check_records(rec_off, n_rec))
 		return -1;
-	CU(cudaSetDevice(c->device));
-	if (sync_uploads(c)) // the previous upload's staging is reused
-		return -1;
-	if (set_records(c, rec_off, n_rec))
-		return -1;
-	if (c->total_nt > 0 && seq == NULL)
+	if (rec_off[n_rec] > 0 && seq == NULL)
 		return fail("seq is NULL");
-	if (upload_chunks(c, (const uint8_t *)seq, NULL))
+	if (begin_upload(c) || set_records(c, rec_off, n_rec) || upload_chunks(c, (const uint8_t *)seq, NULL))
 		return -1;
 	c->stats.h2d_bytes = (uint64_t)c->total_nt + (uint64_t)(n_rec + 1) * 8;
+	c->db = DB_CHARS;
 	return 0;
+}
+
+// Nucleotides [o, o + hp) of a host-packed chunk [o, o + len) are packed on the host, [o + hp, o + len)
+// travel as characters; `frac` = the host-packed share.
+static int64_t host_share(int64_t len, double frac)
+{
+	const int64_t hp = frac >= 1.0 ? len : std::min<int64_t>(len, ((int64_t)(frac * (double)len) + 4095) & ~(int64_t)4095);
+	return len - hp < 4096 ? len : hp;
 }
 
 // Host-packed upload: the thread team turns (a share of) chunk i into 4-bit codes in a pinned
@@ -1592,10 +1625,7 @@ static void uploader_main(gm_ctx *c, const uint8_t *seq, int64_t chunk, double f
 	const int n_chunks = (int)c->chunk_end.size();
 	for (int i = 0; i < n_chunks; i++) {
 		const int64_t o = (int64_t)i * chunk, len = c->chunk_end[i] - o;
-		// [o, o + hp) is packed here, [o + hp, o + len) travels as characters
-		int64_t hp = frac >= 1.0 ? len : std::min<int64_t>(len, ((int64_t)(frac * (double)len) + 4095) & ~(int64_t)4095);
-		if (len - hp < 4096)
-			hp = len;
+		const int64_t hp = host_share(len, frac);
 		if (hp < len) {
 			// the character share first: the link works on it while the team packs
 			const int64_t oc = o + hp, lc = len - hp;
@@ -1603,9 +1633,7 @@ static void uploader_main(gm_ctx *c, const uint8_t *seq, int64_t chunk, double f
 			    (e = cudaEventRecord(c->cp_ev[i], c->copy_stream)) != cudaSuccess ||
 			    (e = cudaStreamWaitEvent(c->pack_stream, c->cp_ev[i], 0)) != cudaSuccess)
 				return bail("enqueue (characters)", e);
-			const int64_t groups = (lc + 15) / 16;
-			const int blocks = (int)std::min<int64_t>((groups + 255) / 256, (int64_t)c->n_sm * 16);
-			gm_pack_kernel<<<blocks, 256, 0, c->pack_stream>>>(c->d_chars + oc, c->d_packed + (oc >> 1), lc);
+			gm_pack_kernel<<<pack_blocks(c, lc), 256, 0, c->pack_stream>>>(c->d_chars + oc, c->d_packed + (oc >> 1), lc);
 			if ((e = cudaGetLastError()) != cudaSuccess)
 				return bail("pack kernel", e);
 		}
@@ -1639,22 +1667,12 @@ static void uploader_main(gm_ctx *c, const uint8_t *seq, int64_t chunk, double f
 
 extern "C" int gm_db_upload_chars_hostpack(gm_ctx *c, const char *seq, const int64_t *rec_off, int n_rec)
 {
-	if (c == NULL)
-		return fail("ctx is NULL");
-	if (c->pending)
-		return fail("a scan is in flight");
-	if (join_uploader(c))
+	if (check_records(rec_off, n_rec))
 		return -1;
-	CU(cudaSetDevice(c->device));
-	if (sync_uploads(c))
-		return -1;
-	if (set_records(c, rec_off, n_rec))
-		return -1;
-	const int64_t n = c->total_nt;
+	const int64_t n = rec_off[n_rec];
 	if (n > 0 && seq == NULL)
 		return fail("seq is NULL");
-	const size_t pbytes = (size_t)(((n + 15) / 16) * 8) + 1024;
-	if (ensure((void **)&c->d_packed, &c->packed_cap, pbytes))
+	if (begin_upload(c) || set_records(c, rec_off, n_rec) || ensure_packed(c, n))
 		return -1;
 	if (c->team == NULL)
 		c->team = new PackTeam(host_pack_default_threads());
@@ -1694,10 +1712,7 @@ extern "C" int gm_db_upload_chars_hostpack(gm_ctx *c, const char *seq, const int
 	for (int i = 0; i < GM_PACK_SLOTS; i++)
 		if (c->slot_ev[i] == NULL)
 			CU(cudaEventCreateWithFlags(&c->slot_ev[i], cudaEventDisableTiming));
-	c->d_seq_chars = NULL;
-	c->codes_exact = false;
 	c->up_published = 0;
-	c->up_err[0] = 0;
 	CU(cudaEventRecord(c->up_ev[0], c->copy_stream));
 	if (n_chunks == 0)
 		CU(cudaEventRecord(c->up_ev[1], c->copy_stream));
@@ -1706,37 +1721,27 @@ extern "C" int gm_db_upload_chars_hostpack(gm_ctx *c, const char *seq, const int
 		// bytes over the link: half a byte per host-packed nucleotide, one per character sent as it is
 		uint64_t b = (uint64_t)(n_rec + 1) * 8;
 		for (int i = 0; i < n_chunks; i++) {
-			const int64_t o = (int64_t)i * chunk, len = c->chunk_end[i] - o;
-			int64_t hp = frac >= 1.0 ? len : std::min<int64_t>(len, ((int64_t)(frac * (double)len) + 4095) & ~(int64_t)4095);
-			if (len - hp < 4096)
-				hp = len;
+			const int64_t len = c->chunk_end[i] - (int64_t)i * chunk, hp = host_share(len, frac);
 			b += (uint64_t)((hp + 1) >> 1) + (uint64_t)(len - hp);
 		}
 		c->stats.h2d_bytes = b;
 	}
 	if (n_chunks > 0)
 		c->up_thread = std::thread(uploader_main, c, (const uint8_t *)seq, chunk, frac);
+	c->db = DB_HOSTPACK;
 	return 0;
 }
 
 extern "C" int gm_db_set_device_chars(gm_ctx *c, const void *d_seq, const int64_t *rec_off, int n_rec)
 {
-	if (c == NULL)
-		return fail("ctx is NULL");
-	if (c->pending)
-		return fail("a scan is in flight");
-	if (join_uploader(c))
+	if (check_records(rec_off, n_rec))
 		return -1;
-	CU(cudaSetDevice(c->device));
-	if (sync_uploads(c))
-		return -1;
-	if (set_records(c, rec_off, n_rec))
-		return -1;
-	if (c->total_nt > 0 && d_seq == NULL)
+	if (rec_off[n_rec] > 0 && d_seq == NULL)
 		return fail("d_seq is NULL");
-	if (upload_chunks(c, NULL, (const uint8_t *)d_seq))
+	if (begin_upload(c) || set_records(c, rec_off, n_rec) || upload_chunks(c, NULL, (const uint8_t *)d_seq))
 		return -1;
 	c->stats.h2d_bytes = (uint64_t)(n_rec + 1) * 8;
+	c->db = DB_CHARS;
 	return 0;
 }
 
@@ -1747,11 +1752,6 @@ extern "C" int gm_db_set_device_chars(gm_ctx *c, const void *d_seq, const int64_
 extern "C" int gm_db_upload_2bit(gm_ctx *c, const uint8_t *dna, size_t n_bytes, const int64_t *dna_off,
 				 const int64_t *rec_off, int n_rec, const int64_t *nblk, int64_t n_nblk)
 {
-	if (c == NULL)
-		return fail("ctx is NULL");
-	if (c->pending)
-		return fail("a scan is in flight");
-	// everything is checked before the previous batch is touched
 	if (check_records(rec_off, n_rec))
 		return -1;
 	const int64_t n = rec_off[n_rec];
@@ -1785,12 +1785,7 @@ extern "C" int gm_db_upload_2bit(gm_ctx *c, const uint8_t *dna, size_t n_bytes, 
 			return fail("N range %lld [%lld, %lld) is out of order or overlaps the one before", (long long)k, (long long)s,
 				    (long long)e);
 	}
-	if (join_uploader(c))
-		return -1;
-	CU(cudaSetDevice(c->device));
-	if (sync_uploads(c)) // the previous upload's staging is reused
-		return -1;
-	if (set_records(c, rec_off, n_rec))
+	if (begin_upload(c) || set_records(c, rec_off, n_rec))
 		return -1;
 	// the span copied: [b0, b_end) of dna, record r's bases at dna_off[r] - b0 on the device
 	const int64_t b0 = n_rec > 0 ? dna_off[0] : 0;
@@ -1801,17 +1796,13 @@ extern "C" int gm_db_upload_2bit(gm_ctx *c, const uint8_t *dna, size_t n_bytes, 
 	if (n_nblk > 0)
 		memcpy(c->tb.data() + n_rec, nblk, (size_t)n_nblk * 2 * sizeof(int64_t));
 	const size_t tb_bytes = c->tb.size() * sizeof(int64_t);
-	const size_t pbytes = (size_t)(((n + 15) / 16) * 8) + 1024; // slack: kernels read whole 16-byte groups past the end
-	if (ensure((void **)&c->d_packed, &c->packed_cap, pbytes) || ensure((void **)&c->d_chars, &c->chars_cap, (size_t)span + 64) ||
+	if (ensure_packed(c, n) || ensure((void **)&c->d_chars, &c->chars_cap, (size_t)span + 64) ||
 	    ensure((void **)&c->d_tb, &c->tb_cap, tb_bytes + 16))
 		return -1;
 	int64_t chunk;
 	if (cut_device_chunks(c, n, true, &chunk))
 		return -1;
 	const int n_chunks = (int)c->chunk_end.size();
-	c->up_published = -1;
-	c->d_seq_chars = NULL;
-	c->codes_exact = true;
 	CU(cudaEventRecord(c->up_ev[0], c->copy_stream));
 	if (tb_bytes > 0)
 		CU(cudaMemcpyAsync(c->d_tb, c->tb.data(), tb_bytes, cudaMemcpyHostToDevice, c->copy_stream));
@@ -1833,10 +1824,8 @@ extern "C" int gm_db_upload_2bit(gm_ctx *c, const uint8_t *dna, size_t n_bytes, 
 		copied = std::max(copied, upto);
 		CU(cudaEventRecord(c->cp_ev[i], c->copy_stream));
 		CU(cudaStreamWaitEvent(c->pack_stream, c->cp_ev[i], 0));
-		const int64_t groups = (len + 15) / 16;
-		const int blocks = (int)std::min<int64_t>((groups + 255) / 256, (int64_t)c->n_sm * 16);
-		gm_unpack2_kernel<<<blocks, 256, 0, c->pack_stream>>>(c->d_chars, d_dna_off, c->d_rec_off, n_rec, d_nblk, n_nblk, o, len,
-								      c->d_packed);
+		gm_unpack2_kernel<<<pack_blocks(c, len), 256, 0, c->pack_stream>>>(c->d_chars, d_dna_off, c->d_rec_off, n_rec, d_nblk,
+										   n_nblk, o, len, c->d_packed);
 		CU(cudaGetLastError());
 		CU(cudaEventRecord(c->chunk_ev[i], c->pack_stream));
 	}
@@ -1844,6 +1833,7 @@ extern "C" int gm_db_upload_2bit(gm_ctx *c, const uint8_t *dna, size_t n_bytes, 
 	c->upload_fresh = true;
 	// bytes over the link: the span, the record table, dna_off and the N ranges
 	c->stats.h2d_bytes = (uint64_t)span + (uint64_t)(n_rec + 1) * 8 + (uint64_t)tb_bytes;
+	c->db = DB_2BIT;
 	return 0;
 }
 
@@ -1874,11 +1864,7 @@ static int read_fastn(gm_ctx *c, int64_t n)
 		return fail("too many records in one upload");
 	const int n_rec = (int)tot[1];
 	const size_t tab = (size_t)(n_rec + 1) * sizeof(int64_t);
-	size_t cap_bytes = c->rec_cap * sizeof(int64_t);
-	if (ensure((void **)&c->d_rec_off, &cap_bytes, tab))
-		return -1;
-	c->rec_cap = cap_bytes / sizeof(int64_t);
-	if (ensure((void **)&c->d_hdr_off, &c->hdr_cap, tab))
+	if (ensure((void **)&c->d_rec_off, &c->rec_cap, tab) || ensure((void **)&c->d_hdr_off, &c->hdr_cap, tab))
 		return -1;
 	c->rec_off.resize(n_rec + 1);
 	c->hdr_off.resize(n_rec + 1);
@@ -1907,23 +1893,15 @@ static int read_fastn(gm_ctx *c, int64_t n)
 
 extern "C" int gm_db_upload_fastn(gm_ctx *c, const char *text, size_t n_bytes)
 {
-	if (c == NULL)
-		return fail("ctx is NULL");
-	if (c->pending)
-		return fail("a scan is in flight");
 	if (n_bytes > 0 && text == NULL)
 		return fail("text is NULL");
 	if (n_bytes > ((size_t)1 << 40))
 		return fail("text too long");
-	if (join_uploader(c))
-		return -1;
-	c->up_published = -1;
-	CU(cudaSetDevice(c->device));
-	if (sync_uploads(c))
-		return -1;
-	NvtxRange nvtx_("gpumotif: upload fastn (H2D + device reader)");
 	if (n_bytes > 0 && text[0] != '>')
 		return fail("fastn text does not begin with '>' (src/dbutil.c:56-60)");
+	if (begin_upload(c))
+		return -1;
+	NvtxRange nvtx_("gpumotif: upload fastn (H2D + device reader)");
 	if (ensure((void **)&c->d_text, &c->text_cap, n_bytes + 64))
 		return -1;
 	CU(cudaEventRecord(c->up_ev[0], c->copy_stream));
@@ -1932,23 +1910,11 @@ extern "C" int gm_db_upload_fastn(gm_ctx *c, const char *text, size_t n_bytes)
 	if (read_fastn(c, (int64_t)n_bytes))
 		return -1;
 	c->stats.h2d_bytes = (uint64_t)n_bytes;
+	c->db = DB_FASTN;
 	return 0;
 }
 
 static uint32_t le32(const uint8_t *p) { return p[0] | (p[1] << 8) | (p[2] << 16) | ((uint32_t)p[3] << 24); }
-
-// The context holds no database: gm_scan, gm_hit_windows, gm_db_get_chars and gm_db_get_text refuse
-// until the next upload succeeds.
-static void drop_database(gm_ctx *c)
-{
-	c->rec_off.clear();
-	c->hdr_off.clear();
-	c->total_nt = 0;
-	c->d_seq_chars = NULL;
-	c->codes_exact = false;
-	c->chunk_end.clear();
-	c->upload_fresh = false;
-}
 
 // BGZF: the member table comes from the headers alone (each member's trailer gives its output
 // size, so its offset in the text is known), the compressed bytes go over in chunks of whole
@@ -1956,13 +1922,9 @@ static void drop_database(gm_ctx *c)
 // is copying.  Then the text is read as gm_db_upload_fastn reads it.
 extern "C" int gm_db_upload_fastn_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_bytes)
 {
-	if (c == NULL)
-		return fail("ctx is NULL");
-	if (c->pending)
-		return fail("a scan is in flight");
 	if (n_bytes > 0 && gz == NULL)
 		return fail("gz is NULL");
-	// the member table; everything is checked before the previous batch is touched
+	// the member table
 	std::vector<BgzfMember> mem;
 	std::vector<size_t> starts; // each member's offset in gz
 	uint64_t total = 0;
@@ -2030,11 +1992,7 @@ extern "C" int gm_db_upload_fastn_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_by
 	}
 	if (mem.size() > 0x7fffffffu)
 		return fail("too many BGZF members");
-	if (join_uploader(c))
-		return -1;
-	c->up_published = -1;
-	CU(cudaSetDevice(c->device));
-	if (sync_uploads(c))
+	if (begin_upload(c))
 		return -1;
 	NvtxRange nvtx_("gpumotif: upload BGZF fastn (H2D + inflate + device reader)");
 	const int n_mem = (int)mem.size();
@@ -2089,18 +2047,16 @@ extern "C" int gm_db_upload_fastn_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_by
 		CU(cudaStreamSynchronize(c->pack_stream));
 		if (res.first != 0xffffffffu) {
 			const unsigned int k = res.first;
-			drop_database(c);
 			CU(cudaMemcpy(&res.st, d_status + k, 1, cudaMemcpyDeviceToHost));
 			return fail("BGZF member %u at byte %zu: %s", k, starts[k], inflate_status_name(res.st));
 		}
-		if (res.ch != '>') {
-			drop_database(c);
+		if (res.ch != '>')
 			return fail("the text of the BGZF members does not begin with '>' (src/dbutil.c:56-60)");
-		}
 	}
 	if (read_fastn(c, (int64_t)total))
 		return -1;
 	c->stats.h2d_bytes = (uint64_t)n_bytes + (uint64_t)tab;
+	c->db = DB_FASTN;
 	return 0;
 }
 
@@ -2108,9 +2064,9 @@ extern "C" int gm_db_get_text(gm_ctx *c, int64_t off, int64_t n, char *out)
 {
 	if (c == NULL || out == NULL || off < 0 || n < 0)
 		return fail("bad argument");
-	if (c->rec_off.empty() || c->hdr_off.size() != c->rec_off.size())
-		return fail(c->rec_off.empty() ? "no database uploaded"
-					       : "no FASTA text on the device: the last upload was not gm_db_upload_fastn or gm_db_upload_fastn_bgzf");
+	if (c->db != DB_FASTN)
+		return fail(c->db == DB_NONE ? "no database uploaded"
+					     : "no FASTA text on the device: the last upload was not gm_db_upload_fastn or gm_db_upload_fastn_bgzf");
 	const int64_t len = c->hdr_off.back();
 	if (off + n > len)
 		return fail("range [%lld, %lld) outside the %lld bytes of text", (long long)off, (long long)(off + n), (long long)len);
@@ -2126,15 +2082,26 @@ extern "C" int gm_db_records(const gm_ctx *c, const int64_t **rec_off, const int
 {
 	if (c == NULL)
 		return fail("ctx is NULL");
-	if (c->rec_off.empty())
+	if (c->db == DB_NONE)
 		return fail("no database uploaded");
 	if (rec_off)
 		*rec_off = c->rec_off.data();
 	if (hdr_off)
-		*hdr_off = c->hdr_off.size() == c->rec_off.size() ? c->hdr_off.data() : NULL;
+		*hdr_off = c->db == DB_FASTN ? c->hdr_off.data() : NULL;
 	if (n_rec)
 		*n_rec = (int)c->rec_off.size() - 1;
 	return 0;
+}
+
+// Where gm_db_get_chars and gm_hit_windows read the batch's characters: 1 = decoded from the 4-bit codes
+// (exact after gm_db_upload_2bit), 0 = as they sit at d_seq_chars, -1 = refused.
+static int char_source(const gm_ctx *c)
+{
+	if (c->db == DB_NONE)
+		return fail("no database uploaded");
+	if (c->db == DB_HOSTPACK)
+		return fail("the device holds no characters after gm_db_upload_chars_hostpack (the caller has them)");
+	return c->db == DB_2BIT ? 1 : 0;
 }
 
 // Characters [off, off + n) of the uploaded batch (forward strand), as fm_sbuf
@@ -2143,17 +2110,17 @@ extern "C" int gm_db_get_chars(gm_ctx *c, int64_t off, int64_t n, char *out)
 {
 	if (c == NULL || out == NULL || off < 0 || n < 0)
 		return fail("bad argument");
-	if (c->d_seq_chars == NULL && !c->codes_exact)
-		return fail(c->up_published >= 0 ? "the device holds no characters after gm_db_upload_chars_hostpack (the caller has them)"
-					   : "no database uploaded");
+	const int codes = char_source(c);
+	if (codes < 0)
+		return -1;
 	if (off + n > c->total_nt)
 		return fail("range [%lld, %lld) outside the %lld uploaded nucleotides", (long long)off, (long long)(off + n),
 			    (long long)c->total_nt);
 	CU(cudaSetDevice(c->device));
 	if (sync_uploads(c))
 		return -1;
-	if (c->codes_exact) {
-		// after gm_db_upload_2bit: the 4-bit codes back, decoded here (a, c, g, t and n are all they hold)
+	if (codes) {
+		// the 4-bit codes back, decoded here (a, c, g, t and n are all they hold)
 		if (n == 0)
 			return 0;
 		const int64_t b0 = off >> 1, b1 = (off + n + 1) >> 1;
@@ -2174,7 +2141,7 @@ extern "C" int gm_db_get_chars(gm_ctx *c, int64_t off, int64_t n, char *out)
 	return 0;
 }
 
-extern "C" int64_t gm_db_total_nt(const gm_ctx *c) { return c ? c->total_nt : -1; }
+extern "C" int64_t gm_db_total_nt(const gm_ctx *c) { return c == NULL ? -1 : c->db == DB_NONE ? 0 : c->total_nt; }
 
 // ------------------------------------------------------------------ scan
 
@@ -2337,7 +2304,7 @@ extern "C" int gm_scan_launch(gm_ctx *c, int64_t g_begin, int64_t g_end, int str
 		return fail("a scan is already in flight");
 	if (strands != 1 && strands != 2)
 		return fail("strands must be 1 or 2");
-	if (c->rec_off.empty())
+	if (c->db == DB_NONE)
 		return fail("no database uploaded");
 	if (g_begin < 0 || g_end > c->total_nt || g_begin > g_end)
 		return fail("range [%lld, %lld) outside the database of %lld nt", (long long)g_begin,
@@ -2614,9 +2581,9 @@ extern "C" int gm_hit_windows(gm_ctx *c, int lead, int trail, const char **win, 
 		return fail("bad argument");
 	if (c->pending)
 		return fail("a scan is in flight");
-	if (c->d_seq_chars == NULL && !c->codes_exact)
-		return fail(c->up_published >= 0 ? "the device holds no characters after gm_db_upload_chars_hostpack (the caller has them)"
-					   : "no database uploaded");
+	const int codes = char_source(c);
+	if (codes < 0)
+		return -1;
 	CU(cudaSetDevice(c->device));
 	NvtxRange nvtx_("gpumotif: hit windows");
 	const int wlen = (lead + c->par.w_winsize + trail + 1 + 7) & ~7;
@@ -2637,7 +2604,7 @@ extern "C" int gm_hit_windows(gm_ctx *c, int lead, int trail, const char **win, 
 		const int blocks = (int)std::min<size_t>(n_dev, (size_t)c->n_sm * 32);
 		// after a 2-bit upload the windows are decoded from the 4-bit codes
 		const uint32_t *h = c->dev_sorted ? c->d_sorted : c->d_hits;
-		if (c->codes_exact)
+		if (codes)
 			gm_window_kernel<true><<<blocks, 128, 0, c->stream>>>(c->d_packed, c->d_rec_off, h, n_dev, c->stride_words, lead, wlen,
 									      c->d_win);
 		else
