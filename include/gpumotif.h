@@ -188,15 +188,43 @@ int gm_db_upload_fastn(gm_ctx *c, const char *text, size_t n_bytes);
  * gm_scan_stats_t::h2d_bytes = n_bytes + the member table (32 bytes a member). */
 int gm_db_upload_fastn_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_bytes);
 
-/* Bytes [off, off + n) of the text of the last gm_db_upload_fastn or
- * gm_db_upload_fastn_bgzf, read back from the device: the ids and definition lines
- * where hdr_off points, for a caller that never had the text on the host.  Refused
- * after the other uploads and outside [0, hdr_off[n_rec]). */
+/* Sequencing reads as four-line FASTQ: `text` is the file's bytes as read from disk; they go
+ * host -> device as they are, and the reads are taken out, the format checked and the
+ * 4-bit pack done there.  The format accepted:
+ *   - every record is four lines: line 4k starts with '@' (the id and description follow),
+ *     line 4k+1 is the read, line 4k+2 starts with '+', line 4k+3 is the quality string;
+ *     multi-line FASTQ is refused.  A line's role is its index mod 4, never its first byte,
+ *     so a quality string that begins with '@' is harmless;
+ *   - every byte of a read line but a trailing '\r' is one nucleotide, so hit coordinates
+ *     are read coordinates and line up with the quality string.  The pack folds case and
+ *     reads u as t as for FASTA; '.' and any other byte that is not an IUPAC letter gets
+ *     code 0 and never pairs.  Quality values are not used;
+ *   - lines end in '\n' or "\r\n"; the line end after the last line is optional.
+ * Record r is the r-th read; hdr_off[r] = the offset of its '@' (hdr_off[n_rec] = n_bytes), so
+ * gm_db_get_text reads read names as it reads FASTA definition lines.  Refused as bad input: a
+ * NULL text with n_bytes > 0, text not beginning with '@', more than 2^40 bytes.  Refused after
+ * the device has read the text, naming the first failing record and the byte offset of its
+ * '@': a line 4k not starting with '@', a line 4k+2 not starting with '+', a quality string
+ * whose length differs from its read's, a last record of fewer than four lines.  Blocks until
+ * the record table is known and checked; the pack runs on asynchronously.
+ * gm_scan_stats_t::h2d_bytes = n_bytes. */
+int gm_db_upload_fastq(gm_ctx *c, const char *text, size_t n_bytes);
+
+/* FASTQ compressed as BGZF: gm_db_upload_fastq(c, T, |T|) where T is the concatenation of the
+ * decompressed members, inflated on the device as gm_db_upload_fastn_bgzf inflates them, with
+ * the same member refusals and messages; hdr_off in T's coordinates.
+ * gm_scan_stats_t::h2d_bytes = n_bytes + the member table (32 bytes a member). */
+int gm_db_upload_fastq_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_bytes);
+
+/* Bytes [off, off + n) of the text of the last gm_db_upload_fastn, gm_db_upload_fastn_bgzf,
+ * gm_db_upload_fastq or gm_db_upload_fastq_bgzf, read back from the device: the ids and
+ * definition lines where hdr_off points, for a caller that never had the text on the host.
+ * Refused after the other uploads and outside [0, hdr_off[n_rec]). */
 int gm_db_get_text(gm_ctx *c, int64_t off, int64_t n, char *out);
 
 /* Record table of the uploaded batch: rec_off[0..n_rec] as in
- * gm_db_upload_chars, and -- after gm_db_upload_fastn or gm_db_upload_fastn_bgzf only,
- * else NULL -- hdr_off[r] = offset in `text` of record r's '>' (hdr_off[n_rec] = n_bytes), so
+ * gm_db_upload_chars, and -- after the FASTA and FASTQ uploads only, else NULL --
+ * hdr_off[r] = offset in `text` of record r's '>' or '@' (hdr_off[n_rec] = n_bytes), so
  * the caller can read ids and definition lines where they lie.  Owned by the
  * context until the next upload. */
 int gm_db_records(const gm_ctx *c, const int64_t **rec_off, const int64_t **hdr_off, int *n_rec);

@@ -27,6 +27,7 @@
 #include "gpumotif.h"
 #include "gm_machine.cuh"
 #include "gm_fastn.cuh"
+#include "gm_fastq.cuh"
 #include "gm_hostpack.h"
 
 using namespace gm;
@@ -60,8 +61,9 @@ struct NvtxRange {
 
 // What the context's database is (gm_ctx::db).  DB_CHARS: characters on the device (d_seq_chars) and
 // their 4-bit codes; DB_HOSTPACK: the codes only; DB_2BIT: codes that decode to characters (a, c, g, t,
-// n); DB_FASTN: FASTA text, its characters, their codes and the header offsets (hdr_off).
-enum DbKind { DB_NONE, DB_CHARS, DB_HOSTPACK, DB_2BIT, DB_FASTN };
+// n); DB_FASTN: FASTA text, its characters, their codes and the header offsets (hdr_off); DB_FASTQ: the
+// same for FASTQ text (hdr_off = each record's '@').
+enum DbKind { DB_NONE, DB_CHARS, DB_HOSTPACK, DB_2BIT, DB_FASTN, DB_FASTQ };
 
 struct gm_ctx {
 	gm_plan_t plan;
@@ -113,7 +115,10 @@ struct gm_ctx {
 	size_t rec_cap;        // bytes
 	std::vector<int64_t> rec_off;
 	int64_t total_nt;
-	// FASTA text parsed on the device (gm_db_upload_fastn)
+	// start_pre[r] = the starts the sieve path searches on one strand of records 0 .. r-1 (index_starts), so
+	// that gm_scan_finish counts a range's starts without a loop over every record
+	std::vector<uint64_t> start_pre;
+	// FASTA or FASTQ text parsed on the device (gm_db_upload_fastn, gm_db_upload_fastq)
 	uint8_t *d_text;
 	size_t text_cap;
 	int64_t *d_hdr_off;
@@ -1429,12 +1434,37 @@ static int check_records(const int64_t *rec_off, int n_rec)
 	return 0;
 }
 
+// Starts per strand of a record of slen nucleotides on the sieve path (RM_find_motif searches szero in
+// [0, slen - rm_dminlen], src/find_motif.c:184-205): the same number on both strands.
+static int64_t record_starts(const gm_ctx *c, int64_t slen)
+{
+	return std::max<int64_t>(0, slen - std::max(c->par.dminlen - 1, 0));
+}
+
+// start_pre for the record table in c->rec_off (the sieve path only: the other paths count their starts
+// on the device)
+static void index_starts(gm_ctx *c)
+{
+	c->start_pre.clear();
+	if (!c->par.sieve)
+		return;
+	const size_t n_rec = c->rec_off.size() - 1;
+	c->start_pre.resize(n_rec + 1);
+	uint64_t s = 0;
+	for (size_t r = 0; r < n_rec; r++) {
+		c->start_pre[r] = s;
+		s += (uint64_t)record_starts(c, c->rec_off[r + 1] - c->rec_off[r]);
+	}
+	c->start_pre[n_rec] = s;
+}
+
 // a record table check_records has passed, on the host and (enqueued) on the device
 static int set_records(gm_ctx *c, const int64_t *rec_off, int n_rec)
 {
 	const size_t tab = (size_t)(n_rec + 1) * sizeof(int64_t);
 	c->rec_off.assign(rec_off, rec_off + n_rec + 1);
 	c->total_nt = rec_off[n_rec];
+	index_starts(c);
 	if (ensure((void **)&c->d_rec_off, &c->rec_cap, tab))
 		return -1;
 	CU(cudaMemcpyAsync(c->d_rec_off, c->rec_off.data(), tab, cudaMemcpyHostToDevice, c->copy_stream));
@@ -1837,6 +1867,20 @@ extern "C" int gm_db_upload_2bit(gm_ctx *c, const uint8_t *dna, size_t n_bytes, 
 	return 0;
 }
 
+// The record table a device text reader has left in c->rec_off: every record under 2^31, then the
+// 4-bit pack, asynchronously.
+static int pack_text_records(gm_ctx *c)
+{
+	const int n_rec = (int)c->rec_off.size() - 1;
+	for (int r = 0; r < n_rec; r++)
+		if (c->rec_off[r + 1] - c->rec_off[r] > 0x7ffffff0ll)
+			return fail("record %d longer than 2^31", r);
+	index_starts(c);
+	if (upload_chunks(c, NULL, c->d_chars, false))
+		return -1;
+	return 0;
+}
+
 // FN_fgetseq on the device, src/dbutil.c:42-128 (gm_fastn.cuh), over the n bytes of FASTA text in
 // d_text (enqueued on copy_stream, or already there): text -> kept characters + record table
 // (rec_off, hdr_off; blocks until they are known) -> 4-bit codes, asynchronously.
@@ -1883,12 +1927,75 @@ static int read_fastn(gm_ctx *c, int64_t n)
 	c->total_nt = (int64_t)tot[0];
 	if (c->rec_off[0] != 0)
 		return fail("fastn text has sequence before its first header");
-	for (int r = 0; r < n_rec; r++)
-		if (c->rec_off[r + 1] - c->rec_off[r] > 0x7ffffff0ll)
-			return fail("record %d longer than 2^31", r);
-	if (upload_chunks(c, NULL, c->d_chars, false))
+	return pack_text_records(c);
+}
+
+// Four-line FASTQ on the device (gm_fastq.cuh) over the first n of the n_bytes of text in d_text (the
+// caller has cut the line end after the last line): reads + record table (rec_off, hdr_off; blocks
+// until they are known and the format is checked) -> 4-bit codes, asynchronously.
+static int read_fastq(gm_ctx *c, int64_t n, int64_t n_bytes)
+{
+	const int n_seg = (int)((n + GM_FASTN_SEG - 1) / GM_FASTN_SEG);
+	if (ensure((void **)&c->d_chars, &c->chars_cap, (size_t)n + 64) ||
+	    ensure(&c->d_fsum, &c->fsum_cap, (size_t)(n_seg + 1) * sizeof(FastqSum) + 32) ||
+	    ensure(&c->d_fstart, &c->fstart_cap, (size_t)(n_seg + 1) * sizeof(FastqSegStart)))
 		return -1;
-	return 0;
+	// totals (read bytes, records), then the first failing record's key (record << 2 | what)
+	unsigned long long *d_tot = reinterpret_cast<unsigned long long *>(
+		static_cast<uint8_t *>(c->d_fsum) + (size_t)(n_seg + 1) * sizeof(FastqSum));
+	unsigned long long tot[2] = {0, 0}, bad = ~0ull;
+	CU(cudaMemsetAsync(d_tot + 2, 0xff, sizeof(unsigned long long), c->copy_stream));
+	if (n > 0) {
+		const int blocks = (n_seg * 32 + 255) / 256;
+		gm_fastq_summarize<<<blocks, 256, 0, c->copy_stream>>>(c->d_text, n, static_cast<FastqSum *>(c->d_fsum), n_seg);
+		CU(cudaGetLastError());
+		gm_fastq_scan<<<1, GM_FQ_SCAN_THREADS, 0, c->copy_stream>>>(static_cast<const FastqSum *>(c->d_fsum), n_seg,
+			static_cast<FastqSegStart *>(c->d_fstart), d_tot, d_tot + 2);
+		CU(cudaGetLastError());
+		CU(cudaMemcpyAsync(tot, d_tot, sizeof tot, cudaMemcpyDeviceToHost, c->copy_stream));
+		CU(cudaStreamSynchronize(c->copy_stream));
+	}
+	if (tot[1] > 0x7ffffff0ull)
+		return fail("too many records in one upload");
+	const int n_rec = (int)tot[1];
+	const size_t tab = (size_t)(n_rec + 1) * sizeof(int64_t);
+	if (ensure((void **)&c->d_rec_off, &c->rec_cap, tab) || ensure((void **)&c->d_hdr_off, &c->hdr_cap, tab))
+		return -1;
+	c->rec_off.resize(n_rec + 1);
+	c->hdr_off.resize(n_rec + 1);
+	// record 0 starts at byte 0 and character 0; gm_fastq_emit writes every other record's entries
+	const int64_t first = 0, last[2] = {(int64_t)tot[0], n_bytes};
+	if (n_rec > 0) {
+		CU(cudaMemcpyAsync(c->d_rec_off, &first, sizeof(int64_t), cudaMemcpyHostToDevice, c->copy_stream));
+		CU(cudaMemcpyAsync(c->d_hdr_off, &first, sizeof(int64_t), cudaMemcpyHostToDevice, c->copy_stream));
+		const int blocks = (n_seg * 32 + 255) / 256;
+		gm_fastq_emit<<<blocks, 256, 0, c->copy_stream>>>(c->d_text, n, static_cast<const FastqSegStart *>(c->d_fstart),
+			n_seg, c->d_chars, c->d_rec_off, c->d_hdr_off, d_tot + 2);
+		CU(cudaGetLastError());
+	}
+	CU(cudaMemcpyAsync(c->d_rec_off + n_rec, &last[0], sizeof(int64_t), cudaMemcpyHostToDevice, c->copy_stream));
+	CU(cudaMemcpyAsync(c->d_hdr_off + n_rec, &last[1], sizeof(int64_t), cudaMemcpyHostToDevice, c->copy_stream));
+	CU(cudaMemcpyAsync(c->rec_off.data(), c->d_rec_off, tab, cudaMemcpyDeviceToHost, c->copy_stream));
+	CU(cudaMemcpyAsync(c->hdr_off.data(), c->d_hdr_off, tab, cudaMemcpyDeviceToHost, c->copy_stream));
+	CU(cudaMemcpyAsync(&bad, d_tot + 2, sizeof bad, cudaMemcpyDeviceToHost, c->copy_stream));
+	CU(cudaStreamSynchronize(c->copy_stream));
+	c->total_nt = (int64_t)tot[0];
+	if (bad != ~0ull) {
+		const long long r = (long long)(bad >> 2);
+		const long long at = (long long)c->hdr_off[r];
+		switch ((int)(bad & 3)) {
+		case GM_FQ_AT:
+			return fail("FASTQ record %lld at byte %lld: line %lld does not start with '@'", r, at, 4 * r + 1);
+		case GM_FQ_PLUS:
+			return fail("FASTQ record %lld at byte %lld: line %lld does not start with '+' (only four-line FASTQ is "
+				    "accepted)", r, at, 4 * r + 3);
+		case GM_FQ_QLEN:
+			return fail("FASTQ record %lld at byte %lld: its quality string is not as long as its read", r, at);
+		default:
+			return fail("FASTQ record %lld at byte %lld: the last record has fewer than four lines", r, at);
+		}
+	}
+	return pack_text_records(c);
 }
 
 extern "C" int gm_db_upload_fastn(gm_ctx *c, const char *text, size_t n_bytes)
@@ -1914,19 +2021,52 @@ extern "C" int gm_db_upload_fastn(gm_ctx *c, const char *text, size_t n_bytes)
 	return 0;
 }
 
+// FASTQ text without the line end after its last line ('\n', '\r\n' or '\r'): the length the reader
+// reads, from the last two bytes alone
+static int64_t fastq_trim(int64_t n, uint8_t b1, uint8_t b2)
+{
+	if (n > 0 && b2 == '\n') {
+		n--;
+		b2 = b1;
+	}
+	if (n > 0 && b2 == '\r')
+		n--;
+	return n;
+}
+
+extern "C" int gm_db_upload_fastq(gm_ctx *c, const char *text, size_t n_bytes)
+{
+	if (n_bytes > 0 && text == NULL)
+		return fail("text is NULL");
+	if (n_bytes > ((size_t)1 << 40))
+		return fail("text too long");
+	if (n_bytes > 0 && text[0] != '@')
+		return fail("FASTQ text does not begin with '@'");
+	if (begin_upload(c))
+		return -1;
+	NvtxRange nvtx_("gpumotif: upload FASTQ (H2D + device reader)");
+	if (ensure((void **)&c->d_text, &c->text_cap, n_bytes + 64))
+		return -1;
+	CU(cudaEventRecord(c->up_ev[0], c->copy_stream));
+	if (n_bytes > 0)
+		CU(cudaMemcpyAsync(c->d_text, text, n_bytes, cudaMemcpyHostToDevice, c->copy_stream));
+	const int64_t n = (int64_t)n_bytes;
+	if (read_fastq(c, fastq_trim(n, n > 1 ? text[n - 2] : 0, n > 0 ? text[n - 1] : 0), n))
+		return -1;
+	c->stats.h2d_bytes = (uint64_t)n_bytes;
+	c->db = DB_FASTQ;
+	return 0;
+}
+
 static uint32_t le32(const uint8_t *p) { return p[0] | (p[1] << 8) | (p[2] << 16) | ((uint32_t)p[3] << 24); }
 
 // BGZF: the member table comes from the headers alone (each member's trailer gives its output
-// size, so its offset in the text is known), the compressed bytes go over in chunks of whole
-// members, and gm_inflate_kernel inflates chunk i on pack_stream behind its copy while chunk i+1
-// is copying.  Then the text is read as gm_db_upload_fastn reads it.
-extern "C" int gm_db_upload_fastn_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_bytes)
+// size, so its offset in the text is known).  Host checks only; *total = the text's length.
+static int bgzf_members(const uint8_t *gz, size_t n_bytes, std::vector<BgzfMember> &mem, std::vector<size_t> &starts,
+			uint64_t *total_out)
 {
 	if (n_bytes > 0 && gz == NULL)
 		return fail("gz is NULL");
-	// the member table
-	std::vector<BgzfMember> mem;
-	std::vector<size_t> starts; // each member's offset in gz
 	uint64_t total = 0;
 	for (size_t p = 0; p < n_bytes;) {
 		const size_t left = n_bytes - p;
@@ -1992,9 +2132,21 @@ extern "C" int gm_db_upload_fastn_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_by
 	}
 	if (mem.size() > 0x7fffffffu)
 		return fail("too many BGZF members");
-	if (begin_upload(c))
-		return -1;
-	NvtxRange nvtx_("gpumotif: upload BGZF fastn (H2D + inflate + device reader)");
+	*total_out = total;
+	return 0;
+}
+
+// The first byte and the last two of the inflated text (0 where the text is shorter)
+struct TextEnds {
+	uint8_t head, tail[2];
+};
+
+// The members of bgzf_members into d_text, after begin_upload: the compressed bytes go over in chunks
+// of whole members, and gm_inflate_kernel inflates chunk i on pack_stream behind its copy while chunk
+// i+1 is copying.  Blocks until every member is checked; an inflate error names the first failing one.
+static int inflate_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_bytes, std::vector<BgzfMember> &mem,
+			const std::vector<size_t> &starts, uint64_t total, TextEnds *ends)
+{
 	const int n_mem = (int)mem.size();
 	const size_t tab = (size_t)n_mem * sizeof(BgzfMember);
 	if (ensure((void **)&c->d_text, &c->text_cap, (size_t)total + 64) || ensure((void **)&c->d_gz, &c->gz_cap, n_bytes + 16) ||
@@ -2004,55 +2156,77 @@ extern "C" int gm_db_upload_fastn_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_by
 	BgzfMember *d_mem = static_cast<BgzfMember *>(c->d_bgzf);
 	unsigned int *d_first = reinterpret_cast<unsigned int *>(static_cast<uint8_t *>(c->d_bgzf) + tab);
 	uint8_t *d_status = static_cast<uint8_t *>(c->d_bgzf) + tab + 8;
+	*ends = TextEnds{0, {0, 0}};
 	CU(cudaEventRecord(c->up_ev[0], c->copy_stream));
-	if (n_mem > 0) {
-		CU(cudaMemcpyAsync(d_mem, c->bgzf.data(), tab, cudaMemcpyHostToDevice, c->copy_stream));
-		CU(cudaMemsetAsync(d_first, 0xff, sizeof(unsigned int), c->copy_stream));
-		// chunks of the compressed bytes (at least 64 MiB, at most 16; GPUMOTIF_CHUNK_NT lowers the
-		// floor), each ending where the first member starting at or after its cut begins
-		int64_t chunk;
-		if (cut_chunks(c, (int64_t)n_bytes, (int64_t)64 << 20, 16, 1, true, &chunk))
-			return -1;
-		const int n_chunks = (int)c->chunk_end.size();
-		int m0 = 0;
-		size_t copied = 0;
-		for (int i = 0; i < n_chunks; i++) {
-			int m1 = m0;
-			while (m1 < n_mem && (i == n_chunks - 1 || (int64_t)starts[m1] < c->chunk_end[i]))
-				m1++;
-			const size_t upto = m1 < n_mem ? starts[m1] : n_bytes;
-			if (upto > copied)
-				CU(cudaMemcpyAsync(c->d_gz + copied, gz + copied, upto - copied, cudaMemcpyHostToDevice, c->copy_stream));
-			copied = std::max(copied, upto);
-			CU(cudaEventRecord(c->cp_ev[i], c->copy_stream));
-			if (m1 > m0) {
-				CU(cudaStreamWaitEvent(c->pack_stream, c->cp_ev[i], 0));
-				// one thread per member, spread over the SMs: the decode is a chain of dependent loads
-				const int m = m1 - m0;
-				const int tpb = std::min(32, std::max(1, (m + c->n_sm - 1) / c->n_sm));
-				gm_inflate_kernel<<<(m + tpb - 1) / tpb, tpb, 0, c->pack_stream>>>(c->d_gz, d_mem, m0, m1, c->d_text, d_status,
-												    d_first);
-				CU(cudaGetLastError());
-			}
-			m0 = m1;
+	if (n_mem == 0)
+		return 0;
+	CU(cudaMemcpyAsync(d_mem, c->bgzf.data(), tab, cudaMemcpyHostToDevice, c->copy_stream));
+	CU(cudaMemsetAsync(d_first, 0xff, sizeof(unsigned int), c->copy_stream));
+	// chunks of the compressed bytes (at least 64 MiB, at most 16; GPUMOTIF_CHUNK_NT lowers the
+	// floor), each ending where the first member starting at or after its cut begins
+	int64_t chunk;
+	if (cut_chunks(c, (int64_t)n_bytes, (int64_t)64 << 20, 16, 1, true, &chunk))
+		return -1;
+	const int n_chunks = (int)c->chunk_end.size();
+	int m0 = 0;
+	size_t copied = 0;
+	for (int i = 0; i < n_chunks; i++) {
+		int m1 = m0;
+		while (m1 < n_mem && (i == n_chunks - 1 || (int64_t)starts[m1] < c->chunk_end[i]))
+			m1++;
+		const size_t upto = m1 < n_mem ? starts[m1] : n_bytes;
+		if (upto > copied)
+			CU(cudaMemcpyAsync(c->d_gz + copied, gz + copied, upto - copied, cudaMemcpyHostToDevice, c->copy_stream));
+		copied = std::max(copied, upto);
+		CU(cudaEventRecord(c->cp_ev[i], c->copy_stream));
+		if (m1 > m0) {
+			CU(cudaStreamWaitEvent(c->pack_stream, c->cp_ev[i], 0));
+			// one thread per member, spread over the SMs: the decode is a chain of dependent loads
+			const int m = m1 - m0;
+			const int tpb = std::min(32, std::max(1, (m + c->n_sm - 1) / c->n_sm));
+			gm_inflate_kernel<<<(m + tpb - 1) / tpb, tpb, 0, c->pack_stream>>>(c->d_gz, d_mem, m0, m1, c->d_text, d_status,
+											    d_first);
+			CU(cudaGetLastError());
 		}
-		// the first failing member, its status and the text's first byte
-		struct {
-			unsigned int first;
-			uint8_t st, ch;
-		} res = {0xffffffffu, 0, '>'};
-		CU(cudaMemcpyAsync(&res.first, d_first, sizeof res.first, cudaMemcpyDeviceToHost, c->pack_stream));
-		if (total > 0)
-			CU(cudaMemcpyAsync(&res.ch, c->d_text, 1, cudaMemcpyDeviceToHost, c->pack_stream));
-		CU(cudaStreamSynchronize(c->pack_stream));
-		if (res.first != 0xffffffffu) {
-			const unsigned int k = res.first;
-			CU(cudaMemcpy(&res.st, d_status + k, 1, cudaMemcpyDeviceToHost));
-			return fail("BGZF member %u at byte %zu: %s", k, starts[k], inflate_status_name(res.st));
-		}
-		if (res.ch != '>')
-			return fail("the text of the BGZF members does not begin with '>' (src/dbutil.c:56-60)");
+		m0 = m1;
 	}
+	// the first failing member, its status and the text's ends
+	struct {
+		unsigned int first;
+		uint8_t st;
+	} res = {0xffffffffu, 0};
+	CU(cudaMemcpyAsync(&res.first, d_first, sizeof res.first, cudaMemcpyDeviceToHost, c->pack_stream));
+	if (total > 0)
+		CU(cudaMemcpyAsync(&ends->head, c->d_text, 1, cudaMemcpyDeviceToHost, c->pack_stream));
+	const size_t nt = (size_t)std::min<uint64_t>(total, 2);
+	if (nt > 0)
+		CU(cudaMemcpyAsync(ends->tail + 2 - nt, c->d_text + total - nt, nt, cudaMemcpyDeviceToHost, c->pack_stream));
+	CU(cudaStreamSynchronize(c->pack_stream));
+	if (res.first != 0xffffffffu) {
+		const unsigned int k = res.first;
+		CU(cudaMemcpy(&res.st, d_status + k, 1, cudaMemcpyDeviceToHost));
+		return fail("BGZF member %u at byte %zu: %s", k, starts[k], inflate_status_name(res.st));
+	}
+	return 0;
+}
+
+// The members inflated as above, then the text read as gm_db_upload_fastn reads it.
+extern "C" int gm_db_upload_fastn_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_bytes)
+{
+	std::vector<BgzfMember> mem;
+	std::vector<size_t> starts; // each member's offset in gz
+	uint64_t total = 0;
+	if (bgzf_members(gz, n_bytes, mem, starts, &total))
+		return -1;
+	if (begin_upload(c))
+		return -1;
+	NvtxRange nvtx_("gpumotif: upload BGZF fastn (H2D + inflate + device reader)");
+	const size_t tab = mem.size() * sizeof(BgzfMember);
+	TextEnds ends;
+	if (inflate_bgzf(c, gz, n_bytes, mem, starts, total, &ends))
+		return -1;
+	if (total > 0 && ends.head != '>')
+		return fail("the text of the BGZF members does not begin with '>' (src/dbutil.c:56-60)");
 	if (read_fastn(c, (int64_t)total))
 		return -1;
 	c->stats.h2d_bytes = (uint64_t)n_bytes + (uint64_t)tab;
@@ -2060,13 +2234,38 @@ extern "C" int gm_db_upload_fastn_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_by
 	return 0;
 }
 
+// The members inflated as above, then the text read as gm_db_upload_fastq reads it.
+extern "C" int gm_db_upload_fastq_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_bytes)
+{
+	std::vector<BgzfMember> mem;
+	std::vector<size_t> starts; // each member's offset in gz
+	uint64_t total = 0;
+	if (bgzf_members(gz, n_bytes, mem, starts, &total))
+		return -1;
+	if (begin_upload(c))
+		return -1;
+	NvtxRange nvtx_("gpumotif: upload BGZF FASTQ (H2D + inflate + device reader)");
+	const size_t tab = mem.size() * sizeof(BgzfMember);
+	TextEnds ends;
+	if (inflate_bgzf(c, gz, n_bytes, mem, starts, total, &ends))
+		return -1;
+	if (total > 0 && ends.head != '@')
+		return fail("the text of the BGZF members does not begin with '@'");
+	if (read_fastq(c, fastq_trim((int64_t)total, ends.tail[0], ends.tail[1]), (int64_t)total))
+		return -1;
+	c->stats.h2d_bytes = (uint64_t)n_bytes + (uint64_t)tab;
+	c->db = DB_FASTQ;
+	return 0;
+}
+
 extern "C" int gm_db_get_text(gm_ctx *c, int64_t off, int64_t n, char *out)
 {
 	if (c == NULL || out == NULL || off < 0 || n < 0)
 		return fail("bad argument");
-	if (c->db != DB_FASTN)
+	if (c->db != DB_FASTN && c->db != DB_FASTQ)
 		return fail(c->db == DB_NONE ? "no database uploaded"
-					     : "no FASTA text on the device: the last upload was not gm_db_upload_fastn or gm_db_upload_fastn_bgzf");
+					     : "no FASTA or FASTQ text on the device: the last upload was not gm_db_upload_fastn, "
+					       "gm_db_upload_fastn_bgzf, gm_db_upload_fastq or gm_db_upload_fastq_bgzf");
 	const int64_t len = c->hdr_off.back();
 	if (off + n > len)
 		return fail("range [%lld, %lld) outside the %lld bytes of text", (long long)off, (long long)(off + n), (long long)len);
@@ -2087,7 +2286,7 @@ extern "C" int gm_db_records(const gm_ctx *c, const int64_t **rec_off, const int
 	if (rec_off)
 		*rec_off = c->rec_off.data();
 	if (hdr_off)
-		*hdr_off = c->db == DB_FASTN ? c->hdr_off.data() : NULL;
+		*hdr_off = c->db == DB_FASTN || c->db == DB_FASTQ ? c->hdr_off.data() : NULL;
 	if (n_rec)
 		*n_rec = (int)c->rec_off.size() - 1;
 	return 0;
@@ -2526,16 +2725,19 @@ extern "C" int gm_scan_finish(gm_ctx *c)
 	c->stats.n_starts = cnt[2];
 	if (c->par.sieve) {
 		// the sieve does not visit the starts one by one: count them here
-		// (RM_find_motif searches szero in [0, slen - rm_dminlen], src/find_motif.c:184-205)
+		// (RM_find_motif searches szero in [0, slen - rm_dminlen], src/find_motif.c:184-205).
+		// Records wholly inside the range come from start_pre; the (at most two) it cuts are counted
+		// one position at a time.
 		uint64_t ns = 0;
-		for (size_t r = 0; r + 1 < c->rec_off.size(); r++) {
-			const int64_t lo = std::max(c->rec_off[r], c->p_begin);
-			const int64_t hi = std::min(c->rec_off[r + 1], c->p_end);
+		const std::vector<int64_t> &ro = c->rec_off;
+		auto part = [&](size_t r) {
+			const int64_t lo = std::max(ro[r], c->p_begin);
+			const int64_t hi = std::min(ro[r + 1], c->p_end);
 			if (hi <= lo)
-				continue;
+				return;
 			// forward strand: position pos is a start if slen - pos >= dminlen; the
 			// complementary strand maps pos to szero = slen - 1 - pos
-			const int64_t off = c->rec_off[r], slen = c->rec_off[r + 1] - off, dm = c->par.dminlen;
+			const int64_t off = ro[r], slen = ro[r + 1] - off, dm = c->par.dminlen;
 			const int64_t f_hi = std::min(hi, off + slen - dm + 1);
 			if (f_hi > lo)
 				ns += (uint64_t)(f_hi - lo);
@@ -2543,6 +2745,17 @@ extern "C" int gm_scan_finish(gm_ctx *c)
 				const int64_t c_lo = std::max(lo, off + dm - 1);
 				if (hi > c_lo)
 					ns += (uint64_t)(hi - c_lo);
+			}
+		};
+		if (c->p_end > c->p_begin) {
+			// records a and b hold the range's first and last nucleotides
+			const size_t a = (size_t)(std::upper_bound(ro.begin(), ro.end(), c->p_begin) - ro.begin()) - 1;
+			const size_t b = (size_t)(std::upper_bound(ro.begin(), ro.end(), c->p_end - 1) - ro.begin()) - 1;
+			part(a);
+			if (b > a) {
+				part(b);
+				if (b > a + 1)
+					ns += (c->start_pre[b] - c->start_pre[a + 1]) * (uint64_t)c->p_strands;
 			}
 		}
 		c->stats.n_starts = ns;

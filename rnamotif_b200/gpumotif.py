@@ -37,7 +37,7 @@ _lib = None
 
 EXPORTS = ["gm_last_error", "gm_version", "gm_device_count", "gm_host_alloc", "gm_host_free", "gm_ctx_create", "gm_ctx_destroy",
            "gm_plan_check", "gm_plan_describe", "gm_db_upload_chars", "gm_db_upload_chars_hostpack", "gm_host_pack", "gm_db_set_device_chars", "gm_db_upload_fastn",
-           "gm_db_upload_2bit", "gm_db_upload_fastn_bgzf", "gm_db_get_text",
+           "gm_db_upload_2bit", "gm_db_upload_fastn_bgzf", "gm_db_upload_fastq", "gm_db_upload_fastq_bgzf", "gm_db_get_text",
            "gm_db_records", "gm_db_get_chars", "gm_db_total_nt", "gm_hit_windows",
            "gm_scan", "gm_scan_launch", "gm_scan_finish", "gm_hits", "gm_stats",
            "gm_set_hit_capacity", "gm_set_tile", "gm_stream", "gm_prune_hits", "gm_order_hits",
@@ -66,6 +66,8 @@ def lib():
         L.gm_db_upload_2bit.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
                                         C.c_int64]
         L.gm_db_upload_fastn_bgzf.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
+        L.gm_db_upload_fastq.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
+        L.gm_db_upload_fastq_bgzf.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
         L.gm_db_get_text.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p]
         L.gm_db_records.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_int)]
         L.gm_hit_windows.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]
@@ -272,9 +274,33 @@ class MotifSearch:
     def upload_fastn_bgzf_ptr(self, host_ptr: int, n_bytes: int):
         self._ck(lib().gm_db_upload_fastn_bgzf(self._ctx, host_ptr, n_bytes), "gm_db_upload_fastn_bgzf")
 
+    def upload_fastq(self, text):
+        """gm_db_upload_fastq: `text` = four-line FASTQ as it sits in the file (bytes or a uint8
+        array); the reads are taken out and the format is checked on the device."""
+        if isinstance(text, (bytes, bytearray, memoryview)):
+            text = np.frombuffer(text, dtype=np.uint8)
+        text = np.ascontiguousarray(text, dtype=np.uint8)
+        self._keep = text
+        self.upload_fastq_ptr(text.ctypes.data, text.size)
+
+    def upload_fastq_ptr(self, host_ptr: int, n_bytes: int):
+        self._ck(lib().gm_db_upload_fastq(self._ctx, host_ptr, n_bytes), "gm_db_upload_fastq")
+
+    def upload_fastq_bgzf(self, buf):
+        """gm_db_upload_fastq_bgzf: `buf` = a BGZF-compressed FASTQ file's bytes (bytes or a uint8
+        array, pinned or pageable); the members are inflated and read on the device.  Returns when
+        the record table is known, so `buf` may be reused."""
+        if isinstance(buf, (bytes, bytearray, memoryview)):
+            buf = np.frombuffer(buf, dtype=np.uint8)
+        buf = np.ascontiguousarray(buf, dtype=np.uint8)
+        self.upload_fastq_bgzf_ptr(buf.ctypes.data, buf.size)
+
+    def upload_fastq_bgzf_ptr(self, host_ptr: int, n_bytes: int):
+        self._ck(lib().gm_db_upload_fastq_bgzf(self._ctx, host_ptr, n_bytes), "gm_db_upload_fastq_bgzf")
+
     def get_text(self, off: int = 0, n: int | None = None) -> bytes:
-        """gm_db_get_text: bytes [off, off + n) of the FASTA text of the last upload_fastn or
-        upload_fastn_bgzf (n = None: to the end)."""
+        """gm_db_get_text: bytes [off, off + n) of the FASTA or FASTQ text of the last upload_fastn,
+        upload_fastn_bgzf, upload_fastq or upload_fastq_bgzf (n = None: to the end)."""
         if n is None:
             _, hdr = self.records()
             n = (int(hdr[-1]) if hdr is not None else 0) - off
@@ -284,7 +310,7 @@ class MotifSearch:
 
     def records(self):
         """(rec_off, hdr_off) of the uploaded batch; hdr_off is None unless it came
-        through upload_fastn or upload_fastn_bgzf."""
+        through upload_fastn, upload_fastn_bgzf, upload_fastq or upload_fastq_bgzf."""
         ro, ho, n = C.c_void_p(), C.c_void_p(), C.c_int()
         self._ck(lib().gm_db_records(self._ctx, C.byref(ro), C.byref(ho), C.byref(n)), "gm_db_records")
         m = n.value + 1

@@ -59,3 +59,39 @@ GOLDEN_LENGTHS = [5, 0, 21, 22, 45, 46, 62, 63, 64, 94, 95, 96, 101, 118, 119, 2
 def golden_db():
     """The database the committed golden candidate streams were produced on."""
     return random_records(20261018, GOLDEN_LENGTHS, planted=True, iupac_rate=0.004)
+
+
+_COMP_TABLE = np.arange(256, dtype=np.uint8)
+for _a, _b in _COMP.items():
+    _COMP_TABLE[_a] = _b
+
+
+def random_reads(seed: int, lengths, stem_every: int = 120, n_rate: float = 0.002, dot_rate: float = 0.0005):
+    """Seeded sequencing reads: i.i.d. acgt, with a stem-loop planted every `stem_every` nt on average
+    (stems of 3..10 nt, loops of 3..12, placed over the concatenation so that some straddle reads)
+    and no-calls -- 'N' at n_rate and '.' at dot_rate.  Vectorised, so that a profile can draw
+    1 Gnt.  Returns (ids, seq uint8 (characters), rec_off int64)."""
+    rng = np.random.default_rng(seed)
+    lengths = np.asarray(lengths, dtype=np.int64)
+    off = np.zeros(len(lengths) + 1, dtype=np.int64)
+    np.cumsum(lengths, out=off[1:])
+    n = int(off[-1])
+    seq = _ACGT[rng.integers(0, 4, size=n, dtype=np.uint8)]
+    if stem_every > 0 and n > 40:
+        per = 1 << 22  # stems per batch (bounds the index arrays)
+        todo = n // stem_every
+        while todo > 0:
+            k = min(todo, per)
+            todo -= k
+            stem = int(rng.integers(3, 11))
+            loop = int(rng.integers(3, 13))
+            span = 2 * stem + loop
+            p = rng.integers(0, n - span, size=k)
+            j = np.arange(stem)
+            left = seq[p[:, None] + j]
+            seq[p[:, None] + span - 1 - j] = _COMP_TABLE[left]
+    for ch, rate in ((ord("N"), n_rate), (ord("."), dot_rate)):
+        if rate > 0 and n > 0:
+            seq[rng.integers(0, n, size=rng.binomial(n, rate))] = ch
+    ids = ["read%d" % i for i in range(len(lengths))]
+    return ids, seq, off
