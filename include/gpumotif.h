@@ -207,14 +207,34 @@ int gm_db_upload_fastn_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_bytes);
  * '@': a line 4k not starting with '@', a line 4k+2 not starting with '+', a quality string
  * whose length differs from its read's, a last record of fewer than four lines.  Blocks until
  * the record table is known and checked; the pack runs on asynchronously.
- * gm_scan_stats_t::h2d_bytes = n_bytes. */
+ * gm_scan_stats_t::h2d_bytes = n_bytes.  Low-quality bases read as n when the context has a
+ * minimum base quality (gm_ctx_set_min_quality). */
 int gm_db_upload_fastq(gm_ctx *c, const char *text, size_t n_bytes);
 
 /* FASTQ compressed as BGZF: gm_db_upload_fastq(c, T, |T|) where T is the concatenation of the
  * decompressed members, inflated on the device as gm_db_upload_fastn_bgzf inflates them, with
  * the same member refusals and messages; hdr_off in T's coordinates.
- * gm_scan_stats_t::h2d_bytes = n_bytes + the member table (32 bytes a member). */
+ * gm_scan_stats_t::h2d_bytes = n_bytes + the member table (32 bytes a member).  Masks
+ * low-quality bases as gm_db_upload_fastq does (gm_ctx_set_min_quality). */
 int gm_db_upload_fastq_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_bytes);
+
+/* Mask low-quality bases of the FASTQ uploads: from the next gm_db_upload_fastq or
+ * gm_db_upload_fastq_bgzf on, base i of a read reads as n exactly when its quality byte q_i
+ * (byte i of the record's quality string) has q_i - qual_offset < min_qual.  "Reads as n":
+ * the scans, the score pre-screen, gm_db_get_chars and gm_hit_windows (mk_rcmp's letter for
+ * n on the complementary strand) see what they would see with n on the read line, whatever
+ * the byte there was.  gm_db_get_text still returns the text as it is, and gm_db_records and
+ * h2d_bytes do not change.  With masking on, a quality byte outside [qual_offset, 126] (a
+ * Phred+33 file read with offset 64, say) is refused on the device: "FASTQ record R at byte
+ * B: quality byte V is outside [qual_offset, 126]", naming the first record with such a byte
+ * and the offset of its '@'; a record before it, or the record itself, failing a format
+ * check is named with that check's message instead.  After the refusal the context holds no
+ * database.  min_qual = 0, the default, switches masking off: the uploads then do exactly
+ * what they do without this call.  qual_offset: 33 (Sanger, Illumina 1.8+) or 64 (Illumina
+ * 1.3-1.7).  Refused, leaving the setting as it was: a NULL context, any other offset,
+ * min_qual < 0 or > 126 - qual_offset.  The database the context holds does not change, and
+ * the other uploads ignore the setting. */
+int gm_ctx_set_min_quality(gm_ctx *c, int min_qual, int qual_offset);
 
 /* Bytes [off, off + n) of the text of the last gm_db_upload_fastn, gm_db_upload_fastn_bgzf,
  * gm_db_upload_fastq or gm_db_upload_fastq_bgzf, read back from the device: the ids and

@@ -20,9 +20,20 @@ any timing.  The legs run in one process, alternating step by step after a warm-
 The candidate arrays of all legs and the resident run must be byte-equal, else the script fails.
 ire and score.1 run with their score pre-screen on, as bench.py's configs do.
 
-    python profiles/fastq_e2e.py --out DIR [--steps 5] [--warmup 1] [--mnt 1000]
+--min-qual Q adds three legs with low-quality masking (gm_ctx_set_min_quality, offset 33) at Q,
+alternating with the others:
+    chars_q   gm_db_upload_chars         the reads with every base of quality below Q written as n
+                                         on the host
+    fastq_q   gm_db_upload_fastq         the FASTQ text, masked on the device
+    bgzf6_q   gm_db_upload_fastq_bgzf    the level-6 BGZF text, masked on the device
+whose candidate arrays must be byte-equal to each other (fastq_q and bgzf6_q to chars_q), else the
+script fails.  Comparing upload_ms of fastq with fastq_q, and of bgzf6 with bgzf6_q, gives what the
+masking pass costs the upload call.
 
-writes DIR/fastq_e2e.json with the card's name, power limit and SM clock, queried in the same run.
+    python profiles/fastq_e2e.py --out DIR [--steps 5] [--warmup 1] [--mnt 1000] [--min-qual Q]
+
+writes DIR/fastq_e2e.json (with --min-qual: DIR/fastq_mask_e2e.json) with the card's name, power
+limit and SM clock, queried in the same run.
 """
 import argparse
 import concurrent.futures
@@ -41,6 +52,7 @@ from rnamotif_b200 import bgzf, fastq, gpumotif, synth  # noqa: E402
 from bgzf_e2e import card, load, pinned, WORKLOADS  # noqa: E402
 
 LEGS = ["chars", "fastq", "bgzf6", "bgzf1"]
+MASKED_LEGS = ["chars_q", "fastq_q", "bgzf6_q"]
 READ = 150
 ID_DIGITS = 9
 
@@ -78,7 +90,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=1)
     ap.add_argument("--mnt", type=int, default=1000, help="Mnt of reads")
     ap.add_argument("--workloads", default=",".join(WORKLOADS))
+    ap.add_argument("--min-qual", type=int, default=0, help="add the masked legs at this minimum base quality")
     args = ap.parse_args()
+    if not 0 <= args.min_qual <= 93:
+        raise SystemExit("fastq_e2e.py: --min-qual must be in [0, 93]")
+    legs_run = LEGS + (MASKED_LEGS if args.min_qual else [])
     import torch
     if not torch.cuda.is_available():
         raise SystemExit("fastq_e2e.py: no CUDA device; libgpumotif has no CPU path")
@@ -100,6 +116,12 @@ def main():
         ["read%09d" % i for i in range(k)], seq, rec_off[:k + 1], [qual[i * READ:(i + 1) * READ] for i in range(k)])
     assert (fastq.parse_fastq(text[:k * (len(text) // n_reads)].tobytes())[2] == rec_off[:k + 1]).all()
     h_chars = pinned(seq.tobytes())
+    if args.min_qual:
+        seq_q = seq.copy()
+        seq_q[qual < 33 + args.min_qual] = ord("n")
+        masked_share = float((qual < 33 + args.min_qual).mean())
+        h_chars_q = pinned(seq_q.tobytes())
+        del seq_q
     h_text = pinned(text.tobytes())
     threads = len(os.sched_getaffinity(0))
     gz = {lv: pinned(compress(memoryview(text), lv, threads)) for lv in (6, 1)}
@@ -116,6 +138,8 @@ def main():
            "steps": args.steps, "warmup": args.warmup, "timing": "host clock around upload + gm_scan (which ends in a "
            "device synchronise and leaves the sorted candidates in host memory), legs alternating step by step; "
            "upload_ms: the upload call alone", "cpus": threads, "prep_s": t_prep, "workloads": []}
+    if args.min_qual:
+        res["min_qual"] = {"min_qual": args.min_qual, "qual_offset": 33, "bases_masked": masked_share}
     ok_all = True
     for name in args.workloads.split(","):
         plan, score = load(name, "plan"), load(name, "score")
@@ -129,11 +153,19 @@ def main():
             "bgzf6": lambda: ms.upload_fastq_bgzf_ptr(gz[6].data_ptr(), gz[6].numel()),
             "bgzf1": lambda: ms.upload_fastq_bgzf_ptr(gz[1].data_ptr(), gz[1].numel()),
         }
+        if args.min_qual:
+            legs |= {
+                "chars_q": lambda: ms.upload_ptr(h_chars_q.data_ptr(), rec_off),
+                "fastq_q": legs["fastq"],
+                "bgzf6_q": legs["bgzf6"],
+            }
         times = {k: [] for k in legs}
         t_up = {k: [] for k in legs}
         h2d, hits = {}, {}
 
         def step(leg):
+            if args.min_qual:
+                ms.set_min_quality(args.min_qual if leg in MASKED_LEGS else 0)
             torch.cuda.synchronize()
             t = time.perf_counter()
             legs[leg]()
@@ -176,7 +208,10 @@ def main():
             t_small.append(time.perf_counter() - t)
         ms.close()
         ref = hits["resident"].tobytes()
-        same = {k: v.tobytes() == ref for k, v in hits.items()}
+        same = {k: v.tobytes() == ref for k, v in hits.items() if k not in MASKED_LEGS}
+        if args.min_qual:
+            ref_q = hits["chars_q"].tobytes()
+            same |= {k: hits[k].tobytes() == ref_q for k in MASKED_LEGS[1:]}
         ok_all = ok_all and all(same.values())
         work = float(total) * strands
         entry = {"workload": name, "strands": strands, "score_prescreen": score is not None,
@@ -184,6 +219,8 @@ def main():
                  "resident": {"G_strand_nt_s": work / t_res / 1e9, "ms_per_step": 1e3 * t_res},
                  "resident_1mnt": {"G_strand_nt_s": work / t_1m / 1e9, "ms_per_step": 1e3 * t_1m},
                  "small_scan_ms": 1e3 * float(np.median(t_small))}
+        if args.min_qual:
+            entry["candidates_masked"] = int(len(hits["chars_q"]))
         for leg in legs:
             med = float(np.median(times[leg]))
             entry[leg] = {"G_strand_nt_s": work / med / 1e9, "ms_per_step": 1e3 * med,
@@ -193,10 +230,10 @@ def main():
         entry["card_after"] = card()
         res["workloads"].append(entry)
         print(json.dumps({k: entry[k] for k in ("workload", "candidates", "candidates_byte_equal", "small_scan_ms")} |
-                         {k: round(entry[k]["G_strand_nt_s"], 1) for k in ["resident", "resident_1mnt"] + LEGS} |
-                         {k + "_upload_ms": round(entry[k]["upload_ms"], 2) for k in LEGS}), flush=True)
+                         {k: round(entry[k]["G_strand_nt_s"], 1) for k in ["resident", "resident_1mnt"] + legs_run} |
+                         {k + "_upload_ms": round(entry[k]["upload_ms"], 2) for k in legs_run}), flush=True)
     res["ok"] = ok_all
-    with open(os.path.join(args.out, "fastq_e2e.json"), "w") as fh:
+    with open(os.path.join(args.out, "fastq_mask_e2e.json" if args.min_qual else "fastq_e2e.json"), "w") as fh:
         json.dump(res, fh, indent=1)
     if not ok_all:
         raise SystemExit("fastq_e2e.py: the candidate arrays differ between the legs")

@@ -14,6 +14,9 @@
 //                       compacted, and for every record its first character's index (rec_off)
 //                       and the text offset of its '@' (hdr_off); checks every line 4k for '@'
 //                       and 4k+2 for '+', and every read's length against its quality string's
+//   gm_fastq_mask       (only with a minimum base quality set) one warp per segment, after emit:
+//                       writes 'n' over the read bytes whose quality is low, and checks every
+//                       quality byte's range
 //
 // A failing record is reported through one atomicMin over (record << 2 | what), so the host
 // names the first one whatever order the warps ran in.  Quality length: where record r + 1
@@ -232,6 +235,53 @@ __global__ void __launch_bounds__(256) gm_fastq_emit(const uint8_t *__restrict__
 		seq += tot_e;
 		qual += tot_q;
 		rec += tot_r;
+		phase += tot_nl;
+	}
+}
+
+// Low-quality masking (gm_ctx_set_min_quality): one warp per segment again, in its true phase, writes
+// 'n' over the read byte of every quality byte below t = offset + min_qual.  Quality byte q of the
+// text (counted over all records) belongs to read byte q: where every record so far is well formed,
+// the quality bytes before a record equal its rec_off, and a text that is not is refused.  It runs
+// on the stream after gm_fastq_emit: a read line and its quality line may lie in different segments,
+// so only stream order keeps these writes behind the read bytes emit places.  q is below the text's
+// quality byte count, which is at most n, so every write stays in chars (n + 64 bytes) whatever the
+// text.  A quality byte outside [offset, 126] is reported through one atomicMin of
+// (its text offset << 8 | its value): the first such byte of the text, hence of the first record
+// that has one.
+__global__ void __launch_bounds__(256) gm_fastq_mask(const uint8_t *__restrict__ text, int64_t n,
+	const FastqSegStart *__restrict__ starts, int n_seg, unsigned t, unsigned offset, uint8_t *__restrict__ chars,
+	unsigned long long *__restrict__ first_out)
+{
+	const int lane = threadIdx.x & 31;
+	const int seg = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+	if (seg >= n_seg)
+		return;
+	const int64_t base = (int64_t)seg * GM_FASTN_SEG;
+	const FastqSegStart st = starts[seg];
+	int64_t qual = st.qual;
+	unsigned phase = (unsigned)st.phase;
+	for (int it = 0; it < GM_FASTN_SEG / 512; it++) {
+		const int64_t pos = base + it * 512 + lane * 16;
+		if (base + it * 512 >= n)
+			break;
+		uint32_t w[4];
+		unsigned nl, body, next, tot_nl, tot_q, low, out;
+		fastq_lane(text, pos, n, lane, w, nl, body, next);
+		const int e = (int)((phase + fastq_lane_prefix((unsigned)__popc(nl), lane, &tot_nl)) & 3);
+		const unsigned qm = body & fastq_phase_mask(nl, e, 3); // quality bytes
+		fastq_qual16(w, qm, t, offset, low, out);
+		const unsigned pq = fastq_lane_prefix((unsigned)__popc(qm), lane, &tot_q);
+		for (unsigned m = low; m;) {
+			const int k = __ffs(m) - 1;
+			m &= m - 1;
+			chars[qual + pq + __popc(qm & ((1u << k) - 1))] = 'n';
+		}
+		if (out) {
+			const int k = __ffs(out) - 1;
+			atomicMin(first_out, ((unsigned long long)(pos + k) << 8) | ((w[k >> 2] >> (8 * (k & 3))) & 0xffu));
+		}
+		qual += tot_q;
 		phase += tot_nl;
 	}
 }

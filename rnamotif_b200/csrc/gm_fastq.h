@@ -12,7 +12,8 @@
 //   nl    newlines (the same for every entry phase)
 // A '\n' is never kept, nor a '\r' right before a '\n' (CR LF files).  Pieces compose with
 //   C.x[p] = A.x[p] + B.x[(p + A.nl) & 3],   C.nl = A.nl + B.nl
-// which is associative, so one block scans the segment summaries (gm_fastq_scan).
+// which is associative, so one block scans the segment summaries (gm_fastq_scan).  The quality
+// bytes' compare for low-quality masking (fastq_qual16) is here too, with its per-byte definition.
 #pragma once
 #include <stdint.h>
 
@@ -136,6 +137,35 @@ GM_FQ_HD FastqSum fastq_sum16(unsigned nl, unsigned body)
 	}
 	s.nl = (unsigned long long)fastq_popc(nl);
 	return s;
+}
+
+// Low-quality masking (gm_fastq_mask), one quality byte c at a time: c is LOW under the threshold
+// t = offset + min_qual (its value c - offset is below min_qual), and OUT of range outside
+// [offset, 126].
+GM_FQ_HD bool fastq_qual_low(unsigned c, unsigned t) { return c < t; }
+GM_FQ_HD bool fastq_qual_out(unsigned c, unsigned offset) { return c < offset || c > 126; }
+
+// Bit k (k < 4) = byte k of w is below t, for t <= 127: 0x80 | (c & 0x7f) >= t, so no borrow
+// crosses a byte, and the top bit of the difference is set where c & 0x7f >= t.
+GM_FQ_HD unsigned fastq_below4(uint32_t w, unsigned t)
+{
+	const uint32_t ge = ((w & 0x7f7f7f7fu) | 0x80808080u) - t * 0x01010101u;
+	const uint32_t lt = ~ge & ~w & 0x80808080u;
+	return (((lt >> 7) * 0x00204081u) >> 21) & 0xfu; // bits 0, 8, 16, 24 -> 21, 22, 23, 24
+}
+
+// Sixteen bytes as fastq_classify16 takes them; sel = the quality bytes among them, t and offset
+// as above (both <= 127).  low = the LOW bytes of sel, out = the OUT ones.
+GM_FQ_HD void fastq_qual16(const uint32_t w[4], unsigned sel, unsigned t, unsigned offset, unsigned &low, unsigned &out)
+{
+	unsigned lo = 0, under = 0, in = 0;
+	for (int j = 0; j < 4; j++) {
+		lo |= fastq_below4(w[j], t) << (4 * j);
+		under |= fastq_below4(w[j], offset) << (4 * j);
+		in |= fastq_below4(w[j], 127) << (4 * j);
+	}
+	low = lo & sel;
+	out = (under | ~in) & sel;
 }
 
 } // namespace gm

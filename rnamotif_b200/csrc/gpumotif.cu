@@ -104,6 +104,7 @@ struct gm_ctx {
 	gm_plan_t *d_plan;
 	DevSearch *d_ds;
 	gm_score_t *d_score;   // score pre-screen (gm_ctx_set_score) or NULL
+	int min_qual, qual_offset; // FASTQ low-quality masking (gm_ctx_set_min_quality); min_qual 0 = off
 	// database; every upload sets db as its last step, on success only, and nothing below is read while
 	// db is DB_NONE
 	DbKind db;
@@ -1169,6 +1170,8 @@ extern "C" int gm_ctx_create(gm_ctx **out, const gm_plan_t *plan, int device)
 	c->d_plan = NULL;
 	c->d_ds = NULL;
 	c->d_score = NULL;
+	c->min_qual = 0;
+	c->qual_offset = 33;
 	c->d_text = NULL;
 	c->d_hdr_off = NULL;
 	c->d_fsum = c->d_fstart = NULL;
@@ -1374,6 +1377,19 @@ extern "C" int gm_ctx_set_score(gm_ctx *c, const gm_score_t *score)
 	if (c->d_score == NULL)
 		CU(cudaMalloc(&c->d_score, sizeof(gm_score_t)));
 	CU(cudaMemcpy(c->d_score, score, sizeof(gm_score_t), cudaMemcpyHostToDevice));
+	return 0;
+}
+
+extern "C" int gm_ctx_set_min_quality(gm_ctx *c, int min_qual, int qual_offset)
+{
+	if (c == NULL)
+		return fail("ctx is NULL");
+	if (qual_offset != 33 && qual_offset != 64)
+		return fail("quality offset %d: 33 (Sanger, Illumina 1.8+) or 64 (Illumina 1.3-1.7)", qual_offset);
+	if (min_qual < 0 || min_qual > 126 - qual_offset)
+		return fail("minimum quality %d outside [0, %d] for offset %d", min_qual, 126 - qual_offset, qual_offset);
+	c->min_qual = min_qual;
+	c->qual_offset = qual_offset;
 	return 0;
 }
 
@@ -1932,19 +1948,25 @@ static int read_fastn(gm_ctx *c, int64_t n)
 
 // Four-line FASTQ on the device (gm_fastq.cuh) over the first n of the n_bytes of text in d_text (the
 // caller has cut the line end after the last line): reads + record table (rec_off, hdr_off; blocks
-// until they are known and the format is checked) -> 4-bit codes, asynchronously.
+// until they are known and the format is checked) -> 4-bit codes, asynchronously.  With a minimum
+// base quality set, the low-quality read bytes are masked in d_chars before the pack reads them.
 static int read_fastq(gm_ctx *c, int64_t n, int64_t n_bytes)
 {
 	const int n_seg = (int)((n + GM_FASTN_SEG - 1) / GM_FASTN_SEG);
+	const int min_qual = c->min_qual, qual_offset = c->qual_offset;
+	// n + 64 bytes of d_chars also bound gm_fastq_mask's writes: a quality index is below the text's
+	// quality byte count, which is at most n
 	if (ensure((void **)&c->d_chars, &c->chars_cap, (size_t)n + 64) ||
 	    ensure(&c->d_fsum, &c->fsum_cap, (size_t)(n_seg + 1) * sizeof(FastqSum) + 32) ||
 	    ensure(&c->d_fstart, &c->fstart_cap, (size_t)(n_seg + 1) * sizeof(FastqSegStart)))
 		return -1;
-	// totals (read bytes, records), then the first failing record's key (record << 2 | what)
+	// totals (read bytes, records), then the first failing record's key (record << 2 | what), then
+	// (masking only) the first out-of-range quality byte's key (text offset << 8 | value)
 	unsigned long long *d_tot = reinterpret_cast<unsigned long long *>(
 		static_cast<uint8_t *>(c->d_fsum) + (size_t)(n_seg + 1) * sizeof(FastqSum));
-	unsigned long long tot[2] = {0, 0}, bad = ~0ull;
-	CU(cudaMemsetAsync(d_tot + 2, 0xff, sizeof(unsigned long long), c->copy_stream));
+	unsigned long long tot[2] = {0, 0}, bad[2] = {~0ull, ~0ull};
+	const size_t n_bad = min_qual > 0 ? 2 : 1;
+	CU(cudaMemsetAsync(d_tot + 2, 0xff, n_bad * sizeof(unsigned long long), c->copy_stream));
 	if (n > 0) {
 		const int blocks = (n_seg * 32 + 255) / 256;
 		gm_fastq_summarize<<<blocks, 256, 0, c->copy_stream>>>(c->d_text, n, static_cast<FastqSum *>(c->d_fsum), n_seg);
@@ -1972,18 +1994,33 @@ static int read_fastq(gm_ctx *c, int64_t n, int64_t n_bytes)
 		gm_fastq_emit<<<blocks, 256, 0, c->copy_stream>>>(c->d_text, n, static_cast<const FastqSegStart *>(c->d_fstart),
 			n_seg, c->d_chars, c->d_rec_off, c->d_hdr_off, d_tot + 2);
 		CU(cudaGetLastError());
+		if (min_qual > 0) {
+			// behind emit on copy_stream, ahead of the pack (pack_text_records) that reads d_chars
+			gm_fastq_mask<<<blocks, 256, 0, c->copy_stream>>>(c->d_text, n, static_cast<const FastqSegStart *>(c->d_fstart),
+				n_seg, (unsigned)(qual_offset + min_qual), (unsigned)qual_offset, c->d_chars, d_tot + 3);
+			CU(cudaGetLastError());
+		}
 	}
 	CU(cudaMemcpyAsync(c->d_rec_off + n_rec, &last[0], sizeof(int64_t), cudaMemcpyHostToDevice, c->copy_stream));
 	CU(cudaMemcpyAsync(c->d_hdr_off + n_rec, &last[1], sizeof(int64_t), cudaMemcpyHostToDevice, c->copy_stream));
 	CU(cudaMemcpyAsync(c->rec_off.data(), c->d_rec_off, tab, cudaMemcpyDeviceToHost, c->copy_stream));
 	CU(cudaMemcpyAsync(c->hdr_off.data(), c->d_hdr_off, tab, cudaMemcpyDeviceToHost, c->copy_stream));
-	CU(cudaMemcpyAsync(&bad, d_tot + 2, sizeof bad, cudaMemcpyDeviceToHost, c->copy_stream));
+	CU(cudaMemcpyAsync(bad, d_tot + 2, n_bad * sizeof bad[0], cudaMemcpyDeviceToHost, c->copy_stream));
 	CU(cudaStreamSynchronize(c->copy_stream));
 	c->total_nt = (int64_t)tot[0];
-	if (bad != ~0ull) {
-		const long long r = (long long)(bad >> 2);
+	if (bad[1] != ~0ull) {
+		// the record of the first out-of-range quality byte: the last one whose '@' lies before it; it
+		// is named unless a record before it, or the record itself, fails a format check
+		const int64_t b = (int64_t)(bad[1] >> 8);
+		const long long r = (long long)(std::upper_bound(c->hdr_off.begin(), c->hdr_off.end(), b) - c->hdr_off.begin()) - 1;
+		if (bad[0] == ~0ull || r < (long long)(bad[0] >> 2))
+			return fail("FASTQ record %lld at byte %lld: quality byte %u is outside [%d, 126]", r, (long long)c->hdr_off[r],
+				    (unsigned)(bad[1] & 0xff), qual_offset);
+	}
+	if (bad[0] != ~0ull) {
+		const long long r = (long long)(bad[0] >> 2);
 		const long long at = (long long)c->hdr_off[r];
-		switch ((int)(bad & 3)) {
+		switch ((int)(bad[0] & 3)) {
 		case GM_FQ_AT:
 			return fail("FASTQ record %lld at byte %lld: line %lld does not start with '@'", r, at, 4 * r + 1);
 		case GM_FQ_PLUS:

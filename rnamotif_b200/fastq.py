@@ -4,7 +4,9 @@ The format (include/gpumotif.h, gm_db_upload_fastq): every record is four lines 
 description, the read, '+' (anything may follow), the quality string.  A line's role is its index
 mod 4, never its first byte.  Every byte of a read line but a trailing '\\r' is one nucleotide.
 Lines end in '\\n' or '\\r\\n'; the line end after the last line is optional.  parse_fastq raises
-FastqError for each input the device reader refuses, with the record it names.
+FastqError for each input the device reader refuses, with the record it names.  With a minimum base
+quality (gm_ctx_set_min_quality) it masks low-quality bases as n and refuses quality bytes outside
+[qual_offset, 126], as the device does.
 """
 from __future__ import annotations
 
@@ -36,16 +38,20 @@ def trimmed_length(data: bytes) -> int:
     return n
 
 
-def parse_fastq(data: bytes):
+def parse_fastq(data: bytes, min_qual: int = 0, qual_offset: int = 33):
     """Return (ids, seq, rec_off, hdr_off): ids = each record's id (the first blank-delimited
     token after '@'), seq = the reads' characters concatenated as uint8 (lower case, u -> t, as
     MotifSearch.get_chars reads them back), rec_off = n+1 int64 offsets into seq, hdr_off = n+1
-    int64 offsets of each record's '@' in `data` (hdr_off[n] = len(data))."""
+    int64 offsets of each record's '@' in `data` (hdr_off[n] = len(data)).  min_qual > 0: every
+    base whose quality byte q has q - qual_offset < min_qual is n in seq, and a record with a
+    quality byte outside [qual_offset, 126] is refused (after its own format checks)."""
+    if qual_offset not in (33, 64) or not 0 <= min_qual <= 126 - qual_offset:
+        raise ValueError(f"min_qual {min_qual}, qual_offset {qual_offset}: offset 33 or 64, min_qual in [0, 126 - offset]")
     data = bytes(data)
     if data and data[:1] != b"@":
         raise FastqError("FASTQ text does not begin with '@'")
     n = trimmed_length(data)
-    ids, reads, offs, hdrs = [], [], [0], []
+    ids, reads, quals, offs, hdrs = [], [], [], [0], []
     if n:
         lines, starts, p = [], [], 0
         while True:
@@ -73,6 +79,13 @@ def parse_fastq(data: bytes):
                 raise FastqError(f"FASTQ record {r} at byte {at}: the last record has fewer than four lines", r, at)
             if len(rec[1]) != len(rec[3]):
                 raise FastqError(f"FASTQ record {r} at byte {at}: its quality string is not as long as its read", r, at)
+            if min_qual > 0:
+                q = np.frombuffer(rec[3], dtype=np.uint8)
+                out = np.flatnonzero((q < qual_offset) | (q > 126))
+                if out.size:
+                    raise FastqError(f"FASTQ record {r} at byte {at}: quality byte {q[out[0]]} is outside "
+                                     f"[{qual_offset}, 126]", r, at)
+                quals.append(rec[3])
             parts = rec[0][1:].split(None, 1)
             ids.append(parts[0].decode("latin-1") if parts else "")
             reads.append(rec[1])
@@ -80,8 +93,10 @@ def parse_fastq(data: bytes):
             offs.append(total)
             hdrs.append(at)
     hdrs.append(len(data))
-    seq = np.frombuffer(b"".join(reads), dtype=np.uint8)
-    return ids, _LOWER[seq], np.asarray(offs, dtype=np.int64), np.asarray(hdrs, dtype=np.int64)
+    seq = _LOWER[np.frombuffer(b"".join(reads), dtype=np.uint8)]
+    if min_qual > 0:
+        seq[np.frombuffer(b"".join(quals), dtype=np.uint8) < qual_offset + min_qual] = ord("n")
+    return ids, seq, np.asarray(offs, dtype=np.int64), np.asarray(hdrs, dtype=np.int64)
 
 
 def write_fastq(ids, seq, rec_off, qual=None, crlf: bool = False) -> bytes:

@@ -37,7 +37,8 @@ _lib = None
 
 EXPORTS = ["gm_last_error", "gm_version", "gm_device_count", "gm_host_alloc", "gm_host_free", "gm_ctx_create", "gm_ctx_destroy",
            "gm_plan_check", "gm_plan_describe", "gm_db_upload_chars", "gm_db_upload_chars_hostpack", "gm_host_pack", "gm_db_set_device_chars", "gm_db_upload_fastn",
-           "gm_db_upload_2bit", "gm_db_upload_fastn_bgzf", "gm_db_upload_fastq", "gm_db_upload_fastq_bgzf", "gm_db_get_text",
+           "gm_db_upload_2bit", "gm_db_upload_fastn_bgzf", "gm_db_upload_fastq", "gm_db_upload_fastq_bgzf", "gm_ctx_set_min_quality",
+           "gm_db_get_text",
            "gm_db_records", "gm_db_get_chars", "gm_db_total_nt", "gm_hit_windows",
            "gm_scan", "gm_scan_launch", "gm_scan_finish", "gm_hits", "gm_stats",
            "gm_set_hit_capacity", "gm_set_tile", "gm_stream", "gm_prune_hits", "gm_order_hits",
@@ -68,6 +69,7 @@ def lib():
         L.gm_db_upload_fastn_bgzf.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
         L.gm_db_upload_fastq.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
         L.gm_db_upload_fastq_bgzf.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
+        L.gm_ctx_set_min_quality.argtypes = [C.c_void_p, C.c_int, C.c_int]
         L.gm_db_get_text.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p]
         L.gm_db_records.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_int)]
         L.gm_hit_windows.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]
@@ -297,6 +299,12 @@ class MotifSearch:
 
     def upload_fastq_bgzf_ptr(self, host_ptr: int, n_bytes: int):
         self._ck(lib().gm_db_upload_fastq_bgzf(self._ctx, host_ptr, n_bytes), "gm_db_upload_fastq_bgzf")
+
+    def set_min_quality(self, min_qual: int, qual_offset: int = 33):
+        """gm_ctx_set_min_quality: from the next upload_fastq or upload_fastq_bgzf on, read bases whose
+        quality (byte - qual_offset: 33 Sanger / Illumina 1.8+, 64 Illumina 1.3-1.7) is below min_qual
+        as n, and refuse quality bytes outside [qual_offset, 126].  min_qual = 0 switches it off."""
+        self._ck(lib().gm_ctx_set_min_quality(self._ctx, min_qual, qual_offset), "gm_ctx_set_min_quality")
 
     def get_text(self, off: int = 0, n: int | None = None) -> bytes:
         """gm_db_get_text: bytes [off, off + n) of the FASTA or FASTQ text of the last upload_fastn,
