@@ -16,6 +16,7 @@
 #include <cmath>
 #include <cstring>
 #include <condition_variable>
+#include <memory>
 #include <mutex>
 #include <numeric>
 #include <thread>
@@ -57,6 +58,100 @@ struct NvtxRange {
 	~NvtxRange() { nvtxRangePop(); }
 };
 
+// The context's resources are owned by the types below, which free them once: none can be copied.
+struct NoCopy {
+	NoCopy() = default;
+	NoCopy(const NoCopy &) = delete;
+	NoCopy &operator=(const NoCopy &) = delete;
+};
+
+// Device memory.  cap is in bytes; alloc() takes exactly what is asked, ensure() an eighth and 256
+// bytes more, so that a slightly larger upload reuses the buffer.  The contents do not survive either.
+template <class T> struct DevBuf : NoCopy {
+	T *p = nullptr;
+	size_t cap = 0;
+	~DevBuf() { cudaFree(p); }
+	operator T *() const { return p; }
+	void reset()
+	{
+		cudaFree(p);
+		p = nullptr;
+		cap = 0;
+	}
+	cudaError_t alloc(size_t n)
+	{
+		reset();
+		const cudaError_t e = cudaMalloc((void **)&p, n);
+		if (e == cudaSuccess)
+			cap = n;
+		return e;
+	}
+	int ensure(size_t need)
+	{
+		if (need <= cap)
+			return 0;
+		const size_t n = need + need / 8 + 256;
+		if (alloc(n) != cudaSuccess) {
+			// read and cleared here: the next launch's cudaGetLastError() must not report this allocation
+			const cudaError_t e = cudaGetLastError();
+			return fail("cudaMalloc(%zu bytes): %s", n, cudaGetErrorString(e));
+		}
+		return 0;
+	}
+};
+
+// Pinned host memory.  cap is in elements, and ensure() takes a quarter and 4096 elements more than
+// asked.
+template <class T> struct PinnedBuf : NoCopy {
+	T *p = nullptr;
+	size_t cap = 0;
+	~PinnedBuf() { cudaFreeHost(p); }
+	operator T *() const { return p; }
+	int ensure(size_t need)
+	{
+		if (need <= cap)
+			return 0;
+		cudaFreeHost(p);
+		p = nullptr;
+		cap = 0;
+		const size_t n = need + need / 4 + 4096;
+		CU(cudaMallocHost((void **)&p, n * sizeof(T)));
+		cap = n;
+		return 0;
+	}
+};
+
+// Events, created as they are first needed
+struct Events : NoCopy {
+	std::vector<cudaEvent_t> v;
+	~Events()
+	{
+		for (cudaEvent_t e : v)
+			cudaEventDestroy(e);
+	}
+	cudaEvent_t operator[](size_t i) const { return v[i]; }
+	// at least n events; new ones are created with `flags`
+	int grow(size_t n, unsigned flags)
+	{
+		while (v.size() < n) {
+			cudaEvent_t e;
+			CU(cudaEventCreateWithFlags(&e, flags));
+			v.push_back(e);
+		}
+		return 0;
+	}
+};
+
+struct Stream : NoCopy {
+	cudaStream_t s = nullptr;
+	~Stream()
+	{
+		if (s)
+			cudaStreamDestroy(s);
+	}
+	operator cudaStream_t() const { return s; }
+};
+
 #define GM_PACK_SLOTS 4
 
 // What the context's database is (gm_ctx::db).  DB_CHARS: characters on the device (d_seq_chars) and
@@ -66,119 +161,117 @@ struct NvtxRange {
 enum DbKind { DB_NONE, DB_CHARS, DB_HOSTPACK, DB_2BIT, DB_FASTN, DB_FASTQ };
 
 struct gm_ctx {
-	gm_plan_t plan;
-	DevParams par;
-	DevSearch ds[GM_MAX_DESCR];
-	int device;
-	int n_sm;
-	cudaStream_t stream;       // search kernels, hit gather
-	cudaStream_t copy_stream;  // uploads: H2D copies (+ pack kernels of device-side uploads), in chunks
+	gm_plan_t plan = {};
+	DevParams par = {};
+	DevSearch ds[GM_MAX_DESCR] = {};
+	int device = 0;
+	int n_sm = 0;
+	Stream stream;       // search kernels, hit gather
+	Stream copy_stream;  // uploads: H2D copies (+ pack kernels of device-side uploads), in chunks
 	// pack kernels of a character upload from the host: on a stream of their own (highest priority), gated per
 	// chunk on the copy, so that the copy engine never waits for a pack kernel that is itself waiting for the
 	// search kernel of the previous chunk to leave an SM
-	cudaStream_t pack_stream;
-	std::vector<cudaEvent_t> cp_ev;  // chunk i has arrived on the device
-	cudaEvent_t ev[6];
+	Stream pack_stream;
+	Events cp_ev;        // chunk i has arrived on the device
+	Events scan_ev;      // scan start / end on stream
 	// an upload is cut into chunks; chunk_ev[i] fires when chunk i is packed, so the
 	// first scan after an upload starts on chunk 0 while the rest is still copying
-	std::vector<cudaEvent_t> chunk_ev;
+	Events chunk_ev;
 	std::vector<int64_t> chunk_end;  // nucleotide offsets where the chunks end
-	bool upload_fresh;               // no scan has consumed the last upload yet
-	cudaEvent_t up_ev[2];            // upload start / end on copy_stream
+	bool upload_fresh = false;       // no scan has consumed the last upload yet
+	Events up_ev;                    // upload start / end on copy_stream
 	// host-packed upload (gm_db_upload_chars_hostpack): a thread team packs chunk i into
 	// a ring of pinned slots while chunk i-1 is on the wire; the uploader thread
 	// enqueues the copies and PUBLISHES each chunk once its event is recorded (waiting
 	// on an event nobody has recorded yet would not wait at all), and gm_scan_launch
 	// takes the chunks as they are published
-	PackTeam *team;
+	std::unique_ptr<PackTeam> team;
 	std::thread up_thread;
 	std::mutex up_m;
 	std::condition_variable up_cv;
-	int up_published;                // chunks whose event is recorded; -1 = every chunk_ev is (device-side uploads)
-	char up_err[256];                // first error of the uploader thread
-	uint8_t *h_slot[GM_PACK_SLOTS];  // pinned
-	size_t slot_cap;
-	cudaEvent_t slot_ev[GM_PACK_SLOTS]; // the copy out of the slot is done
+	int up_published = -1;           // chunks whose event is recorded; -1 = every chunk_ev is (device-side uploads)
+	char up_err[256] = {};           // first error of the uploader thread
+	PinnedBuf<uint8_t> h_slot[GM_PACK_SLOTS];
+	Events slot_ev;                  // the copy out of the slot is done
 	// this context's device copy of the plan and of the per-search table (the kernels
 	// stage what they use into shared memory; nothing is shared between contexts)
-	gm_plan_t *d_plan;
-	DevSearch *d_ds;
-	gm_score_t *d_score;   // score pre-screen (gm_ctx_set_score) or NULL
-	int min_qual, qual_offset; // FASTQ low-quality masking (gm_ctx_set_min_quality); min_qual 0 = off
+	DevBuf<gm_plan_t> d_plan;
+	DevBuf<DevSearch> d_ds;
+	DevBuf<gm_score_t> d_score; // score pre-screen (gm_ctx_set_score) or NULL
+	int min_qual = 0, qual_offset = 33; // FASTQ low-quality masking (gm_ctx_set_min_quality); min_qual 0 = off
 	// database; every upload sets db as its last step, on success only, and nothing below is read while
 	// db is DB_NONE
-	DbKind db;
-	uint8_t *d_chars;      // staging for uploaded characters
-	size_t chars_cap;
-	uint8_t *d_packed;
-	size_t packed_cap;
-	int64_t *d_rec_off;
-	size_t rec_cap;        // bytes
+	DbKind db = DB_NONE;
+	DevBuf<uint8_t> d_chars; // staging for uploaded characters
+	DevBuf<uint8_t> d_packed;
+	DevBuf<int64_t> d_rec_off;
 	std::vector<int64_t> rec_off;
-	int64_t total_nt;
+	int64_t total_nt = 0;
 	// start_pre[r] = the starts the sieve path searches on one strand of records 0 .. r-1 (index_starts), so
 	// that gm_scan_finish counts a range's starts without a loop over every record
 	std::vector<uint64_t> start_pre;
 	// FASTA or FASTQ text parsed on the device (gm_db_upload_fastn, gm_db_upload_fastq)
-	uint8_t *d_text;
-	size_t text_cap;
-	int64_t *d_hdr_off;
-	size_t hdr_cap;          // bytes
-	void *d_fsum, *d_fstart; // per-segment summaries / starts
-	size_t fsum_cap, fstart_cap;
+	DevBuf<uint8_t> d_text;
+	DevBuf<int64_t> d_hdr_off;
+	DevBuf<void> d_fsum, d_fstart; // per-segment summaries / starts
 	std::vector<int64_t> hdr_off;
-	const uint8_t *d_seq_chars; // the uploaded characters as they sit on the device (window gather)
+	const uint8_t *d_seq_chars = nullptr; // the uploaded characters as they sit on the device (window gather)
 	// 2-bit upload (gm_db_upload_2bit): its bytes go to d_chars; per-record byte offsets into them,
 	// then the N ranges, on the device (d_tb) and on the host (tb)
-	int64_t *d_tb;
-	size_t tb_cap;           // bytes
+	DevBuf<int64_t> d_tb;
 	std::vector<int64_t> tb;
 	// BGZF upload (gm_db_upload_fastn_bgzf): the compressed bytes (d_gz); the member table, then the first
 	// failing member (u32), then a status byte per member (d_bgzf); the member table on the host (bgzf)
-	uint8_t *d_gz;
-	size_t gz_cap;
-	void *d_bgzf;
-	size_t bgzf_cap;
+	DevBuf<uint8_t> d_gz;
+	DevBuf<uint8_t> d_bgzf;
 	std::vector<BgzfMember> bgzf;
 	// windows around the candidates (gm_hit_windows)
-	uint8_t *d_win, *h_win;
-	size_t win_cap, h_win_cap;
+	DevBuf<uint8_t> d_win;
+	PinnedBuf<uint8_t> h_win;
 	std::vector<uint8_t> wins;
 	// scan
-	unsigned long long *d_counters; // [0] tile, [1] hits, [2] starts
-	uint32_t *d_hits;
-	size_t hit_cap;       // records
-	int stride_words;
-	int threads, blocks;
-	size_t smem_bytes;
+	DevBuf<unsigned long long> d_counters; // [0] tile, [1] hits, [2] starts
+	DevBuf<uint32_t> d_hits;
+	size_t hit_cap = (size_t)1 << 20; // records
+	int stride_words = 0;
+	int threads = 0, blocks = 0;
+	size_t smem_bytes = 0;
 	// split path (prefilter kernel -> worklist -> dfs kernel)
-	bool use_split;
-	bool full;            // plan needs the pseudoknot / parallel / triplex / quadruplex code
-	int a_threads, a_blocks, b_threads, b_blocks;
-	size_t a_smem, b_smem;
-	uint32_t *d_wl;
-	size_t wl_cap;        // entries
-	int64_t seg_nt;       // nucleotides per prefilter/dfs launch pair
+	bool use_split = false;
+	bool full = false;    // plan needs the pseudoknot / parallel / triplex / quadruplex code
+	int a_threads = 0, a_blocks = 0, b_threads = 0, b_blocks = 0;
+	size_t a_smem = 0, b_smem = 0;
+	DevBuf<uint32_t> d_wl;
+	size_t wl_cap = 0;    // entries
+	int64_t seg_nt = 0;   // nucleotides per prefilter/dfs launch pair
 	std::vector<uint32_t> hits;    // sorted, host
-	uint32_t *h_raw;               // pinned staging for the device -> host gather
-	size_t h_raw_cap;              // words
+	PinnedBuf<uint32_t> h_raw;     // pinned staging for the device -> host gather
 	std::vector<uint64_t> keys;    // sort keys, reused
 	// device-side ordering of the candidates (gm_scan_finish)
-	void *d_sort;                  // keys in/out, indices in/out, cub temp storage
-	size_t sort_cap;
-	uint32_t *d_sorted;            // the candidates in enumeration order
-	size_t sorted_cap;
-	bool dev_sorted;               // the last scan was ordered on the device
-	std::vector<cudaEvent_t> seg_ev; // split path: (before, after) the filter kernel of every segment
-	int n_seg_ev;                  // pairs recorded by the last launch
-	const uint32_t *hits_view;     // what gm_hits() hands out
-	size_t n_hits;
-	size_t n_raw;                  // candidates in the device buffer (n_hits + those the score pre-screen rejected)
-	gm_scan_stats_t stats;
+	DevBuf<uint8_t> d_sort;        // keys in/out, indices in/out, cub temp storage
+	DevBuf<uint32_t> d_sorted;     // the candidates in enumeration order
+	bool dev_sorted = false;       // the last scan was ordered on the device
+	Events seg_ev;                 // split path: (before, after) the filter kernel of every segment
+	int n_seg_ev = 0;              // pairs recorded by the last launch
+	const uint32_t *hits_view = nullptr; // what gm_hits() hands out
+	size_t n_hits = 0;
+	size_t n_raw = 0;              // candidates in the device buffer (n_hits + those the score pre-screen rejected)
+	gm_scan_stats_t stats = {};
 	// pending launch
-	bool pending;
-	int64_t p_begin, p_end;
-	int p_strands;
+	bool pending = false;
+	int64_t p_begin = 0, p_end = 0;
+	int p_strands = 0;
+
+	~gm_ctx()
+	{
+		// before any member goes: a joinable std::thread that is destroyed calls std::terminate, and the
+		// uploader thread uses the team, the slots and the events
+		if (up_thread.joinable())
+			up_thread.join();
+		for (cudaStream_t s : {stream.s, copy_stream.s, pack_stream.s})
+			if (s)
+				cudaStreamSynchronize(s);
+	}
 };
 
 extern "C" const char *gm_last_error(void) { return g_err; }
@@ -1165,47 +1258,7 @@ extern "C" int gm_ctx_create(gm_ctx **out, const gm_plan_t *plan, int device)
 		return fail("out is NULL");
 	*out = NULL;
 	gm_ctx *c = new gm_ctx();
-	memset(&c->stats, 0, sizeof c->stats);
-	c->d_chars = c->d_packed = NULL;
-	c->d_plan = NULL;
-	c->d_ds = NULL;
-	c->d_score = NULL;
-	c->min_qual = 0;
-	c->qual_offset = 33;
-	c->d_text = NULL;
-	c->d_hdr_off = NULL;
-	c->d_fsum = c->d_fstart = NULL;
-	c->text_cap = c->hdr_cap = c->fsum_cap = c->fstart_cap = 0;
-	c->d_seq_chars = NULL;
-	c->d_tb = NULL;
-	c->tb_cap = 0;
-	c->db = DB_NONE;
-	c->d_gz = NULL;
-	c->d_bgzf = NULL;
-	c->gz_cap = c->bgzf_cap = 0;
-	c->d_win = c->h_win = NULL;
-	c->win_cap = c->h_win_cap = 0;
-	c->d_rec_off = NULL;
-	c->d_counters = NULL;
-	c->d_hits = NULL;
-	c->d_wl = NULL;
-	c->wl_cap = 0;
-	c->h_raw = NULL;
-	c->h_raw_cap = 0;
-	c->d_sort = NULL;
-	c->sort_cap = 0;
-	c->d_sorted = NULL;
-	c->sorted_cap = 0;
-	c->dev_sorted = false;
-	c->hits_view = NULL;
-	c->n_seg_ev = 0;
 	c->seg_nt = getenv("GPUMOTIF_SEG_NT") != NULL && atoll(getenv("GPUMOTIF_SEG_NT")) > 0 ? atoll(getenv("GPUMOTIF_SEG_NT")) : wl_safe_seg();
-	c->use_split = false;
-	c->chars_cap = c->packed_cap = c->rec_cap = 0;
-	c->total_nt = 0;
-	c->n_hits = 0;
-	c->pending = false;
-	c->stream = NULL;
 	if (check_plan(plan, c->ds, &c->par)) {
 		delete c;
 		return -1;
@@ -1222,8 +1275,6 @@ extern "C" int gm_ctx_create(gm_ctx **out, const gm_plan_t *plan, int device)
 		return fail("device %d out of range (%d visible)", device, n);
 	}
 	c->device = device;
-	for (int i = 0; i < 6; i++)
-		c->ev[i] = NULL;
 	cudaDeviceProp prop;
 	cudaError_t e = cudaSetDevice(device);
 	if (e == cudaSuccess)
@@ -1238,53 +1289,38 @@ extern "C" int gm_ctx_create(gm_ctx **out, const gm_plan_t *plan, int device)
 	}
 	c->n_sm = prop.multiProcessorCount;
 	c->stride_words = (int)((sizeof(gm_hit_hdr_t) + plan->n_descr * sizeof(gm_hit_el_t)) / 4);
-	c->hit_cap = (size_t)1 << 20;
-	c->copy_stream = NULL;
-	c->pack_stream = NULL;
-	c->upload_fresh = false;
-	c->up_ev[0] = c->up_ev[1] = NULL;
-	c->team = NULL;
-	c->up_published = -1;
-	c->up_err[0] = 0;
-	c->slot_cap = 0;
-	for (int i = 0; i < GM_PACK_SLOTS; i++) {
-		c->h_slot[i] = NULL;
-		c->slot_ev[i] = NULL;
-	}
-	if (cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess ||
-	    cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking) != cudaSuccess) {
+	if (cudaStreamCreateWithFlags(&c->stream.s, cudaStreamNonBlocking) != cudaSuccess ||
+	    cudaStreamCreateWithFlags(&c->copy_stream.s, cudaStreamNonBlocking) != cudaSuccess) {
 		delete c;
 		return fail("cudaStreamCreate failed");
 	}
-	{
-		int lo_pri = 0, hi_pri = 0;
-		cudaDeviceGetStreamPriorityRange(&lo_pri, &hi_pri);
-		if (cudaStreamCreateWithPriority(&c->pack_stream, cudaStreamNonBlocking, hi_pri) != cudaSuccess) {
-			gm_ctx_destroy(c);
-			return fail("cudaStreamCreateWithPriority failed");
-		}
+	int lo_pri = 0, hi_pri = 0;
+	cudaDeviceGetStreamPriorityRange(&lo_pri, &hi_pri);
+	if (cudaStreamCreateWithPriority(&c->pack_stream.s, cudaStreamNonBlocking, hi_pri) != cudaSuccess) {
+		delete c;
+		return fail("cudaStreamCreateWithPriority failed");
 	}
-	cudaEventCreate(&c->up_ev[0]);
-	cudaEventCreate(&c->up_ev[1]);
-	for (int i = 0; i < 6; i++)
-		cudaEventCreate(&c->ev[i]);
-	if (cudaMalloc(&c->d_counters, 32 * sizeof(unsigned long long)) != cudaSuccess) {
-		gm_ctx_destroy(c);
+	if (c->up_ev.grow(2, cudaEventDefault) || c->scan_ev.grow(2, cudaEventDefault)) {
+		delete c;
+		return -1;
+	}
+	if (c->d_counters.alloc(32 * sizeof(unsigned long long)) != cudaSuccess) {
+		delete c;
 		return fail("cudaMalloc(counters) failed");
 	}
-	if (cudaMalloc(&c->d_plan, sizeof(gm_plan_t)) != cudaSuccess ||
-	    cudaMalloc(&c->d_ds, sizeof(DevSearch) * GM_MAX_DESCR) != cudaSuccess ||
+	if (c->d_plan.alloc(sizeof(gm_plan_t)) != cudaSuccess ||
+	    c->d_ds.alloc(sizeof(DevSearch) * GM_MAX_DESCR) != cudaSuccess ||
 	    cudaMemcpyAsync(c->d_plan, &c->plan, sizeof c->plan, cudaMemcpyHostToDevice, c->stream) != cudaSuccess ||
 	    cudaMemcpyAsync(c->d_ds, c->ds, sizeof(DevSearch) * GM_MAX_DESCR, cudaMemcpyHostToDevice, c->stream) != cudaSuccess) {
-		gm_ctx_destroy(c);
+		delete c;
 		return fail("plan upload failed: %s", cudaGetErrorString(cudaGetLastError()));
 	}
 	if (configure_launch(c, 0)) {
-		gm_ctx_destroy(c);
+		delete c;
 		return -1;
 	}
 	if (cudaStreamSynchronize(c->stream) != cudaSuccess) {
-		gm_ctx_destroy(c);
+		delete c;
 		return fail("plan upload failed: %s", cudaGetErrorString(cudaGetLastError()));
 	}
 	*out = c;
@@ -1296,59 +1332,6 @@ extern "C" void gm_ctx_destroy(gm_ctx *c)
 	if (c == NULL)
 		return;
 	cudaSetDevice(c->device);
-	if (c->up_thread.joinable())
-		c->up_thread.join();
-	delete c->team;
-	if (c->stream)
-		cudaStreamSynchronize(c->stream);
-	if (c->copy_stream)
-		cudaStreamSynchronize(c->copy_stream);
-	if (c->pack_stream)
-		cudaStreamSynchronize(c->pack_stream);
-	for (cudaEvent_t e : c->cp_ev)
-		cudaEventDestroy(e);
-	for (int i = 0; i < GM_PACK_SLOTS; i++) {
-		if (c->slot_ev[i])
-			cudaEventDestroy(c->slot_ev[i]);
-		cudaFreeHost(c->h_slot[i]);
-	}
-	for (cudaEvent_t e : c->chunk_ev)
-		cudaEventDestroy(e);
-	for (cudaEvent_t e : c->seg_ev)
-		cudaEventDestroy(e);
-	for (int i = 0; i < 2; i++)
-		if (c->up_ev[i])
-			cudaEventDestroy(c->up_ev[i]);
-	if (c->copy_stream)
-		cudaStreamDestroy(c->copy_stream);
-	if (c->pack_stream)
-		cudaStreamDestroy(c->pack_stream);
-	cudaFree(c->d_plan);
-	cudaFree(c->d_ds);
-	cudaFree(c->d_score);
-	cudaFree(c->d_chars);
-	cudaFree(c->d_text);
-	cudaFree(c->d_hdr_off);
-	cudaFree(c->d_tb);
-	cudaFree(c->d_gz);
-	cudaFree(c->d_bgzf);
-	cudaFree(c->d_fsum);
-	cudaFree(c->d_fstart);
-	cudaFree(c->d_win);
-	cudaFreeHost(c->h_win);
-	cudaFree(c->d_packed);
-	cudaFree(c->d_rec_off);
-	cudaFree(c->d_counters);
-	cudaFree(c->d_hits);
-	cudaFree(c->d_wl);
-	cudaFreeHost(c->h_raw);
-	cudaFree(c->d_sort);
-	cudaFree(c->d_sorted);
-	for (int i = 0; i < 6; i++)
-		if (c->ev[i])
-			cudaEventDestroy(c->ev[i]);
-	if (c->stream)
-		cudaStreamDestroy(c->stream);
 	delete c;
 }
 
@@ -1363,8 +1346,7 @@ extern "C" int gm_ctx_set_score(gm_ctx *c, const gm_score_t *score)
 	CU(cudaSetDevice(c->device));
 	CU(cudaStreamSynchronize(c->stream));
 	if (score == NULL || !score->present) {
-		cudaFree(c->d_score);
-		c->d_score = NULL;
+		c->d_score.reset();
 		return 0;
 	}
 	if (score->n_inst <= 0 || score->n_inst > GM_SC_MAX_INST || score->n_var < 0 || score->n_var > GM_SC_MAX_VAR ||
@@ -1374,8 +1356,8 @@ extern "C" int gm_ctx_set_score(gm_ctx *c, const gm_score_t *score)
 	for (int x = 0; x < score->n_xel; x++)
 		if (score->xel[x].elem >= c->plan.n_descr)
 			return fail("score program does not belong to this plan");
-	if (c->d_score == NULL)
-		CU(cudaMalloc(&c->d_score, sizeof(gm_score_t)));
+	if (c->d_score.p == NULL)
+		CU(c->d_score.alloc(sizeof(gm_score_t)));
 	CU(cudaMemcpy(c->d_score, score, sizeof(gm_score_t), cudaMemcpyHostToDevice));
 	return 0;
 }
@@ -1401,8 +1383,7 @@ extern "C" int gm_set_hit_capacity(gm_ctx *c, size_t n)
 		return fail("a scan is in flight");
 	c->hit_cap = n;
 	cudaSetDevice(c->device);
-	cudaFree(c->d_hits);
-	c->d_hits = NULL;
+	c->d_hits.reset();
 	return 0;
 }
 
@@ -1417,23 +1398,6 @@ extern "C" int gm_set_tile(gm_ctx *c, int tile)
 }
 
 // -------------------------------------------------------------- database
-
-static int ensure(void **p, size_t *cap, size_t need)
-{
-	if (need <= *cap)
-		return 0;
-	cudaFree(*p);
-	*p = NULL;
-	*cap = 0;
-	size_t n = need + need / 8 + 256;
-	if (cudaMalloc(p, n) != cudaSuccess) {
-		// read and cleared here: the next launch's cudaGetLastError() must not report this allocation
-		const cudaError_t e = cudaGetLastError();
-		return fail("cudaMalloc(%zu bytes): %s", n, cudaGetErrorString(e));
-	}
-	*cap = n;
-	return 0;
-}
 
 static int check_records(const int64_t *rec_off, int n_rec)
 {
@@ -1481,7 +1445,7 @@ static int set_records(gm_ctx *c, const int64_t *rec_off, int n_rec)
 	c->rec_off.assign(rec_off, rec_off + n_rec + 1);
 	c->total_nt = rec_off[n_rec];
 	index_starts(c);
-	if (ensure((void **)&c->d_rec_off, &c->rec_cap, tab))
+	if (c->d_rec_off.ensure(tab))
 		return -1;
 	CU(cudaMemcpyAsync(c->d_rec_off, c->rec_off.data(), tab, cudaMemcpyHostToDevice, c->copy_stream));
 	return 0;
@@ -1508,7 +1472,7 @@ static void drop_database(gm_ctx *c)
 // Every upload, once its host-side input has been checked, starts here: the uploader thread of the
 // last host-packed upload has enqueued everything (or failed), the previous upload has left the
 // device (its staging is reused), and the context holds no database, so a failure anywhere later
-// leaves none.  The upload sets c->db as its last step.
+// leaves none.  The upload ends with finish_upload.
 static int begin_upload(gm_ctx *c)
 {
 	if (c == NULL)
@@ -1528,10 +1492,22 @@ static int begin_upload(gm_ctx *c)
 	return sync_uploads(c);
 }
 
+// Every upload that succeeds ends here: the end of its copies is marked on copy_stream (by the uploader
+// thread, when there is one), the next scan streams its chunks in, and c->db is set last.
+static int finish_upload(gm_ctx *c, DbKind kind, uint64_t h2d_bytes)
+{
+	if (!c->up_thread.joinable())
+		CU(cudaEventRecord(c->up_ev[1], c->copy_stream));
+	c->upload_fresh = true;
+	c->stats.h2d_bytes = h2d_bytes;
+	c->db = kind;
+	return 0;
+}
+
 // the 4-bit codes of n nucleotides; slack: kernels read whole 16-byte groups past the end
 static int ensure_packed(gm_ctx *c, int64_t n)
 {
-	return ensure((void **)&c->d_packed, &c->packed_cap, (size_t)(((n + 15) / 16) * 8) + 1024);
+	return c->d_packed.ensure((size_t)(((n + 15) / 16) * 8) + 1024);
 }
 
 // blocks of 256 threads for a pack / expand kernel over len nucleotides, one 16-nt group per thread
@@ -1564,16 +1540,8 @@ static int cut_chunks(gm_ctx *c, int64_t n, int64_t floor_nt, int n_target, int6
 	int64_t ch = std::max<int64_t>(floor_nt, (n + n_target - 1) / n_target);
 	ch = (ch + align - 1) / align * align;
 	const int n_chunks = n > 0 ? (int)((n + ch - 1) / ch) : 0;
-	while ((int)c->chunk_ev.size() < n_chunks) {
-		cudaEvent_t e;
-		CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-		c->chunk_ev.push_back(e);
-	}
-	while (copies && (int)c->cp_ev.size() < n_chunks) {
-		cudaEvent_t e;
-		CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-		c->cp_ev.push_back(e);
-	}
+	if (c->chunk_ev.grow(n_chunks, cudaEventDisableTiming) || (copies && c->cp_ev.grow(n_chunks, cudaEventDisableTiming)))
+		return -1;
 	c->chunk_end.clear();
 	for (int i = 0; i < n_chunks; i++)
 		c->chunk_end.push_back(std::min<int64_t>(n, (int64_t)(i + 1) * ch));
@@ -1591,6 +1559,21 @@ static int cut_device_chunks(gm_ctx *c, int64_t n, bool copies, int64_t *chunk)
 	return cut_chunks(c, n, (int64_t)64 << 20, n_target, 16, copies, chunk);
 }
 
+// The copy behind chunk i's kernel on pack_stream: bytes [*copied, upto) of src to the same offsets of
+// dst on copy_stream (none when upto <= *copied), then cp_ev[i], which pack_stream waits for.
+static cudaError_t stage_copy(gm_ctx *c, int i, uint8_t *dst, const uint8_t *src, int64_t *copied, int64_t upto)
+{
+	cudaError_t e = cudaSuccess;
+	if (upto > *copied)
+		e = cudaMemcpyAsync(dst + *copied, src + *copied, (size_t)(upto - *copied), cudaMemcpyHostToDevice, c->copy_stream);
+	*copied = std::max(*copied, upto);
+	if (e == cudaSuccess)
+		e = cudaEventRecord(c->cp_ev[i], c->copy_stream);
+	if (e == cudaSuccess)
+		e = cudaStreamWaitEvent(c->pack_stream, c->cp_ev[i], 0);
+	return e;
+}
+
 // Enqueue the upload on copy_stream in chunks: [H2D copy of chunk i,] pack chunk i,
 // record chunk_ev[i].  Returns without waiting.
 static int upload_chunks(gm_ctx *c, const uint8_t *h_chars, const uint8_t *d_src, bool mark_start = true)
@@ -1599,7 +1582,7 @@ static int upload_chunks(gm_ctx *c, const uint8_t *h_chars, const uint8_t *d_src
 	const int64_t n = c->total_nt;
 	if (ensure_packed(c, n))
 		return -1;
-	if (h_chars != NULL && ensure((void **)&c->d_chars, &c->chars_cap, (size_t)n + 64))
+	if (h_chars != NULL && c->d_chars.ensure((size_t)n + 64))
 		return -1;
 	int64_t chunk;
 	if (cut_device_chunks(c, n, h_chars != NULL, &chunk))
@@ -1611,21 +1594,18 @@ static int upload_chunks(gm_ctx *c, const uint8_t *h_chars, const uint8_t *d_src
 	// from the host: copies back to back on the copy stream, pack kernels on the pack stream behind
 	// each chunk's copy; on the device: pack kernels on the copy stream
 	cudaStream_t ps = h_chars != NULL ? c->pack_stream : c->copy_stream;
+	int64_t copied = 0;
 	for (int i = 0; i < n_chunks; i++) {
 		const int64_t o = (int64_t)i * chunk, len = c->chunk_end[i] - o;
 		const uint8_t *src = d_src;
 		if (h_chars != NULL) {
-			CU(cudaMemcpyAsync(c->d_chars + o, h_chars + o, (size_t)len, cudaMemcpyHostToDevice, c->copy_stream));
-			CU(cudaEventRecord(c->cp_ev[i], c->copy_stream));
-			CU(cudaStreamWaitEvent(ps, c->cp_ev[i], 0));
+			CU(stage_copy(c, i, c->d_chars, h_chars, &copied, c->chunk_end[i]));
 			src = c->d_chars;
 		}
 		gm_pack_kernel<<<pack_blocks(c, len), 256, 0, ps>>>(src + o, c->d_packed + (o >> 1), len);
 		CU(cudaGetLastError());
 		CU(cudaEventRecord(c->chunk_ev[i], ps));
 	}
-	CU(cudaEventRecord(c->up_ev[1], c->copy_stream));
-	c->upload_fresh = true;
 	return 0;
 }
 
@@ -1637,9 +1617,7 @@ extern "C" int gm_db_upload_chars(gm_ctx *c, const char *seq, const int64_t *rec
 		return fail("seq is NULL");
 	if (begin_upload(c) || set_records(c, rec_off, n_rec) || upload_chunks(c, (const uint8_t *)seq, NULL))
 		return -1;
-	c->stats.h2d_bytes = (uint64_t)c->total_nt + (uint64_t)(n_rec + 1) * 8;
-	c->db = DB_CHARS;
-	return 0;
+	return finish_upload(c, DB_CHARS, (uint64_t)c->total_nt + (uint64_t)(n_rec + 1) * 8);
 }
 
 // Nucleotides [o, o + hp) of a host-packed chunk [o, o + len) are packed on the host, [o + hp, o + len)
@@ -1675,9 +1653,8 @@ static void uploader_main(gm_ctx *c, const uint8_t *seq, int64_t chunk, double f
 		if (hp < len) {
 			// the character share first: the link works on it while the team packs
 			const int64_t oc = o + hp, lc = len - hp;
-			if ((e = cudaMemcpyAsync(c->d_chars + oc, seq + oc, (size_t)lc, cudaMemcpyHostToDevice, c->copy_stream)) != cudaSuccess ||
-			    (e = cudaEventRecord(c->cp_ev[i], c->copy_stream)) != cudaSuccess ||
-			    (e = cudaStreamWaitEvent(c->pack_stream, c->cp_ev[i], 0)) != cudaSuccess)
+			int64_t copied = oc;
+			if ((e = stage_copy(c, i, c->d_chars, seq, &copied, o + len)) != cudaSuccess)
 				return bail("enqueue (characters)", e);
 			gm_pack_kernel<<<pack_blocks(c, lc), 256, 0, c->pack_stream>>>(c->d_chars + oc, c->d_packed + (oc >> 1), lc);
 			if ((e = cudaGetLastError()) != cudaSuccess)
@@ -1720,8 +1697,8 @@ extern "C" int gm_db_upload_chars_hostpack(gm_ctx *c, const char *seq, const int
 		return fail("seq is NULL");
 	if (begin_upload(c) || set_records(c, rec_off, n_rec) || ensure_packed(c, n))
 		return -1;
-	if (c->team == NULL)
-		c->team = new PackTeam(host_pack_default_threads());
+	if (!c->team)
+		c->team = std::make_unique<PackTeam>(host_pack_default_threads());
 	// share of every chunk packed on the host: all of it from pageable memory (a DMA from
 	// there would be staged synchronously); from pinned memory what the team keeps up with
 	// beside the link (GPUMOTIF_PACK_FRAC overrides; measured with 16 threads over 1 Gnt, ire: share
@@ -1736,7 +1713,7 @@ extern "C" int gm_db_upload_chars_hostpack(gm_ctx *c, const char *seq, const int
 		if (getenv("GPUMOTIF_PACK_FRAC") != NULL && (pinned || atof(getenv("GPUMOTIF_PACK_FRAC")) >= 1.0))
 			frac = std::max(0.05, std::min(1.0, atof(getenv("GPUMOTIF_PACK_FRAC"))));
 	}
-	if (frac < 1.0 && ensure((void **)&c->d_chars, &c->chars_cap, (size_t)n + 64))
+	if (frac < 1.0 && c->d_chars.ensure((size_t)n + 64))
 		return -1;
 	// at most 16 chunks (gm_scan_launch streams up to 16 in) of at least 16 Mnt, a multiple of
 	// 4096 nucleotides
@@ -1744,38 +1721,22 @@ extern "C" int gm_db_upload_chars_hostpack(gm_ctx *c, const char *seq, const int
 	if (cut_chunks(c, n, (int64_t)16 << 20, 16, 4096, frac < 1.0, &chunk))
 		return -1;
 	const int n_chunks = (int)c->chunk_end.size();
-	const size_t slot_need = (size_t)(chunk >> 1) + 64;
-	if (c->slot_cap < slot_need) {
-		for (int i = 0; i < GM_PACK_SLOTS; i++) {
-			cudaFreeHost(c->h_slot[i]);
-			c->h_slot[i] = NULL;
-		}
-		c->slot_cap = 0;
-		for (int i = 0; i < GM_PACK_SLOTS; i++)
-			CU(cudaMallocHost((void **)&c->h_slot[i], slot_need));
-		c->slot_cap = slot_need;
-	}
 	for (int i = 0; i < GM_PACK_SLOTS; i++)
-		if (c->slot_ev[i] == NULL)
-			CU(cudaEventCreateWithFlags(&c->slot_ev[i], cudaEventDisableTiming));
+		if (c->h_slot[i].ensure((size_t)(chunk >> 1) + 64))
+			return -1;
+	if (c->slot_ev.grow(GM_PACK_SLOTS, cudaEventDisableTiming))
+		return -1;
 	c->up_published = 0;
 	CU(cudaEventRecord(c->up_ev[0], c->copy_stream));
-	if (n_chunks == 0)
-		CU(cudaEventRecord(c->up_ev[1], c->copy_stream));
-	c->upload_fresh = true;
-	{
-		// bytes over the link: half a byte per host-packed nucleotide, one per character sent as it is
-		uint64_t b = (uint64_t)(n_rec + 1) * 8;
-		for (int i = 0; i < n_chunks; i++) {
-			const int64_t len = c->chunk_end[i] - (int64_t)i * chunk, hp = host_share(len, frac);
-			b += (uint64_t)((hp + 1) >> 1) + (uint64_t)(len - hp);
-		}
-		c->stats.h2d_bytes = b;
+	// bytes over the link: half a byte per host-packed nucleotide, one per character sent as it is
+	uint64_t b = (uint64_t)(n_rec + 1) * 8;
+	for (int i = 0; i < n_chunks; i++) {
+		const int64_t len = c->chunk_end[i] - (int64_t)i * chunk, hp = host_share(len, frac);
+		b += (uint64_t)((hp + 1) >> 1) + (uint64_t)(len - hp);
 	}
 	if (n_chunks > 0)
 		c->up_thread = std::thread(uploader_main, c, (const uint8_t *)seq, chunk, frac);
-	c->db = DB_HOSTPACK;
-	return 0;
+	return finish_upload(c, DB_HOSTPACK, b);
 }
 
 extern "C" int gm_db_set_device_chars(gm_ctx *c, const void *d_seq, const int64_t *rec_off, int n_rec)
@@ -1786,9 +1747,7 @@ extern "C" int gm_db_set_device_chars(gm_ctx *c, const void *d_seq, const int64_
 		return fail("d_seq is NULL");
 	if (begin_upload(c) || set_records(c, rec_off, n_rec) || upload_chunks(c, NULL, (const uint8_t *)d_seq))
 		return -1;
-	c->stats.h2d_bytes = (uint64_t)(n_rec + 1) * 8;
-	c->db = DB_CHARS;
-	return 0;
+	return finish_upload(c, DB_CHARS, (uint64_t)(n_rec + 1) * 8);
 }
 
 // UCSC .2bit input: the byte span from the first record's bases to the end of the last one goes
@@ -1842,8 +1801,7 @@ extern "C" int gm_db_upload_2bit(gm_ctx *c, const uint8_t *dna, size_t n_bytes, 
 	if (n_nblk > 0)
 		memcpy(c->tb.data() + n_rec, nblk, (size_t)n_nblk * 2 * sizeof(int64_t));
 	const size_t tb_bytes = c->tb.size() * sizeof(int64_t);
-	if (ensure_packed(c, n) || ensure((void **)&c->d_chars, &c->chars_cap, (size_t)span + 64) ||
-	    ensure((void **)&c->d_tb, &c->tb_cap, tb_bytes + 16))
+	if (ensure_packed(c, n) || c->d_chars.ensure((size_t)span + 64) || c->d_tb.ensure(tb_bytes + 16))
 		return -1;
 	int64_t chunk;
 	if (cut_device_chunks(c, n, true, &chunk))
@@ -1864,23 +1822,14 @@ extern "C" int gm_db_upload_2bit(gm_ctx *c, const uint8_t *dna, size_t n_bytes, 
 				r++;
 			upto = c->tb[r] + (g - rec_off[r]) / 4 + 1;
 		}
-		if (upto > copied)
-			CU(cudaMemcpyAsync(c->d_chars + copied, dna + b0 + copied, (size_t)(upto - copied), cudaMemcpyHostToDevice,
-					   c->copy_stream));
-		copied = std::max(copied, upto);
-		CU(cudaEventRecord(c->cp_ev[i], c->copy_stream));
-		CU(cudaStreamWaitEvent(c->pack_stream, c->cp_ev[i], 0));
+		CU(stage_copy(c, i, c->d_chars, dna + b0, &copied, upto));
 		gm_unpack2_kernel<<<pack_blocks(c, len), 256, 0, c->pack_stream>>>(c->d_chars, d_dna_off, c->d_rec_off, n_rec, d_nblk,
 										   n_nblk, o, len, c->d_packed);
 		CU(cudaGetLastError());
 		CU(cudaEventRecord(c->chunk_ev[i], c->pack_stream));
 	}
-	CU(cudaEventRecord(c->up_ev[1], c->copy_stream));
-	c->upload_fresh = true;
 	// bytes over the link: the span, the record table, dna_off and the N ranges
-	c->stats.h2d_bytes = (uint64_t)span + (uint64_t)(n_rec + 1) * 8 + (uint64_t)tb_bytes;
-	c->db = DB_2BIT;
-	return 0;
+	return finish_upload(c, DB_2BIT, (uint64_t)span + (uint64_t)(n_rec + 1) * 8 + (uint64_t)tb_bytes);
 }
 
 // The record table a device text reader has left in c->rec_off: every record under 2^31, then the
@@ -1897,50 +1846,69 @@ static int pack_text_records(gm_ctx *c)
 	return 0;
 }
 
-// FN_fgetseq on the device, src/dbutil.c:42-128 (gm_fastn.cuh), over the n bytes of FASTA text in
-// d_text (enqueued on copy_stream, or already there): text -> kept characters + record table
-// (rec_off, hdr_off; blocks until they are known) -> 4-bit codes, asynchronously.
-static int read_fastn(gm_ctx *c, int64_t n)
+// The record table of a device text reader once its totals are known: n_rec + 1 entries on the device
+// and on the host, for the reader's emit kernel to fill
+static int size_records(gm_ctx *c, unsigned long long n_rec)
 {
-	const int n_seg = (int)((n + GM_FASTN_SEG - 1) / GM_FASTN_SEG);
-	if (ensure((void **)&c->d_chars, &c->chars_cap, (size_t)n + 64) ||
-	    ensure(&c->d_fsum, &c->fsum_cap, (size_t)(n_seg + 1) * sizeof(FastnSum) + 16) ||
-	    ensure(&c->d_fstart, &c->fstart_cap, (size_t)(n_seg + 1) * sizeof(FastnSegStart)))
-		return -1;
-	unsigned long long *d_tot = reinterpret_cast<unsigned long long *>(
-		static_cast<uint8_t *>(c->d_fsum) + (size_t)(n_seg + 1) * sizeof(FastnSum));
-	unsigned long long tot[2] = {0, 0};
-	if (n > 0) {
-		const int blocks = (n_seg * 32 + 255) / 256;
-		gm_fastn_summarize<<<blocks, 256, 0, c->copy_stream>>>(c->d_text, n, static_cast<FastnSum *>(c->d_fsum), n_seg);
-		CU(cudaGetLastError());
-		gm_fastn_scan<<<1, 1024, 0, c->copy_stream>>>(static_cast<const FastnSum *>(c->d_fsum), n_seg,
-			static_cast<FastnSegStart *>(c->d_fstart), d_tot);
-		CU(cudaGetLastError());
-		CU(cudaMemcpyAsync(tot, d_tot, sizeof tot, cudaMemcpyDeviceToHost, c->copy_stream));
-		CU(cudaStreamSynchronize(c->copy_stream));
-	}
-	if (tot[1] > 0x7ffffff0ull)
+	if (n_rec > 0x7ffffff0ull)
 		return fail("too many records in one upload");
-	const int n_rec = (int)tot[1];
 	const size_t tab = (size_t)(n_rec + 1) * sizeof(int64_t);
-	if (ensure((void **)&c->d_rec_off, &c->rec_cap, tab) || ensure((void **)&c->d_hdr_off, &c->hdr_cap, tab))
+	if (c->d_rec_off.ensure(tab) || c->d_hdr_off.ensure(tab))
 		return -1;
 	c->rec_off.resize(n_rec + 1);
 	c->hdr_off.resize(n_rec + 1);
-	if (n > 0) {
-		const int blocks = (n_seg * 32 + 255) / 256;
-		gm_fastn_emit<<<blocks, 256, 0, c->copy_stream>>>(c->d_text, n, static_cast<const FastnSegStart *>(c->d_fstart),
-			n_seg, c->d_chars, c->d_rec_off, c->d_hdr_off);
-		CU(cudaGetLastError());
-	}
-	const int64_t last[2] = {(int64_t)tot[0], n};
+	return 0;
+}
+
+// ... and once the emit kernel is enqueued: the last entries (total_nt characters, the text's n_bytes),
+// both tables back to the host, and `extra` bytes from d_extra to h_extra, in one synchronise.
+static int fetch_records(gm_ctx *c, int64_t total_nt, int64_t n_bytes, void *h_extra, const void *d_extra, size_t extra)
+{
+	const size_t n_rec = c->rec_off.size() - 1, tab = (n_rec + 1) * sizeof(int64_t);
+	const int64_t last[2] = {total_nt, n_bytes};
 	CU(cudaMemcpyAsync(c->d_rec_off + n_rec, &last[0], sizeof(int64_t), cudaMemcpyHostToDevice, c->copy_stream));
 	CU(cudaMemcpyAsync(c->d_hdr_off + n_rec, &last[1], sizeof(int64_t), cudaMemcpyHostToDevice, c->copy_stream));
 	CU(cudaMemcpyAsync(c->rec_off.data(), c->d_rec_off, tab, cudaMemcpyDeviceToHost, c->copy_stream));
 	CU(cudaMemcpyAsync(c->hdr_off.data(), c->d_hdr_off, tab, cudaMemcpyDeviceToHost, c->copy_stream));
+	if (extra > 0)
+		CU(cudaMemcpyAsync(h_extra, d_extra, extra, cudaMemcpyDeviceToHost, c->copy_stream));
 	CU(cudaStreamSynchronize(c->copy_stream));
-	c->total_nt = (int64_t)tot[0];
+	c->total_nt = total_nt;
+	return 0;
+}
+
+// FN_fgetseq on the device, src/dbutil.c:42-128 (gm_fastn.cuh), over the n bytes of FASTA text in
+// d_text (enqueued on copy_stream, or already there; n_bytes = n): text -> kept characters + record
+// table (rec_off, hdr_off; blocks until they are known) -> 4-bit codes, asynchronously.
+static int read_fastn(gm_ctx *c, int64_t n, int64_t n_bytes)
+{
+	const int n_seg = (int)((n + GM_FASTN_SEG - 1) / GM_FASTN_SEG);
+	if (c->d_chars.ensure((size_t)n + 64) || c->d_fsum.ensure((size_t)(n_seg + 1) * sizeof(FastnSum) + 16) ||
+	    c->d_fstart.ensure((size_t)(n_seg + 1) * sizeof(FastnSegStart)))
+		return -1;
+	unsigned long long *d_tot = reinterpret_cast<unsigned long long *>(
+		static_cast<uint8_t *>(c->d_fsum.p) + (size_t)(n_seg + 1) * sizeof(FastnSum));
+	unsigned long long tot[2] = {0, 0};
+	if (n > 0) {
+		const int blocks = (n_seg * 32 + 255) / 256;
+		gm_fastn_summarize<<<blocks, 256, 0, c->copy_stream>>>(c->d_text, n, static_cast<FastnSum *>(c->d_fsum.p), n_seg);
+		CU(cudaGetLastError());
+		gm_fastn_scan<<<1, 1024, 0, c->copy_stream>>>(static_cast<const FastnSum *>(c->d_fsum.p), n_seg,
+			static_cast<FastnSegStart *>(c->d_fstart.p), d_tot);
+		CU(cudaGetLastError());
+		CU(cudaMemcpyAsync(tot, d_tot, sizeof tot, cudaMemcpyDeviceToHost, c->copy_stream));
+		CU(cudaStreamSynchronize(c->copy_stream));
+	}
+	if (size_records(c, tot[1]))
+		return -1;
+	if (n > 0) {
+		const int blocks = (n_seg * 32 + 255) / 256;
+		gm_fastn_emit<<<blocks, 256, 0, c->copy_stream>>>(c->d_text, n, static_cast<const FastnSegStart *>(c->d_fstart.p),
+			n_seg, c->d_chars, c->d_rec_off, c->d_hdr_off);
+		CU(cudaGetLastError());
+	}
+	if (fetch_records(c, (int64_t)tot[0], n_bytes, NULL, NULL, 0))
+		return -1;
 	if (c->rec_off[0] != 0)
 		return fail("fastn text has sequence before its first header");
 	return pack_text_records(c);
@@ -1956,58 +1924,46 @@ static int read_fastq(gm_ctx *c, int64_t n, int64_t n_bytes)
 	const int min_qual = c->min_qual, qual_offset = c->qual_offset;
 	// n + 64 bytes of d_chars also bound gm_fastq_mask's writes: a quality index is below the text's
 	// quality byte count, which is at most n
-	if (ensure((void **)&c->d_chars, &c->chars_cap, (size_t)n + 64) ||
-	    ensure(&c->d_fsum, &c->fsum_cap, (size_t)(n_seg + 1) * sizeof(FastqSum) + 32) ||
-	    ensure(&c->d_fstart, &c->fstart_cap, (size_t)(n_seg + 1) * sizeof(FastqSegStart)))
+	if (c->d_chars.ensure((size_t)n + 64) || c->d_fsum.ensure((size_t)(n_seg + 1) * sizeof(FastqSum) + 32) ||
+	    c->d_fstart.ensure((size_t)(n_seg + 1) * sizeof(FastqSegStart)))
 		return -1;
 	// totals (read bytes, records), then the first failing record's key (record << 2 | what), then
 	// (masking only) the first out-of-range quality byte's key (text offset << 8 | value)
 	unsigned long long *d_tot = reinterpret_cast<unsigned long long *>(
-		static_cast<uint8_t *>(c->d_fsum) + (size_t)(n_seg + 1) * sizeof(FastqSum));
+		static_cast<uint8_t *>(c->d_fsum.p) + (size_t)(n_seg + 1) * sizeof(FastqSum));
 	unsigned long long tot[2] = {0, 0}, bad[2] = {~0ull, ~0ull};
 	const size_t n_bad = min_qual > 0 ? 2 : 1;
 	CU(cudaMemsetAsync(d_tot + 2, 0xff, n_bad * sizeof(unsigned long long), c->copy_stream));
 	if (n > 0) {
 		const int blocks = (n_seg * 32 + 255) / 256;
-		gm_fastq_summarize<<<blocks, 256, 0, c->copy_stream>>>(c->d_text, n, static_cast<FastqSum *>(c->d_fsum), n_seg);
+		gm_fastq_summarize<<<blocks, 256, 0, c->copy_stream>>>(c->d_text, n, static_cast<FastqSum *>(c->d_fsum.p), n_seg);
 		CU(cudaGetLastError());
-		gm_fastq_scan<<<1, GM_FQ_SCAN_THREADS, 0, c->copy_stream>>>(static_cast<const FastqSum *>(c->d_fsum), n_seg,
-			static_cast<FastqSegStart *>(c->d_fstart), d_tot, d_tot + 2);
+		gm_fastq_scan<<<1, GM_FQ_SCAN_THREADS, 0, c->copy_stream>>>(static_cast<const FastqSum *>(c->d_fsum.p), n_seg,
+			static_cast<FastqSegStart *>(c->d_fstart.p), d_tot, d_tot + 2);
 		CU(cudaGetLastError());
 		CU(cudaMemcpyAsync(tot, d_tot, sizeof tot, cudaMemcpyDeviceToHost, c->copy_stream));
 		CU(cudaStreamSynchronize(c->copy_stream));
 	}
-	if (tot[1] > 0x7ffffff0ull)
-		return fail("too many records in one upload");
-	const int n_rec = (int)tot[1];
-	const size_t tab = (size_t)(n_rec + 1) * sizeof(int64_t);
-	if (ensure((void **)&c->d_rec_off, &c->rec_cap, tab) || ensure((void **)&c->d_hdr_off, &c->hdr_cap, tab))
+	if (size_records(c, tot[1]))
 		return -1;
-	c->rec_off.resize(n_rec + 1);
-	c->hdr_off.resize(n_rec + 1);
 	// record 0 starts at byte 0 and character 0; gm_fastq_emit writes every other record's entries
-	const int64_t first = 0, last[2] = {(int64_t)tot[0], n_bytes};
-	if (n_rec > 0) {
+	const int64_t first = 0;
+	if (tot[1] > 0) {
 		CU(cudaMemcpyAsync(c->d_rec_off, &first, sizeof(int64_t), cudaMemcpyHostToDevice, c->copy_stream));
 		CU(cudaMemcpyAsync(c->d_hdr_off, &first, sizeof(int64_t), cudaMemcpyHostToDevice, c->copy_stream));
 		const int blocks = (n_seg * 32 + 255) / 256;
-		gm_fastq_emit<<<blocks, 256, 0, c->copy_stream>>>(c->d_text, n, static_cast<const FastqSegStart *>(c->d_fstart),
+		gm_fastq_emit<<<blocks, 256, 0, c->copy_stream>>>(c->d_text, n, static_cast<const FastqSegStart *>(c->d_fstart.p),
 			n_seg, c->d_chars, c->d_rec_off, c->d_hdr_off, d_tot + 2);
 		CU(cudaGetLastError());
 		if (min_qual > 0) {
 			// behind emit on copy_stream, ahead of the pack (pack_text_records) that reads d_chars
-			gm_fastq_mask<<<blocks, 256, 0, c->copy_stream>>>(c->d_text, n, static_cast<const FastqSegStart *>(c->d_fstart),
+			gm_fastq_mask<<<blocks, 256, 0, c->copy_stream>>>(c->d_text, n, static_cast<const FastqSegStart *>(c->d_fstart.p),
 				n_seg, (unsigned)(qual_offset + min_qual), (unsigned)qual_offset, c->d_chars, d_tot + 3);
 			CU(cudaGetLastError());
 		}
 	}
-	CU(cudaMemcpyAsync(c->d_rec_off + n_rec, &last[0], sizeof(int64_t), cudaMemcpyHostToDevice, c->copy_stream));
-	CU(cudaMemcpyAsync(c->d_hdr_off + n_rec, &last[1], sizeof(int64_t), cudaMemcpyHostToDevice, c->copy_stream));
-	CU(cudaMemcpyAsync(c->rec_off.data(), c->d_rec_off, tab, cudaMemcpyDeviceToHost, c->copy_stream));
-	CU(cudaMemcpyAsync(c->hdr_off.data(), c->d_hdr_off, tab, cudaMemcpyDeviceToHost, c->copy_stream));
-	CU(cudaMemcpyAsync(bad, d_tot + 2, n_bad * sizeof bad[0], cudaMemcpyDeviceToHost, c->copy_stream));
-	CU(cudaStreamSynchronize(c->copy_stream));
-	c->total_nt = (int64_t)tot[0];
+	if (fetch_records(c, (int64_t)tot[0], n_bytes, bad, d_tot + 2, n_bad * sizeof bad[0]))
+		return -1;
 	if (bad[1] != ~0ull) {
 		// the record of the first out-of-range quality byte: the last one whose '@' lies before it; it
 		// is named unless a record before it, or the record itself, fails a format check
@@ -2035,29 +1991,6 @@ static int read_fastq(gm_ctx *c, int64_t n, int64_t n_bytes)
 	return pack_text_records(c);
 }
 
-extern "C" int gm_db_upload_fastn(gm_ctx *c, const char *text, size_t n_bytes)
-{
-	if (n_bytes > 0 && text == NULL)
-		return fail("text is NULL");
-	if (n_bytes > ((size_t)1 << 40))
-		return fail("text too long");
-	if (n_bytes > 0 && text[0] != '>')
-		return fail("fastn text does not begin with '>' (src/dbutil.c:56-60)");
-	if (begin_upload(c))
-		return -1;
-	NvtxRange nvtx_("gpumotif: upload fastn (H2D + device reader)");
-	if (ensure((void **)&c->d_text, &c->text_cap, n_bytes + 64))
-		return -1;
-	CU(cudaEventRecord(c->up_ev[0], c->copy_stream));
-	if (n_bytes > 0)
-		CU(cudaMemcpyAsync(c->d_text, text, n_bytes, cudaMemcpyHostToDevice, c->copy_stream));
-	if (read_fastn(c, (int64_t)n_bytes))
-		return -1;
-	c->stats.h2d_bytes = (uint64_t)n_bytes;
-	c->db = DB_FASTN;
-	return 0;
-}
-
 // FASTQ text without the line end after its last line ('\n', '\r\n' or '\r'): the length the reader
 // reads, from the last two bytes alone
 static int64_t fastq_trim(int64_t n, uint8_t b1, uint8_t b2)
@@ -2071,28 +2004,45 @@ static int64_t fastq_trim(int64_t n, uint8_t b1, uint8_t b2)
 	return n;
 }
 
-extern "C" int gm_db_upload_fastq(gm_ctx *c, const char *text, size_t n_bytes)
+// What the text uploads (gm_db_upload_fastn / _fastq and their BGZF forms) know of a format
+struct TextFormat {
+	char first;                       // the byte the text begins with
+	const char *not_first;            // refusal when it does not (plain text)
+	const char *not_first_bgzf;       // ... (the inflated text of BGZF members)
+	const char *nvtx, *nvtx_bgzf;     // range over the upload
+	int (*read)(gm_ctx *, int64_t n, int64_t n_bytes); // reads the first n of the n_bytes in d_text
+	bool trim;                        // the reader reads the text without its last line end (fastq_trim)
+	DbKind kind;
+};
+static const TextFormat FASTN_TEXT = {'>', "fastn text does not begin with '>' (src/dbutil.c:56-60)",
+				      "the text of the BGZF members does not begin with '>' (src/dbutil.c:56-60)",
+				      "gpumotif: upload fastn (H2D + device reader)",
+				      "gpumotif: upload BGZF fastn (H2D + inflate + device reader)", read_fastn, false, DB_FASTN};
+static const TextFormat FASTQ_TEXT = {'@', "FASTQ text does not begin with '@'",
+				      "the text of the BGZF members does not begin with '@'",
+				      "gpumotif: upload FASTQ (H2D + device reader)",
+				      "gpumotif: upload BGZF FASTQ (H2D + inflate + device reader)", read_fastq, true, DB_FASTQ};
+
+static int upload_text(gm_ctx *c, const TextFormat &f, const char *text, size_t n_bytes)
 {
 	if (n_bytes > 0 && text == NULL)
 		return fail("text is NULL");
 	if (n_bytes > ((size_t)1 << 40))
 		return fail("text too long");
-	if (n_bytes > 0 && text[0] != '@')
-		return fail("FASTQ text does not begin with '@'");
+	if (n_bytes > 0 && text[0] != f.first)
+		return fail("%s", f.not_first);
 	if (begin_upload(c))
 		return -1;
-	NvtxRange nvtx_("gpumotif: upload FASTQ (H2D + device reader)");
-	if (ensure((void **)&c->d_text, &c->text_cap, n_bytes + 64))
+	NvtxRange nvtx_(f.nvtx);
+	if (c->d_text.ensure(n_bytes + 64))
 		return -1;
 	CU(cudaEventRecord(c->up_ev[0], c->copy_stream));
 	if (n_bytes > 0)
 		CU(cudaMemcpyAsync(c->d_text, text, n_bytes, cudaMemcpyHostToDevice, c->copy_stream));
 	const int64_t n = (int64_t)n_bytes;
-	if (read_fastq(c, fastq_trim(n, n > 1 ? text[n - 2] : 0, n > 0 ? text[n - 1] : 0), n))
+	if (f.read(c, f.trim ? fastq_trim(n, n > 1 ? text[n - 2] : 0, n > 0 ? text[n - 1] : 0) : n, n))
 		return -1;
-	c->stats.h2d_bytes = (uint64_t)n_bytes;
-	c->db = DB_FASTQ;
-	return 0;
+	return finish_upload(c, f.kind, (uint64_t)n_bytes);
 }
 
 static uint32_t le32(const uint8_t *p) { return p[0] | (p[1] << 8) | (p[2] << 16) | ((uint32_t)p[3] << 24); }
@@ -2186,13 +2136,12 @@ static int inflate_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_bytes, std::vecto
 {
 	const int n_mem = (int)mem.size();
 	const size_t tab = (size_t)n_mem * sizeof(BgzfMember);
-	if (ensure((void **)&c->d_text, &c->text_cap, (size_t)total + 64) || ensure((void **)&c->d_gz, &c->gz_cap, n_bytes + 16) ||
-	    ensure(&c->d_bgzf, &c->bgzf_cap, tab + 8 + (size_t)n_mem))
+	if (c->d_text.ensure((size_t)total + 64) || c->d_gz.ensure(n_bytes + 16) || c->d_bgzf.ensure(tab + 8 + (size_t)n_mem))
 		return -1;
 	c->bgzf.swap(mem);
-	BgzfMember *d_mem = static_cast<BgzfMember *>(c->d_bgzf);
-	unsigned int *d_first = reinterpret_cast<unsigned int *>(static_cast<uint8_t *>(c->d_bgzf) + tab);
-	uint8_t *d_status = static_cast<uint8_t *>(c->d_bgzf) + tab + 8;
+	BgzfMember *d_mem = reinterpret_cast<BgzfMember *>(c->d_bgzf.p);
+	unsigned int *d_first = reinterpret_cast<unsigned int *>(c->d_bgzf + tab);
+	uint8_t *d_status = c->d_bgzf + tab + 8;
 	*ends = TextEnds{0, {0, 0}};
 	CU(cudaEventRecord(c->up_ev[0], c->copy_stream));
 	if (n_mem == 0)
@@ -2206,18 +2155,13 @@ static int inflate_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_bytes, std::vecto
 		return -1;
 	const int n_chunks = (int)c->chunk_end.size();
 	int m0 = 0;
-	size_t copied = 0;
+	int64_t copied = 0;
 	for (int i = 0; i < n_chunks; i++) {
 		int m1 = m0;
 		while (m1 < n_mem && (i == n_chunks - 1 || (int64_t)starts[m1] < c->chunk_end[i]))
 			m1++;
-		const size_t upto = m1 < n_mem ? starts[m1] : n_bytes;
-		if (upto > copied)
-			CU(cudaMemcpyAsync(c->d_gz + copied, gz + copied, upto - copied, cudaMemcpyHostToDevice, c->copy_stream));
-		copied = std::max(copied, upto);
-		CU(cudaEventRecord(c->cp_ev[i], c->copy_stream));
+		CU(stage_copy(c, i, c->d_gz, gz, &copied, (int64_t)(m1 < n_mem ? starts[m1] : n_bytes)));
 		if (m1 > m0) {
-			CU(cudaStreamWaitEvent(c->pack_stream, c->cp_ev[i], 0));
 			// one thread per member, spread over the SMs: the decode is a chain of dependent loads
 			const int m = m1 - m0;
 			const int tpb = std::min(32, std::max(1, (m + c->n_sm - 1) / c->n_sm));
@@ -2247,8 +2191,8 @@ static int inflate_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_bytes, std::vecto
 	return 0;
 }
 
-// The members inflated as above, then the text read as gm_db_upload_fastn reads it.
-extern "C" int gm_db_upload_fastn_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_bytes)
+// The members inflated as above, then the text read as upload_text reads it.
+static int upload_text_bgzf(gm_ctx *c, const TextFormat &f, const uint8_t *gz, size_t n_bytes)
 {
 	std::vector<BgzfMember> mem;
 	std::vector<size_t> starts; // each member's offset in gz
@@ -2257,42 +2201,28 @@ extern "C" int gm_db_upload_fastn_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_by
 		return -1;
 	if (begin_upload(c))
 		return -1;
-	NvtxRange nvtx_("gpumotif: upload BGZF fastn (H2D + inflate + device reader)");
+	NvtxRange nvtx_(f.nvtx_bgzf);
 	const size_t tab = mem.size() * sizeof(BgzfMember);
 	TextEnds ends;
 	if (inflate_bgzf(c, gz, n_bytes, mem, starts, total, &ends))
 		return -1;
-	if (total > 0 && ends.head != '>')
-		return fail("the text of the BGZF members does not begin with '>' (src/dbutil.c:56-60)");
-	if (read_fastn(c, (int64_t)total))
+	if (total > 0 && ends.head != f.first)
+		return fail("%s", f.not_first_bgzf);
+	const int64_t n = (int64_t)total;
+	if (f.read(c, f.trim ? fastq_trim(n, ends.tail[0], ends.tail[1]) : n, n))
 		return -1;
-	c->stats.h2d_bytes = (uint64_t)n_bytes + (uint64_t)tab;
-	c->db = DB_FASTN;
-	return 0;
+	return finish_upload(c, f.kind, (uint64_t)n_bytes + (uint64_t)tab);
 }
 
-// The members inflated as above, then the text read as gm_db_upload_fastq reads it.
+extern "C" int gm_db_upload_fastn(gm_ctx *c, const char *text, size_t n_bytes) { return upload_text(c, FASTN_TEXT, text, n_bytes); }
+extern "C" int gm_db_upload_fastq(gm_ctx *c, const char *text, size_t n_bytes) { return upload_text(c, FASTQ_TEXT, text, n_bytes); }
+extern "C" int gm_db_upload_fastn_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_bytes)
+{
+	return upload_text_bgzf(c, FASTN_TEXT, gz, n_bytes);
+}
 extern "C" int gm_db_upload_fastq_bgzf(gm_ctx *c, const uint8_t *gz, size_t n_bytes)
 {
-	std::vector<BgzfMember> mem;
-	std::vector<size_t> starts; // each member's offset in gz
-	uint64_t total = 0;
-	if (bgzf_members(gz, n_bytes, mem, starts, &total))
-		return -1;
-	if (begin_upload(c))
-		return -1;
-	NvtxRange nvtx_("gpumotif: upload BGZF FASTQ (H2D + inflate + device reader)");
-	const size_t tab = mem.size() * sizeof(BgzfMember);
-	TextEnds ends;
-	if (inflate_bgzf(c, gz, n_bytes, mem, starts, total, &ends))
-		return -1;
-	if (total > 0 && ends.head != '@')
-		return fail("the text of the BGZF members does not begin with '@'");
-	if (read_fastq(c, fastq_trim((int64_t)total, ends.tail[0], ends.tail[1]), (int64_t)total))
-		return -1;
-	c->stats.h2d_bytes = (uint64_t)n_bytes + (uint64_t)tab;
-	c->db = DB_FASTQ;
-	return 0;
+	return upload_text_bgzf(c, FASTQ_TEXT, gz, n_bytes);
 }
 
 extern "C" int gm_db_get_text(gm_ctx *c, int64_t off, int64_t n, char *out)
@@ -2384,9 +2314,8 @@ extern "C" int64_t gm_db_total_nt(const gm_ctx *c) { return c == NULL ? -1 : c->
 static int launch(gm_ctx *c)
 {
 	NvtxRange nvtx_("gpumotif: launch sieve / enumeration kernels");
-	if (c->d_hits == NULL) {
-		CU(cudaMalloc(&c->d_hits, c->hit_cap * (size_t)c->stride_words * 4));
-	}
+	if (c->d_hits.p == NULL)
+		CU(c->d_hits.alloc(c->hit_cap * (size_t)c->stride_words * 4));
 	CU(cudaMemsetAsync(c->d_counters, 0, 32 * sizeof(unsigned long long), c->stream));
 	ScanArgs A;
 	A.par = c->par;
@@ -2410,7 +2339,7 @@ static int launch(gm_ctx *c)
 	A.wl_count = c->d_counters + 3;
 	A.wl_head = c->d_counters + 4;
 	A.wl_cap = 0;
-	CU(cudaEventRecord(c->ev[3], c->stream));
+	CU(cudaEventRecord(c->scan_ev[0], c->stream));
 	c->n_seg_ev = 0;
 	const int n_chunks = (int)c->chunk_end.size();
 	if (A.n_tiles > 0 && !c->use_split && c->upload_fresh && n_chunks > 1 && n_chunks <= 16) {
@@ -2470,10 +2399,8 @@ static int launch(gm_ctx *c)
 		// segments (gm_scan_finish), nothing is lost.
 		const size_t need = wl_entries();
 		const int64_t seg = std::min<int64_t>(c->seg_nt, c->p_end - c->p_begin);
-		if (c->d_wl == NULL || c->wl_cap < need) {
-			cudaFree(c->d_wl);
-			c->d_wl = NULL;
-			CU(cudaMalloc(&c->d_wl, need * GM_WL_WORDS * 4));
+		if (c->d_wl.p == NULL || c->wl_cap < need) {
+			CU(c->d_wl.alloc(need * GM_WL_WORDS * 4));
 			c->wl_cap = need;
 		}
 		A.wl = c->d_wl;
@@ -2509,11 +2436,8 @@ static int launch(gm_ctx *c)
 			// the tile counter restarts for every filter launch
 			CU(cudaMemsetAsync(c->d_counters + 0, 0, sizeof(unsigned long long), c->stream));
 			int ablocks = (int)std::min<int64_t>(c->a_blocks, A.n_tiles);
-			while ((int)c->seg_ev.size() < 2 * (c->n_seg_ev + 1)) {
-				cudaEvent_t e;
-				CU(cudaEventCreate(&e));
-				c->seg_ev.push_back(e);
-			}
+			if (c->seg_ev.grow(2 * (c->n_seg_ev + 1), cudaEventDefault))
+				return -1;
 			CU(cudaEventRecord(c->seg_ev[2 * c->n_seg_ev], c->stream));
 			pre_kernel(pre_pf(c->par))<<<ablocks, c->a_threads, c->a_smem, c->stream>>>(A);
 			CU(cudaGetLastError());
@@ -2527,7 +2451,7 @@ static int launch(gm_ctx *c)
 			}
 		}
 	}
-	CU(cudaEventRecord(c->ev[4], c->stream));
+	CU(cudaEventRecord(c->scan_ev[1], c->stream));
 	c->upload_fresh = false;
 	return 0;
 }
@@ -2560,11 +2484,6 @@ extern "C" int gm_scan_launch(gm_ctx *c, int64_t g_begin, int64_t g_end, int str
 	c->pending = true;
 	return 0;
 }
-
-struct HitKey {
-	uint32_t rec, comp, szero, seq;
-	uint32_t idx;
-};
 
 // ---- ordering the candidates on the device --------------------------------
 // Enumeration order = (record, strand, start, DFS rank).  A start is enumerated
@@ -2609,7 +2528,7 @@ extern "C" int gm_scan_finish(gm_ctx *c)
 		CU(cudaMemcpyAsync(cnt, c->d_counters, sizeof cnt, cudaMemcpyDeviceToHost, c->stream));
 		CU(cudaStreamSynchronize(c->stream));
 		float ms = 0;
-		cudaEventElapsedTime(&ms, c->ev[3], c->ev[4]);
+		cudaEventElapsedTime(&ms, c->scan_ev[0], c->scan_ev[1]);
 		c->stats.kernel_ms += ms;
 		for (int i = 0; i < c->n_seg_ev; i++) {
 			float f = 0;
@@ -2653,8 +2572,7 @@ extern "C" int gm_scan_finish(gm_ctx *c)
 				    "(gm_scan(ctx, lo, hi, ...)) or tighten the descriptor",
 				    cnt[1], (double)cnt[1] * c->stride_words * 4 / 1e9);
 		c->stats.n_retries++;
-		cudaFree(c->d_hits);
-		c->d_hits = NULL;
+		c->d_hits.reset();
 		c->hit_cap = (size_t)cnt[1] + (size_t)cnt[1] / 16 + 1024;
 		if (launch(c))
 			return -1;
@@ -2678,14 +2596,8 @@ extern "C" int gm_scan_finish(gm_ctx *c)
 		n_rej = (size_t)rej;
 	}
 	const size_t n = n_all - n_rej; // candidates handed to the caller
-	if (n_all * sw > c->h_raw_cap) {
-		cudaFreeHost(c->h_raw);
-		c->h_raw = NULL;
-		c->h_raw_cap = 0;
-		const size_t want = n_all * sw + n_all * sw / 4 + 4096;
-		CU(cudaMallocHost(&c->h_raw, want * 4));
-		c->h_raw_cap = want;
-	}
+	if (c->h_raw.ensure(n_all * sw))
+		return -1;
 	const uint32_t *raw = c->h_raw;
 	auto t0 = std::chrono::steady_clock::now();
 	auto t1 = t0, t2 = t0;
@@ -2696,13 +2608,9 @@ extern "C" int gm_scan_finish(gm_ctx *c)
 		cub::DeviceRadixSort::SortPairs(NULL, temp, (unsigned long long *)NULL, (unsigned long long *)NULL,
 			(uint32_t *)NULL, (uint32_t *)NULL, (unsigned long long)n_all, 0, 64, c->stream);
 		const size_t k_bytes = (n_all * 8 + 255) & ~(size_t)255, i_bytes = (n_all * 4 + 255) & ~(size_t)255;
-		if (ensure(&c->d_sort, &c->sort_cap, 2 * k_bytes + 2 * i_bytes + temp + 256))
+		if (c->d_sort.ensure(2 * k_bytes + 2 * i_bytes + temp + 256) || c->d_sorted.ensure(std::max<size_t>(n, 1) * sw * 4))
 			return -1;
-		size_t sorted_bytes = c->sorted_cap;
-		if (ensure((void **)&c->d_sorted, &sorted_bytes, std::max<size_t>(n, 1) * sw * 4))
-			return -1;
-		c->sorted_cap = sorted_bytes;
-		uint8_t *b = (uint8_t *)c->d_sort;
+		uint8_t *b = c->d_sort;
 		unsigned long long *k_in = (unsigned long long *)b, *k_out = (unsigned long long *)(b + k_bytes);
 		uint32_t *i_in = (uint32_t *)(b + 2 * k_bytes), *i_out = (uint32_t *)(b + 2 * k_bytes + i_bytes);
 		void *d_temp = b + 2 * k_bytes + 2 * i_bytes;
@@ -2722,30 +2630,30 @@ extern "C" int gm_scan_finish(gm_ctx *c)
 		c->hits_view = c->h_raw;
 		// (sort_ms = device ordering, d2h_ms = the copy; swapped below)
 	} else {
-	if (n_all > 0)
-		CU(cudaMemcpy(c->h_raw, c->d_hits, n_all * sw * 4, cudaMemcpyDeviceToHost));
-	t1 = std::chrono::steady_clock::now();
-	// enumeration order: record, strand, start, DFS rank.  Two 64-bit keys per
-	// hit: (rec, comp, szero) and (seq, index into the gathered array)
-	std::vector<uint64_t> &keys = c->keys;
-	keys.resize(2 * n);
-	for (size_t i = 0, k = 0; i < n_all; i++) {
-		const uint32_t *h = &raw[i * sw];
-		if (h[3] >> 31)
-			continue; // rejected by the score pre-screen
-		keys[2 * k] = ((uint64_t)h[0] << 32) | ((uint64_t)(h[3] & 1) << 31) | (uint64_t)(h[1] & 0x7fffffffu);
-		keys[2 * k + 1] = ((uint64_t)h[2] << 32) | (uint64_t)i;
-		k++;
-	}
-	struct K2 { uint64_t a, b; };
-	K2 *kp = reinterpret_cast<K2 *>(keys.data());
-	std::sort(kp, kp + n, [](const K2 &x, const K2 &y) { return x.a != y.a ? x.a < y.a : x.b < y.b; });
-	if (c->hits.size() < n * sw)
-		c->hits.resize(n * sw + n * sw / 4);
-	for (size_t i = 0; i < n; i++)
-		memcpy(&c->hits[i * sw], &raw[(size_t)(uint32_t)kp[i].b * sw], sw * 4);
-	t2 = std::chrono::steady_clock::now();
-	c->hits_view = c->hits.data();
+		if (n_all > 0)
+			CU(cudaMemcpy(c->h_raw, c->d_hits, n_all * sw * 4, cudaMemcpyDeviceToHost));
+		t1 = std::chrono::steady_clock::now();
+		// enumeration order: record, strand, start, DFS rank.  Two 64-bit keys per
+		// hit: (rec, comp, szero) and (seq, index into the gathered array)
+		std::vector<uint64_t> &keys = c->keys;
+		keys.resize(2 * n);
+		for (size_t i = 0, k = 0; i < n_all; i++) {
+			const uint32_t *h = &raw[i * sw];
+			if (h[3] >> 31)
+				continue; // rejected by the score pre-screen
+			keys[2 * k] = ((uint64_t)h[0] << 32) | ((uint64_t)(h[3] & 1) << 31) | (uint64_t)(h[1] & 0x7fffffffu);
+			keys[2 * k + 1] = ((uint64_t)h[2] << 32) | (uint64_t)i;
+			k++;
+		}
+		struct K2 { uint64_t a, b; };
+		K2 *kp = reinterpret_cast<K2 *>(keys.data());
+		std::sort(kp, kp + n, [](const K2 &x, const K2 &y) { return x.a != y.a ? x.a < y.a : x.b < y.b; });
+		if (c->hits.size() < n * sw)
+			c->hits.resize(n * sw + n * sw / 4);
+		for (size_t i = 0; i < n; i++)
+			memcpy(&c->hits[i * sw], &raw[(size_t)(uint32_t)kp[i].b * sw], sw * 4);
+		t2 = std::chrono::steady_clock::now();
+		c->hits_view = c->hits.data();
 	}
 	c->n_hits = n;
 	c->n_raw = n_all;
@@ -2840,16 +2748,8 @@ extern "C" int gm_hit_windows(gm_ctx *c, int lead, int trail, const char **win, 
 	const size_t n = c->n_hits;
 	const size_t n_dev = c->dev_sorted ? n : c->n_raw; // the unsorted buffer still holds the rejected ones
 	const size_t bytes = n_dev * (size_t)wlen;
-	if (ensure((void **)&c->d_win, &c->win_cap, bytes + 16))
+	if (c->d_win.ensure(bytes + 16) || c->h_win.ensure(bytes))
 		return -1;
-	if (bytes > c->h_win_cap) {
-		cudaFreeHost(c->h_win);
-		c->h_win = NULL;
-		c->h_win_cap = 0;
-		const size_t want = bytes + bytes / 4 + 4096;
-		CU(cudaMallocHost(&c->h_win, want));
-		c->h_win_cap = want;
-	}
 	if (n_dev > 0) {
 		const int blocks = (int)std::min<size_t>(n_dev, (size_t)c->n_sm * 32);
 		// after a 2-bit upload the windows are decoded from the 4-bit codes

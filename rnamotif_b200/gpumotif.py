@@ -130,6 +130,13 @@ def _err():
     return lib().gm_last_error().decode("utf-8", "replace")
 
 
+def _u8(data) -> np.ndarray:
+    """bytes, bytearray, memoryview or an array as a contiguous uint8 array (no copy where it already is one)."""
+    if isinstance(data, (bytes, bytearray, memoryview)):
+        data = np.frombuffer(data, dtype=np.uint8)
+    return np.ascontiguousarray(data, dtype=np.uint8)
+
+
 def plan_describe(plan: bytes) -> str:
     """What the library derives from a plan (per-search table, level-0 filter,
     look-ahead targets, probes) as text.  Host side, needs no device."""
@@ -236,10 +243,7 @@ class MotifSearch:
     def upload_fastn(self, text):
         """gm_db_upload_fastn: `text` = FASTA as it sits in the file (bytes or a uint8
         array); the reader of src/dbutil.c:42-128 runs on the device."""
-        if isinstance(text, (bytes, bytearray, memoryview)):
-            text = np.frombuffer(text, dtype=np.uint8)
-        text = np.ascontiguousarray(text, dtype=np.uint8)
-        self._keep = text
+        text = self._keep = _u8(text)
         self._ck(lib().gm_db_upload_fastn(self._ctx, text.ctypes.data, text.size), "gm_db_upload_fastn")
 
     def upload_fastn_ptr(self, host_ptr: int, n_bytes: int):
@@ -268,9 +272,7 @@ class MotifSearch:
         """gm_db_upload_fastn_bgzf: `buf` = a BGZF-compressed FASTA file's bytes (bytes or a uint8
         array, pinned or pageable); the members are inflated and read on the device.  Returns when
         the record table is known, so `buf` may be reused."""
-        if isinstance(buf, (bytes, bytearray, memoryview)):
-            buf = np.frombuffer(buf, dtype=np.uint8)
-        buf = np.ascontiguousarray(buf, dtype=np.uint8)
+        buf = _u8(buf)
         self.upload_fastn_bgzf_ptr(buf.ctypes.data, buf.size)
 
     def upload_fastn_bgzf_ptr(self, host_ptr: int, n_bytes: int):
@@ -279,10 +281,7 @@ class MotifSearch:
     def upload_fastq(self, text):
         """gm_db_upload_fastq: `text` = four-line FASTQ as it sits in the file (bytes or a uint8
         array); the reads are taken out and the format is checked on the device."""
-        if isinstance(text, (bytes, bytearray, memoryview)):
-            text = np.frombuffer(text, dtype=np.uint8)
-        text = np.ascontiguousarray(text, dtype=np.uint8)
-        self._keep = text
+        text = self._keep = _u8(text)
         self.upload_fastq_ptr(text.ctypes.data, text.size)
 
     def upload_fastq_ptr(self, host_ptr: int, n_bytes: int):
@@ -292,9 +291,7 @@ class MotifSearch:
         """gm_db_upload_fastq_bgzf: `buf` = a BGZF-compressed FASTQ file's bytes (bytes or a uint8
         array, pinned or pageable); the members are inflated and read on the device.  Returns when
         the record table is known, so `buf` may be reused."""
-        if isinstance(buf, (bytes, bytearray, memoryview)):
-            buf = np.frombuffer(buf, dtype=np.uint8)
-        buf = np.ascontiguousarray(buf, dtype=np.uint8)
+        buf = _u8(buf)
         self.upload_fastq_bgzf_ptr(buf.ctypes.data, buf.size)
 
     def upload_fastq_bgzf_ptr(self, host_ptr: int, n_bytes: int):
