@@ -156,6 +156,36 @@ int gm_host_pack(const char *seq, int64_t n, uint8_t *packed, int n_threads);
 int gm_db_upload_2bit(gm_ctx *c, const uint8_t *dna, size_t n_bytes, const int64_t *dna_off,
 		      const int64_t *rec_off, int n_rec, const int64_t *nblk, int64_t n_nblk);
 
+/* A new batch built on the device from blocks of the batch the context holds, whichever upload
+ * (or earlier gm_db_assemble) made it -- spliced transcripts, UTRs or any other regions of an
+ * uploaded genome, without a pass over the sequence on the host.  The new batch replaces the held
+ * one like an upload.  Block k is [blk[2k], blk[2k+1]) in the held batch's rec_off coordinates and
+ * lies inside one held record; blocks may come in any order, overlap and repeat, and may be empty.
+ * New record r is blocks rec_blk[r] .. rec_blk[r+1]-1 concatenated in that order; with strand[r] = 1
+ * it is the reverse complement of that concatenation as mk_rcmp builds it (src/rnamot.c:193-216:
+ * reversed, a <-> t, c <-> g, every other code n), i.e. what the held batch's complementary strand
+ * reads over those nucleotides.  Empty records are fine; n_rec = 0 gives an empty database.
+ *   - what the new batch holds: after a batch with characters on the device (gm_db_upload_chars,
+ *     gm_db_set_device_chars, the FASTA and FASTQ uploads) characters again -- a plus record's bytes
+ *     as they were, a minus record's mk_rcmp letters (a c g t n) -- in a buffer of the context's
+ *     own, so gm_hit_windows and gm_db_get_chars work and a caller's device buffer is only read;
+ *     after gm_db_upload_2bit exact codes, which the same calls decode; after
+ *     gm_db_upload_chars_hostpack the codes only (those two calls are refused).  FASTQ
+ *     quality masking already applied stays applied.  gm_db_records gives hdr_off = NULL and
+ *     gm_db_get_text is refused;
+ *   - it waits for the previous upload to finish (its copies and the host-pack thread); if that
+ *     upload failed, so does this call, leaving no database;
+ *   - refused with the held batch intact: no database held, a scan in flight, a NULL table with
+ *     counts > 0, n_rec < 0 or n_blk < 0, rec_blk[0] != 0, rec_blk not ascending, rec_blk[n_rec] !=
+ *     n_blk, a block that ends before it starts, lies outside [0, total_nt) or crosses the end of
+ *     the held record it starts in (the message names the block and the record), a strand byte
+ *     other than 0 or 1, a new record longer than gm_db_upload_chars accepts;
+ *   - cut into chunks that the next gm_scan streams in, like the uploads.
+ * gm_scan_stats_t::h2d_bytes = the new record table + the block table as sent (16 bytes per
+ * non-empty block, 8 more). */
+int gm_db_assemble(gm_ctx *c, const int64_t *blk, int64_t n_blk, const int64_t *rec_blk, const uint8_t *strand,
+		   int n_rec);
+
 /* Same, for characters that already live in device memory (a CUDA device
  * pointer, e.g. torch tensor storage). */
 int gm_db_set_device_chars(gm_ctx *c, const void *d_seq, const int64_t *rec_off, int n_rec);

@@ -3,6 +3,8 @@
 //   gm_pack_kernel     chars (what FN_fgetseq leaves, src/dbutil.c:105-111)
 //                      -> 4-bit IUPAC codes, two per byte
 //   gm_unpack2_kernel  UCSC .2bit bytes + N ranges -> the same 4-bit codes
+//   gm_assemble_kernel blocks of the held codes (and characters), reverse-complemented
+//                      where asked -> a new batch's codes (and characters)
 //   gm_inflate_kernel  BGZF members -> FASTA text, one thread per member
 //   gm_search_kernel   persistent CTAs; each takes tiles of consecutive start
 //                      positions from a global counter, stages the packed
@@ -19,6 +21,7 @@
 #include "gm_search.cuh"
 #include "gm_score.h"
 #include "gm_twobit.h"
+#include "gm_assemble.h"
 #include "gm_inflate.h"
 
 namespace gm {
@@ -205,6 +208,81 @@ __global__ void __launch_bounds__(256) gm_unpack2_kernel(const uint8_t *__restri
 				}
 			}
 			*reinterpret_cast<uint2 *>(packed + (gg >> 1)) = make_uint2(lo, hi);
+		}
+		__syncthreads(); // br is rewritten by the next round
+	}
+}
+
+// gm_db_assemble: nucleotides [g0, g0 + n) of a new batch gathered from the packed codes of the held one
+// (g0 a multiple of 16; nucleotides past g0 + n, the end of the batch, read 0).  The new batch is n_seg
+// non-empty segments, segment k at [seg_out[k], seg_out[k+1]) of it (seg_out ascending, seg_out[0] = 0).
+// seg_src[k] >= 0: a plus segment, a copy of src from nucleotide seg_src[k] on; seg_src[k] < 0: a minus
+// segment, read from nucleotide ~seg_src[k] of src DOWNWARDS and complemented (comp4).  One thread per
+// 16-nucleotide group, one 8-byte store; a block first brackets the segments its 256 groups touch, as
+// gm_unpack2_kernel brackets records.  Fast path: the group lies in one segment -- two aligned 64-bit
+// loads and a funnel shift (gm_assemble.h) at any nibble offset, reversed and complemented on a minus
+// segment.  Otherwise nucleotide by nucleotide.  CHARS: also the characters, into `chars`: a plus
+// segment's bytes as they are in src_chars, a minus segment's as the letters of the complemented codes.
+template <bool CHARS>
+__global__ void __launch_bounds__(256) gm_assemble_kernel(const uint8_t *__restrict__ src, const uint8_t *__restrict__ src_chars,
+	const int64_t *__restrict__ seg_out, const int64_t *__restrict__ seg_src, int64_t n_seg, int64_t g0, int64_t n,
+	uint8_t *__restrict__ packed, uint8_t *__restrict__ chars)
+{
+	__shared__ int64_t br[2]; // segments of the block's first and last nucleotide
+	const uint64_t *__restrict__ src64 = reinterpret_cast<const uint64_t *>(src);
+	const int64_t span = 256 * 16, end = g0 + n;
+	for (int64_t b0 = g0 + (int64_t)blockIdx.x * span; b0 < end; b0 += (int64_t)gridDim.x * span) {
+		const int64_t b1 = min(b0 + span, end);
+		if (threadIdx.x == 0)
+			br[0] = last_le(seg_out, 0, n_seg - 1, b0);
+		else if (threadIdx.x == 1)
+			br[1] = last_le(seg_out, 0, n_seg - 1, b1 - 1);
+		__syncthreads();
+		const int64_t gg = b0 + (int64_t)threadIdx.x * 16;
+		if (gg < b1) {
+			int64_t k = last_le(seg_out, br[0], br[1], gg);
+			uint64_t out = 0;
+			uint32_t ch[4] = {0, 0, 0, 0};
+			if (gg + 16 <= seg_out[k + 1]) {
+				const int64_t s = seg_src[k], d = gg - seg_out[k];
+				const int64_t p = s >= 0 ? s + d : ~s - d - 15; // the lowest source nucleotide
+				const uint64_t w0 = src64[p >> 4], w1 = src64[(p >> 4) + 1];
+				if (s >= 0) {
+					out = asm_window(w0, w1, (int)(p & 15));
+					if (CHARS)
+						for (int j = 0; j < 16; j++)
+							ch[j >> 2] |= (uint32_t)src_chars[p + j] << (8 * (j & 3));
+				} else {
+					out = asm_rc16(w0, w1, (int)(p & 15));
+					if (CHARS)
+						for (int j = 0; j < 16; j++)
+							ch[j >> 2] |= acgtn_letter((uint32_t)(out >> (4 * j)) & 15) << (8 * (j & 3));
+				}
+			} else {
+				for (int j = 0; j < 16; j++) {
+					const int64_t g = gg + j;
+					if (g >= end)
+						break;
+					while (g >= seg_out[k + 1])
+						k++;
+					const int64_t s = seg_src[k];
+					const int64_t p = s >= 0 ? s + (g - seg_out[k]) : ~s - (g - seg_out[k]);
+					uint32_t code = (src[p >> 1] >> (4 * (int)(p & 1))) & 15;
+					if (s < 0)
+						code = comp4(code);
+					out |= (uint64_t)code << (4 * j);
+					if (CHARS)
+						ch[j >> 2] |= (s >= 0 ? (uint32_t)src_chars[p] : acgtn_letter(code)) << (8 * (j & 3));
+				}
+			}
+			*reinterpret_cast<uint2 *>(packed + (gg >> 1)) = make_uint2((uint32_t)out, (uint32_t)(out >> 32));
+			if (CHARS) {
+				if (gg + 16 <= end)
+					*reinterpret_cast<uint4 *>(chars + gg) = make_uint4(ch[0], ch[1], ch[2], ch[3]);
+				else
+					for (int j = 0; gg + j < end; j++)
+						chars[gg + j] = (uint8_t)(ch[j >> 2] >> (8 * (j & 3)));
+			}
 		}
 		__syncthreads(); // br is rewritten by the next round
 	}

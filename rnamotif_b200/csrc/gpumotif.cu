@@ -98,6 +98,11 @@ template <class T> struct DevBuf : NoCopy {
 		}
 		return 0;
 	}
+	void swap(DevBuf &o)
+	{
+		std::swap(p, o.p);
+		std::swap(cap, o.cap);
+	}
 };
 
 // Pinned host memory.  cap is in elements, and ensure() takes a quarter and 4096 elements more than
@@ -220,6 +225,11 @@ struct gm_ctx {
 	// then the N ranges, on the device (d_tb) and on the host (tb)
 	DevBuf<int64_t> d_tb;
 	std::vector<int64_t> tb;
+	// gm_db_assemble: the new batch's segments (seg_out, then seg_src: gm_assemble_kernel) on the device
+	// and on the host, and the buffers it gathers into, swapped with d_packed and d_chars when it is done
+	DevBuf<int64_t> d_asm;
+	std::vector<int64_t> asm_tab;
+	DevBuf<uint8_t> d_packed_spare, d_chars_spare;
 	// BGZF upload (gm_db_upload_fastn_bgzf): the compressed bytes (d_gz); the member table, then the first
 	// failing member (u32), then a status byte per member (d_bgzf); the member table on the host (bgzf)
 	DevBuf<uint8_t> d_gz;
@@ -1505,10 +1515,8 @@ static int finish_upload(gm_ctx *c, DbKind kind, uint64_t h2d_bytes)
 }
 
 // the 4-bit codes of n nucleotides; slack: kernels read whole 16-byte groups past the end
-static int ensure_packed(gm_ctx *c, int64_t n)
-{
-	return c->d_packed.ensure((size_t)(((n + 15) / 16) * 8) + 1024);
-}
+static size_t packed_bytes(int64_t n) { return (size_t)(((n + 15) / 16) * 8) + 1024; }
+static int ensure_packed(gm_ctx *c, int64_t n) { return c->d_packed.ensure(packed_bytes(n)); }
 
 // blocks of 256 threads for a pack / expand kernel over len nucleotides, one 16-nt group per thread
 static int pack_blocks(const gm_ctx *c, int64_t len)
@@ -1830,6 +1838,109 @@ extern "C" int gm_db_upload_2bit(gm_ctx *c, const uint8_t *dna, size_t n_bytes, 
 	}
 	// bytes over the link: the span, the record table, dna_off and the N ranges
 	return finish_upload(c, DB_2BIT, (uint64_t)span + (uint64_t)(n_rec + 1) * 8 + (uint64_t)tb_bytes);
+}
+
+// A new batch from blocks of the held one, gathered on the device (gm_assemble_kernel).  Every check is
+// made against the held batch's record table before begin_upload drops it; the kernels read the held
+// codes (and characters) in place and write the spare buffers, which then take d_packed's and d_chars's
+// place.
+extern "C" int gm_db_assemble(gm_ctx *c, const int64_t *blk, int64_t n_blk, const int64_t *rec_blk, const uint8_t *strand,
+			      int n_rec)
+{
+	if (c == NULL)
+		return fail("ctx is NULL");
+	if (c->pending)
+		return fail("a scan is in flight");
+	if (c->db == DB_NONE)
+		return fail("no database uploaded");
+	if (n_rec < 0 || n_blk < 0 || (n_blk > 0 && blk == NULL) || (n_rec > 0 && (rec_blk == NULL || strand == NULL)))
+		return fail("bad assembly table");
+	if (rec_blk != NULL && rec_blk[0] != 0)
+		return fail("rec_blk[0] must be 0");
+	for (int r = 0; r < n_rec; r++)
+		if (rec_blk[r + 1] < rec_blk[r])
+			return fail("rec_blk not ascending at %d", r);
+	if ((rec_blk != NULL ? rec_blk[n_rec] : 0) != n_blk)
+		return fail("rec_blk[%d] = %lld, not n_blk = %lld", n_rec, (long long)(rec_blk != NULL ? rec_blk[n_rec] : 0),
+			    (long long)n_blk);
+	const std::vector<int64_t> &held = c->rec_off;
+	const int64_t held_nt = c->total_nt;
+	for (int64_t k = 0; k < n_blk; k++) {
+		const int64_t s = blk[2 * k], e = blk[2 * k + 1];
+		if (e < s)
+			return fail("block %lld [%lld, %lld) ends before it starts", (long long)k, (long long)s, (long long)e);
+		if (s < 0 || e > held_nt)
+			return fail("block %lld [%lld, %lld) outside the %lld held nucleotides", (long long)k, (long long)s, (long long)e,
+				    (long long)held_nt);
+		if (e > s) {
+			const size_t r = (size_t)(std::upper_bound(held.begin(), held.end(), s) - held.begin()) - 1;
+			if (e > held[r + 1])
+				return fail("block %lld [%lld, %lld) crosses the end of held record %lld [%lld, %lld)", (long long)k,
+					    (long long)s, (long long)e, (long long)r, (long long)held[r], (long long)held[r + 1]);
+		}
+	}
+	std::vector<int64_t> rec_off((size_t)n_rec + 1, 0);
+	for (int r = 0; r < n_rec; r++) {
+		if (strand[r] > 1)
+			return fail("strand[%d] = %u: 0 (plus) or 1 (minus)", r, (unsigned)strand[r]);
+		int64_t len = 0;
+		for (int64_t k = rec_blk[r]; k < rec_blk[r + 1] && len <= 0x7ffffff0ll; k++)
+			len += blk[2 * k + 1] - blk[2 * k];
+		if (len > 0x7ffffff0ll)
+			return fail("record %d longer than 2^31", r);
+		rec_off[r + 1] = rec_off[r] + len;
+	}
+	// the non-empty blocks in the new batch's order: seg_out (n_seg + 1 entries), then seg_src
+	std::vector<int64_t> seg_out(1, 0), seg_src;
+	for (int r = 0; r < n_rec; r++)
+		for (int64_t i = rec_blk[r]; i < rec_blk[r + 1]; i++) {
+			const int64_t k = strand[r] ? rec_blk[r + 1] - 1 - (i - rec_blk[r]) : i; // minus: the last block first
+			const int64_t s = blk[2 * k], e = blk[2 * k + 1];
+			if (e == s)
+				continue;
+			seg_src.push_back(strand[r] ? ~(e - 1) : s);
+			seg_out.push_back(seg_out.back() + (e - s));
+		}
+	const DbKind src_kind = c->db;
+	const bool chars = src_kind == DB_CHARS || src_kind == DB_FASTN || src_kind == DB_FASTQ;
+	const uint8_t *src_chars = chars ? c->d_seq_chars : nullptr;
+	if (begin_upload(c))
+		return -1;
+	NvtxRange nvtx_("gpumotif: assemble (device gather)");
+	const int64_t n_seg = (int64_t)seg_src.size();
+	c->asm_tab = std::move(seg_out);
+	c->asm_tab.insert(c->asm_tab.end(), seg_src.begin(), seg_src.end());
+	const size_t tab_bytes = c->asm_tab.size() * sizeof(int64_t);
+	if (set_records(c, rec_off.data(), n_rec))
+		return -1;
+	const int64_t n = c->total_nt;
+	if (c->d_packed_spare.ensure(packed_bytes(n)) || (chars && c->d_chars_spare.ensure((size_t)n + 64)) ||
+	    c->d_asm.ensure(tab_bytes))
+		return -1;
+	int64_t chunk;
+	if (cut_device_chunks(c, n, false, &chunk))
+		return -1;
+	CU(cudaEventRecord(c->up_ev[0], c->copy_stream));
+	CU(cudaMemcpyAsync(c->d_asm, c->asm_tab.data(), tab_bytes, cudaMemcpyHostToDevice, c->copy_stream));
+	const int64_t *d_seg_out = c->d_asm, *d_seg_src = c->d_asm + n_seg + 1;
+	for (int i = 0; i < (int)c->chunk_end.size(); i++) {
+		const int64_t o = (int64_t)i * chunk, len = c->chunk_end[i] - o;
+		if (chars)
+			gm_assemble_kernel<true><<<pack_blocks(c, len), 256, 0, c->copy_stream>>>(
+				c->d_packed, src_chars, d_seg_out, d_seg_src, n_seg, o, len, c->d_packed_spare, c->d_chars_spare);
+		else
+			gm_assemble_kernel<false><<<pack_blocks(c, len), 256, 0, c->copy_stream>>>(
+				c->d_packed, nullptr, d_seg_out, d_seg_src, n_seg, o, len, c->d_packed_spare, nullptr);
+		CU(cudaGetLastError());
+		CU(cudaEventRecord(c->chunk_ev[i], c->copy_stream));
+	}
+	// the held buffers become the spares: nothing reads them once the kernels above are done, and the
+	// next write to them comes after the next upload's begin_upload
+	c->d_packed.swap(c->d_packed_spare);
+	if (chars)
+		c->d_chars.swap(c->d_chars_spare);
+	c->d_seq_chars = chars ? c->d_chars.p : nullptr;
+	return finish_upload(c, chars ? DB_CHARS : src_kind, (uint64_t)(n_rec + 1) * 8 + (uint64_t)tab_bytes);
 }
 
 // The record table a device text reader has left in c->rec_off: every record under 2^31, then the

@@ -37,7 +37,7 @@ _lib = None
 
 EXPORTS = ["gm_last_error", "gm_version", "gm_device_count", "gm_host_alloc", "gm_host_free", "gm_ctx_create", "gm_ctx_destroy",
            "gm_plan_check", "gm_plan_describe", "gm_db_upload_chars", "gm_db_upload_chars_hostpack", "gm_host_pack", "gm_db_set_device_chars", "gm_db_upload_fastn",
-           "gm_db_upload_2bit", "gm_db_upload_fastn_bgzf", "gm_db_upload_fastq", "gm_db_upload_fastq_bgzf", "gm_ctx_set_min_quality",
+           "gm_db_upload_2bit", "gm_db_assemble", "gm_db_upload_fastn_bgzf", "gm_db_upload_fastq", "gm_db_upload_fastq_bgzf", "gm_ctx_set_min_quality",
            "gm_db_get_text",
            "gm_db_records", "gm_db_get_chars", "gm_db_total_nt", "gm_hit_windows",
            "gm_scan", "gm_scan_launch", "gm_scan_finish", "gm_hits", "gm_stats",
@@ -66,6 +66,7 @@ def lib():
         L.gm_db_upload_fastn.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
         L.gm_db_upload_2bit.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
                                         C.c_int64]
+        L.gm_db_assemble.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int]
         L.gm_db_upload_fastn_bgzf.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
         L.gm_db_upload_fastq.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
         L.gm_db_upload_fastq_bgzf.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
@@ -267,6 +268,20 @@ class MotifSearch:
         self._ck(lib().gm_db_upload_2bit(self._ctx, host_ptr, n_bytes, dna_off.ctypes.data, rec_off.ctypes.data,
                                          len(rec_off) - 1, nblk.ctypes.data if nblk.size else None, nblk.size // 2),
                  "gm_db_upload_2bit")
+
+    def assemble(self, blk, rec_blk, strand):
+        """gm_db_assemble: a new batch from blocks of the held one, gathered on the device.  blk: flat
+        [start, end) pairs in the held batch's rec_off coordinates; record r = blocks rec_blk[r] ..
+        rec_blk[r+1]-1 concatenated, reverse-complemented where strand[r] = 1."""
+        blk = np.ascontiguousarray(blk, dtype=np.int64).reshape(-1)
+        rec_blk = np.ascontiguousarray(rec_blk, dtype=np.int64)
+        strand = np.ascontiguousarray(strand, dtype=np.uint8)
+        self._ck(lib().gm_db_assemble(self._ctx, blk.ctypes.data if blk.size else None, blk.size // 2, rec_blk.ctypes.data,
+                                      strand.ctypes.data if strand.size else None, len(rec_blk) - 1), "gm_db_assemble")
+
+    def assemble_bed(self, asm):
+        """assemble() of a bed.Assembly (bed.read_bed over the held batch's names and rec_off)."""
+        self.assemble(asm.blk, asm.rec_blk, asm.strand)
 
     def upload_fastn_bgzf(self, buf):
         """gm_db_upload_fastn_bgzf: `buf` = a BGZF-compressed FASTA file's bytes (bytes or a uint8

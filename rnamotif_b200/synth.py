@@ -95,3 +95,84 @@ def random_reads(seed: int, lengths, stem_every: int = 120, n_rate: float = 0.00
             seq[rng.integers(0, n, size=rng.binomial(n, rate))] = ch
     ids = ["read%d" % i for i in range(len(lengths))]
     return ids, seq, off
+
+
+def random_transcripts(seed: int, names, sizes, n: int, exon: float = 130, first: float = 250, last: float = 900,
+                       intron: float = 1500, utr5: float = 150, utr3: float = 700, max_exons: int = 16,
+                       isoforms: int = 3, coding: float = 0.8, p_one: float = 0.03, p_edge: float = 0.03) -> str:
+    """Seeded BED12 lines: n transcripts over chromosomes `names` of `sizes` nt, about `isoforms` per gene.
+    Exon, intron and UTR lengths are log-normal around the given medians (the defaults are those of a
+    human annotation: internal exons ~130 nt, first and last exons longer, 5' UTRs ~150, 3' UTRs ~700).
+    What the lines include:
+      - one- and multi-exon transcripts on both strands, exons at odd and even offsets, and 1-nt
+        exons (share p_one);
+      - isoforms of a gene that share exons (exon skipping) and overlap them (an exon end moved);
+      - thick ranges inside the exons, a `coding` share of lines; the rest have thickStart == thickEnd;
+      - genes that start at 0 or end at the chromosome's end (share p_edge each)."""
+    import random
+    rng = random.Random(seed)
+    sizes = [int(s) for s in sizes]
+    chroms = [i for i, s in enumerate(sizes) if s > 0]
+    weights = [sizes[i] for i in chroms]
+
+    def draw(median):
+        return max(1, int(rng.lognormvariate(np.log(median), 0.8)))
+
+    lines = []
+    while len(lines) < n:
+        c = rng.choices(chroms, weights)[0]
+        size = sizes[c]
+        m = min(max_exons, 1 + int(rng.expovariate(1 / 6)))
+        ex = [draw(first)] + [draw(exon) for _ in range(m - 2)] + ([draw(last)] if m > 1 else [])
+        ex = [1 if rng.random() < p_one else z for z in ex]
+        gaps = [draw(intron) for _ in range(m - 1)]
+        while len(ex) > 1 and sum(ex) + sum(gaps) > size:
+            ex.pop()
+            gaps.pop()
+        ex[0] = min(ex[0], size)
+        span = sum(ex) + sum(gaps)
+        u = rng.random()
+        g0 = 0 if u < p_edge else size - span if u < 2 * p_edge else rng.randrange(0, size - span + 1)
+        gene = []
+        p = g0
+        for k, z in enumerate(ex):
+            gene.append((p, p + z))
+            p += z + (gaps[k] if k < len(gaps) else 0)
+        minus = rng.random() < 0.5
+        for _ in range(1 + rng.randrange(isoforms)):
+            if len(lines) >= n:
+                break
+            # exon skipping: the internal exons are kept with probability 0.8; an exon end moved now and then
+            keep = [s_e for k, s_e in enumerate(gene) if k in (0, len(gene) - 1) or rng.random() < 0.8]
+            tx = []
+            for k, (s, e) in enumerate(keep):
+                if e - s > 2 and rng.random() < 0.15:
+                    if k < len(keep) - 1:
+                        e -= rng.randrange(1, e - s)
+                    else:
+                        s += rng.randrange(1, e - s)
+                tx.append((s, e))
+            cs, ce = tx[0][0], tx[-1][1]
+            ln = sum(e - s for s, e in tx)
+            ts = te = cs
+            if rng.random() < coding and ln > 3:
+                # the UTRs as exonic lengths from either end, 5' on the transcript's own strand
+                a, b = draw(utr5), draw(utr3)
+                if minus:
+                    a, b = b, a
+                if a + b >= ln:
+                    a, b = rng.randrange(0, ln // 2), rng.randrange(0, ln // 2)
+                ts, te = _exonic(tx, a), _exonic(tx, ln - b)
+            lines.append("\t".join(map(str, [names[c], cs, ce, "tx%d" % len(lines), 0, "-" if minus else "+", ts, te, 0,
+                                             len(tx), "".join("%d," % (e - s) for s, e in tx),
+                                             "".join("%d," % (s - cs) for s, e in tx)])))
+    return "".join(line + "\n" for line in lines)
+
+
+def _exonic(exons, k):
+    """The chromosome position of exonic base k of ascending exons (k = their length: the last end)."""
+    for s, e in exons:
+        if k < e - s:
+            return s + k
+        k -= e - s
+    return exons[-1][1]
