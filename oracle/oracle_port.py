@@ -34,6 +34,9 @@ def lib():
         _lib.gmo_scan_db.restype = C.c_int64
         _lib.gmo_scan_db.argtypes = [C.c_char_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
                                      C.c_void_p, C.c_size_t, C.POINTER(Stats)]
+        _lib.gmo_scan_db_range.restype = C.c_int64
+        _lib.gmo_scan_db_range.argtypes = [C.c_char_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_int64,
+                                           C.c_void_p, C.c_size_t, C.POINTER(Stats)]
         _lib.gmo_hit_stride.restype = C.c_size_t
         _lib.gmo_hit_stride.argtypes = [C.c_char_p]
     return _lib
@@ -49,9 +52,12 @@ def hit_dtype(n_descr: int) -> np.dtype:
                      ("el", [("off", "<i4"), ("len", "<i2"), ("mpr", "i1"), ("mm", "i1")], n_descr)])
 
 
-def scan_db(plan: bytes, seq: np.ndarray, rec_off: np.ndarray, both: bool, cap_hits: int = 1 << 20):
+def scan_db(plan: bytes, seq: np.ndarray, rec_off: np.ndarray, both: bool, cap_hits: int = 1 << 20,
+            f_range: tuple[int, int] | None = None):
     """Run the oracle over a database.  Returns (hits structured array in the
-    reference's enumeration order, Stats)."""
+    reference's enumeration order, Stats).  f_range = (lo, hi): only the starts whose
+    5' end lies at a forward position in [lo, hi) of each record (a complementary-strand
+    start owns forward position slen - 1 - szero)."""
     L = lib()
     n_descr = plan_n_descr(plan)
     dt = hit_dtype(n_descr)
@@ -61,8 +67,12 @@ def scan_db(plan: bytes, seq: np.ndarray, rec_off: np.ndarray, both: bool, cap_h
     st = Stats()
     while True:
         out = np.zeros(cap_hits, dtype=dt)
-        n = L.gmo_scan_db(plan, seq.ctypes.data, rec_off.ctypes.data, len(rec_off) - 1, int(both),
-                          out.ctypes.data, out.nbytes, C.byref(st))
+        if f_range is None:
+            n = L.gmo_scan_db(plan, seq.ctypes.data, rec_off.ctypes.data, len(rec_off) - 1, int(both),
+                              out.ctypes.data, out.nbytes, C.byref(st))
+        else:
+            n = L.gmo_scan_db_range(plan, seq.ctypes.data, rec_off.ctypes.data, len(rec_off) - 1, int(both),
+                                    int(f_range[0]), int(f_range[1]), out.ctypes.data, out.nbytes, C.byref(st))
         if n < 0:
             raise RuntimeError("oracle scan failed (bad plan?)")
         if n <= cap_hits:

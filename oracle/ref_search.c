@@ -22,6 +22,7 @@
  * stack, lazy candidates, window-relative), so agreement between the two is
  * evidence, not tautology.  Each function cites what it restates.
  */
+#include <limits.h>
 #include <stdint.h>
 #include <stdlib.h>
 #include <string.h>
@@ -1164,9 +1165,11 @@ static int o_find_motif(gmo_t *g, int s)
 }
 
 /* RM_find_motif, src/find_motif.c:164-207 (without the output-neutral literal
- * prefilter adjust_szero, :209-243) */
-int gmo_scan_strand(const gm_plan_t *pl, const uint8_t *codes, int slen, int comp,
-	uint32_t rec, gmo_sink_fn sink, void *user, gmo_stats_t *stats)
+ * prefilter adjust_szero, :209-243), over the starts szero in [s_lo, s_hi) only:
+ * each start's search depends on the strand and szero alone, so a range gives
+ * exactly the whole strand's candidates of those starts */
+static int scan_strand_range(const gm_plan_t *pl, const uint8_t *codes, int slen, int comp,
+	uint32_t rec, int s_lo, int s_hi, gmo_sink_fn sink, void *user, gmo_stats_t *stats)
 {
 	gmo_t *g;
 	int w_winsize, l_szero, d, i, rv = 0, wsz;
@@ -1201,7 +1204,7 @@ int gmo_scan_strand(const gm_plan_t *pl, const uint8_t *codes, int slen, int com
 
 	w_winsize = pl->dmaxlen < pl->windowsize ? pl->dmaxlen : pl->windowsize;
 	l_szero = slen - w_winsize;
-	for (g->szero = 0; g->szero < l_szero; g->szero++) {
+	for (g->szero = OMAX(s_lo, 0); g->szero < l_szero && g->szero < s_hi; g->szero++) {
 		g->s_zero[0] = g->szero;
 		g->s_dollar[0] = OMIN(g->szero + w_winsize - 1, slen - 1);
 		g->seq = 0;
@@ -1210,7 +1213,7 @@ int gmo_scan_strand(const gm_plan_t *pl, const uint8_t *codes, int slen, int com
 	}
 	l_szero = slen - pl->dminlen;
 	g->s_dollar[0] = slen - 1;
-	for (; g->szero <= l_szero; g->szero++) {
+	for (; g->szero <= l_szero && g->szero < s_hi; g->szero++) {
 		g->s_zero[0] = g->szero;
 		g->seq = 0;
 		g->st->n_starts++;
@@ -1219,6 +1222,12 @@ int gmo_scan_strand(const gm_plan_t *pl, const uint8_t *codes, int slen, int com
 	free(g->winbuf);
 	free(g);
 	return rv;
+}
+
+int gmo_scan_strand(const gm_plan_t *pl, const uint8_t *codes, int slen, int comp,
+	uint32_t rec, gmo_sink_fn sink, void *user, gmo_stats_t *stats)
+{
+	return scan_strand_range(pl, codes, slen, comp, rec, 0, INT_MAX, sink, user, stats);
 }
 
 /* ------------------------------------------------ convenience for ctypes */
@@ -1256,9 +1265,12 @@ size_t gmo_hit_stride(const gm_plan_t *pl)
  * (gm_hit_hdr_t + n_descr gm_hit_el_t) are written to `out` in the
  * reference's enumeration order.  Returns the number of candidates (which
  * may exceed what fitted: compare with out_cap / stride), or -1.
+ * gmo_scan_db_range searches only the starts whose 5' end lies at a forward
+ * position in [f_lo, f_hi) of each record (gm_scan's range contract, in
+ * record coordinates); gmo_scan_db searches them all.
  */
-int64_t gmo_scan_db(const gm_plan_t *pl, const char *seq, const int64_t *rec_off,
-	int n_rec, int both, void *out, size_t out_cap, gmo_stats_t *stats)
+int64_t gmo_scan_db_range(const gm_plan_t *pl, const char *seq, const int64_t *rec_off,
+	int n_rec, int both, int64_t f_lo, int64_t f_hi, void *out, size_t out_cap, gmo_stats_t *stats)
 {
 	gmo_collect_t c;
 	int r;
@@ -1281,12 +1293,18 @@ int64_t gmo_scan_db(const gm_plan_t *pl, const char *seq, const int64_t *rec_off
 	}
 	for (r = 0; r < n_rec; r++) {
 		int64_t n = rec_off[r + 1] - rec_off[r];
+		/* the starts whose 5' end lies at a forward position in [f_lo, f_hi): a
+		 * complementary-strand start owns forward position n - 1 - szero */
+		int64_t lo = OMAX(f_lo, 0), hi = OMIN(f_hi, n);
+		if (hi <= lo)
+			continue;
 		gmo_encode(seq + rec_off[r], n, codes);
-		if (gmo_scan_strand(pl, codes, (int)n, 0, (uint32_t)r, collect_sink, &c, stats) < 0)
+		if (scan_strand_range(pl, codes, (int)n, 0, (uint32_t)r, (int)lo, (int)hi, collect_sink, &c, stats) < 0)
 			goto fail;
 		if (both) {
 			gmo_revcomp(codes, n, rc);
-			if (gmo_scan_strand(pl, rc, (int)n, 1, (uint32_t)r, collect_sink, &c, stats) < 0)
+			if (scan_strand_range(pl, rc, (int)n, 1, (uint32_t)r, (int)(n - hi), (int)(n - lo), collect_sink, &c,
+					      stats) < 0)
 				goto fail;
 		}
 	}
@@ -1297,4 +1315,10 @@ fail:
 	free(codes);
 	free(rc);
 	return -1;
+}
+
+int64_t gmo_scan_db(const gm_plan_t *pl, const char *seq, const int64_t *rec_off,
+	int n_rec, int both, void *out, size_t out_cap, gmo_stats_t *stats)
+{
+	return gmo_scan_db_range(pl, seq, rec_off, n_rec, both, 0, INT64_MAX, out, out_cap, stats);
 }

@@ -575,7 +575,8 @@ __device__ __noinline__ bool sink_context(const Lane &L, int ctx[4])
 	if (PV.rctx.present) {
 		int last = L.ND - 1;
 		int roff = L.szero + m_off(L, last) + m_len(L, last);
-		int end = min(roff + PV.rctx.maxlen, L.slen);
+		// roff + maxlen passes 2^31 - 1 near the end of a record at the length cap
+		int end = roff + min(PV.rctx.maxlen, L.slen - roff);
 		int len = end - roff;
 		ctx[2] = roff;
 		ctx[3] = len;
